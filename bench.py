@@ -43,10 +43,39 @@ def parse():
                          "are mixed and the step time is the stationary one")
     ap.add_argument("--cpu-baseline-seconds", type=float, default=20.0)
     ap.add_argument("--e2e-steps", type=int, default=0,
-                    help="steps of the end-to-end passes (default: max(--steps, 200): a 20-step window is 4-8 ms of wall "
-                         "clock and +-10 %% noisy)")
+                    help="steps of the end-to-end passes (default: --steps; a 20-step window is 4-8 ms of wall clock and "
+                         "+-10 %% noisy, 200 steps give a steadier e2e figure)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned to rank 0's caller (obs, reward, "
+                         "done, term) as DIR/<name>.npy; the inputs depend only on the arguments, so two builds can be "
+                         "compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "fwgym":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl fwgym)")
+    return a
+
+
+DUMP_LIMIT_BYTES = 60 * 1024 * 1024     # keeps a dump, .npy headers included, under 64 MB
+
+
+def dump_outputs(path, arrays, limit=DUMP_LIMIT_BYTES):
+    """Write the per-env host arrays of `arrays` (name -> [N, ...], float32 or float64) as path/<name>.npy.  Above
+    `limit` bytes in all, every array keeps the same fixed, seeded sample of env rows, ascending, and env_index.npy
+    (float64) lists them."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(x[:1].nbytes for x in arrays.values())
+    if n * row_bytes > limit:
+        keep = limit // (row_bytes + 8)     # + the float64 index entry of each kept row
+        idx = np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+        arrays = {k: x[idx] for k, x in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    for k, x in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), x)
 
 
 # ------------------------------------------------------------------------------------------------ CPU reference arm
@@ -239,10 +268,14 @@ def run_gpu_arm(a):
     for k in range(a.steps):
         flush_l2()                          # L2 flush between timed iterations (not inside the timed interval)
         ev[k][0].record()
-        vec.step_tensors(actions[a.warmup + k])
+        last = vec.step_tensors(actions[a.warmup + k])
         ev[k][1].record()
     barrier()
     wall = time.perf_counter() - t_wall0
+    if a.dump_outputs and rank == 0:        # the env's output buffers: the passes below overwrite them
+        obs, rew, done, term = (x.cpu().numpy() for x in last)
+        dump_outputs(a.dump_outputs, {"obs": obs, "reward": rew, "done": done.astype(np.float32),
+                                      "term": term.astype(np.float64)})
     step_ms = sorted(e0.elapsed_time(e1) for e0, e1 in ev)
     ms = sum(step_ms)
     ctr = vec.counters()
@@ -333,7 +366,7 @@ def run_gpu_arm(a):
     #   open loop, depth 2 (round 1's number): action t+1 is sent before observation t is read - an upper bound no
     #     policy can use.
     from fwgym_b200 import HostStepper
-    e2e_steps = a.e2e_steps or max(a.steps, 200)
+    e2e_steps = a.e2e_steps or a.steps
     n_act = 48
     host_actions = (torch.rand((n_act, n, 3)) * 2 - 1).pin_memory()
     checksum = 0.0

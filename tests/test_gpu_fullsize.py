@@ -98,6 +98,31 @@ def test_ppo_loop_runs(built_lib, graph):
     env.close()
 
 
+def test_bench_dump_outputs_repeat(built_lib, tmp_path):
+    """bench.py --dump-outputs: the last timed step's obs / reward / done / term, the same in two runs with the same
+    arguments, and every timed pass runs --steps steps."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for rep in range(2):
+        out_dir = tmp_path / str(rep)
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "3", "--warmup", "2",
+                              "--envs-per-gpu", "512", "--burn-in", "20", "--no-cpu-baseline",
+                              "--dump-outputs", str(out_dir)], capture_output=True, text=True, timeout=600, cwd=root)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads(out.stdout)
+        assert line["steps"] == 3 and line["e2e"]["steps"] == 3
+        dumps.append({k: np.load(out_dir / (k + ".npy")) for k in ("obs", "reward", "done", "term")})
+    d = dumps[0]
+    assert d["obs"].shape == (512, 14) and d["obs"].dtype == np.float32 and d["reward"].shape == (512,)
+    assert set(np.unique(d["done"])) <= {0.0, 1.0} and np.isfinite(d["obs"]).all()
+    for k in d:
+        assert np.array_equal(d[k], dumps[1][k]), k
+
+
 def test_vecnormalize_and_gae_on_device(built_lib):
     """DeviceVecNormalize / compute_gae on cuda:0 against the numpy twins of stable-baselines' VecNormalize and PPO2's
     GAE (tests/test_ppo_cpu.py holds the oracle and runs the same check on the CPU)."""
