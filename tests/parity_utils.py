@@ -61,10 +61,11 @@ def run_parity(vec, oracles, actions, check_state=True):
 
 # ---- oracle rollouts over all host cores (BASELINE configs[1] at its stated size: 4096 envs x 100 steps) -------------
 def oracle_rollout_slice(args):
-    """Worker (own process): free-running rollout of oracle envs [lo, hi) on `actions` [T, hi - lo, 3].
-    -> dict of per-step arrays: obs [T + 1, n, D], rew / done / k / term [T, n], state [T, n, 27]."""
-    config, config_kw, sim_kw, seed, lo, hi, actions = args
-    orcs = make_oracles(hi - lo, config, config_kw, sim_kw, seed, env_offset=lo)
+    """Worker (own process): free-running rollout of the oracle envs with global ids `env_ids` on `actions`
+    [T, len(env_ids), 3].  -> dict of per-step arrays: obs [T + 1, n, D], rew / done / k / term [T, n], state [T, n, 27]."""
+    config, config_kw, sim_kw, seed, env_ids, actions = args
+    orcs = [harness.OracleRunner(harness.make_env("restated", config, config_kw, sim_kw), seed, int(gid))
+            for gid in env_ids]
     T = actions.shape[0]
     obs = [np.stack([np.asarray(o.reset(), dtype=np.float64).ravel() for o in orcs])]
     rew, done, k, state, term = [], [], [], [], []
@@ -80,13 +81,15 @@ def oracle_rollout_slice(args):
                 term=np.array(term))
 
 
-def oracle_rollout_parallel(config, config_kw, sim_kw, seed, actions, procs=None):
-    """Split the envs of `actions` [T, N, 3] over `procs` spawned worker processes (spawn, not fork: the caller holds a
-    CUDA context) and stitch the per-step arrays back together along the env axis."""
+def oracle_rollout_ids(config, config_kw, sim_kw, seed, env_ids, actions, procs=None):
+    """Free-running oracle rollout of the envs with global ids `env_ids` (any order, need not be contiguous: the Philox
+    streams are keyed by the global id) on `actions` [T, len(env_ids), 3].  The envs are split over `procs` spawned
+    worker processes (spawn, not fork: the caller holds a CUDA context); the per-step arrays come back in the order of
+    `env_ids` along the env axis."""
     import multiprocessing as mp
     import os
-    import sys
-    n = actions.shape[1]
+    env_ids = np.asarray(env_ids, dtype=np.int64)
+    n = len(env_ids)
     procs = min(procs or os.cpu_count() or 1, n)
     bounds = np.linspace(0, n, procs + 1).astype(int)
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -96,8 +99,13 @@ def oracle_rollout_parallel(config, config_kw, sim_kw, seed, actions, procs=None
         ctx = mp.get_context("spawn")
         with ctx.Pool(procs) as pool:
             parts = pool.map(oracle_rollout_slice,
-                             [(config, config_kw, sim_kw, seed, int(lo), int(hi), actions[:, lo:hi])
+                             [(config, config_kw, sim_kw, seed, env_ids[lo:hi], actions[:, lo:hi])
                               for lo, hi in zip(bounds[:-1], bounds[1:]) if hi > lo], chunksize=1)
     finally:
         os.environ["PYTHONPATH"] = old
     return {key: np.concatenate([p[key] for p in parts], axis=1) for key in parts[0]}
+
+
+def oracle_rollout_parallel(config, config_kw, sim_kw, seed, actions, procs=None):
+    """oracle_rollout_ids over the contiguous envs 0 .. N - 1 of `actions` [T, N, 3]."""
+    return oracle_rollout_ids(config, config_kw, sim_kw, seed, np.arange(actions.shape[1]), actions, procs)
