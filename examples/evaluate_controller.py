@@ -5,11 +5,13 @@
     python examples/evaluate_controller.py tests/golden/test_set_wind_none.npz --PID
     python examples/evaluate_controller.py tests/golden/test_set_wind_none.npz --model-path tests/golden/mlp_controller.npz
     python examples/evaluate_controller.py path/to/test_set.npy --PID --turbulence-intensity moderate
+    python examples/evaluate_controller.py tests/golden/test_set_wind_none.npz --PID --turbulence-intensity none light moderate severe
 
 `path_to_file`: the reference's pickled test set (.npy, list of {"state", "target"}) or the plain-array fixture
 (.npz).  `--model-path`: an .npz with the arrays of a stable-baselines PPO2 MlpPolicy and its VecNormalize statistics
 (oracle/make_golden_policy.py writes one from examples/models/mlp_controller).  Prints the reference's result table
-(nan-mean per metric and state, evaluate_controller.py:32-41) and optionally saves the result dictionary in the
+(nan-mean per metric and state, evaluate_controller.py:32-41; one table per level when several turbulence levels are
+given: they fly as one batch, each scenario once per level) and optionally saves the result dictionary in the
 reference's layout (res[metric][state] = [value per scenario], res["rewards"])."""
 import argparse
 import os
@@ -25,7 +27,8 @@ if __name__ == "__main__":
     ap.add_argument("--PID", dest="use_pid", action="store_true", help="use the PID controller")
     ap.add_argument("--model-path", help=".npz with the MlpPolicy arrays (tests/golden/mlp_controller.npz)")
     ap.add_argument("--env-config-path", help="env configuration JSON (default: the examples configuration)")
-    ap.add_argument("--turbulence-intensity", default="none", choices=["none", "light", "moderate", "severe"])
+    ap.add_argument("--turbulence-intensity", nargs="+", default=["none"], choices=["none", "light", "moderate", "severe"],
+                    help="one or more levels; several levels run as one batch (a result table per level)")
     ap.add_argument("--save", help="write the result dictionary to this .npy")
     a = ap.parse_args()
     if not a.use_pid and not a.model_path:
@@ -37,13 +40,19 @@ if __name__ == "__main__":
     cfg = a.env_config_path or os.path.join(os.path.dirname(DEFAULT_ENV_CONFIG), "fixed_wing_config_examples.json")
     scenarios = evaluate.load_test_set(a.path_to_file)
     controller = "pid" if a.use_pid else dict(np.load(a.model_path))
+    levels = a.turbulence_intensity
     res, vec = evaluate.evaluate_on_set(scenarios, cfg, controller=controller,
-                                        turbulence_intensity=a.turbulence_intensity)
-    print("%d scenarios, mean episode length %.1f steps" % (len(scenarios), float(np.mean(res["lengths"]))))
-    for key, val in sorted(evaluate.summarise(res).items()):
-        print("\t%-28s %.4f" % (key, val))
+                                        turbulence_intensity=levels[0] if len(levels) == 1 else levels)
+    by_level = {levels[0]: res} if len(levels) == 1 else res
+    saved = {}
+    for lv, r in by_level.items():
+        print("turbulence %s: %d scenarios, mean episode length %.1f steps" % (lv, len(scenarios),
+                                                                           float(np.mean(r["lengths"]))))
+        for key, val in sorted(evaluate.summarise(r).items()):
+            print("\t%-28s %.4f" % (key, val))
+        out = {m: r[m] for m in evaluate.DEFAULT_METRICS}
+        out["rewards"] = [np.asarray(x) for x in r["rewards"]]
+        saved[lv] = out
     if a.save:
-        out = {m: res[m] for m in evaluate.DEFAULT_METRICS}
-        out["rewards"] = [np.asarray(r) for r in res["rewards"]]
-        np.save(a.save, out, allow_pickle=True)
+        np.save(a.save, saved[levels[0]] if len(levels) == 1 else saved, allow_pickle=True)
     vec.close()

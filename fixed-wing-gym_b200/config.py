@@ -29,6 +29,8 @@ F32_MAX = float(np.finfo(np.float32).max)
 FCLASS = {"linear": 0, "exponential": 1, "quadratic": 2}
 TCLASS = {"constant": 0, "linear": 1, "sinusoidal": 2, "compensate": 3}
 ACT_NAMES = ["elevator", "aileron", "throttle"]
+# Dryden intensities of a mixed handle, in level order (include/fwgym.h fw_sim_t.turb_mixed)
+TURB_LEVELS = ("none", "light", "moderate", "severe")
 
 
 class ConfigError(ValueError):
@@ -135,6 +137,23 @@ def dryden_transfer_functions(b, intensity, h=100.0, V_a=25.0):
     ]
 
 
+def turbulence_cdf(probabilities):
+    """Level probabilities [p_none, p_light, p_moderate, p_severe] -> the fp64 cumulative table the reset draw searches
+    (fw_sim_t.turb_cdf): running sums in level order, and 1 from the last level with a non-zero probability on, so a
+    uniform in [0, 1) never lands past it."""
+    cdf, acc = [], 0.0
+    last = max(i for i, p in enumerate(probabilities) if p > 0)
+    for i, p in enumerate(probabilities):
+        acc += float(p)
+        cdf.append(1.0 if i >= last else acc)
+    return cdf
+
+
+def draw_turbulence_level(cdf, u):
+    """The level a reset draws for the uniform `u` (csrc/env.cuh fw_reset_env_body): the first l with u < cdf[l]."""
+    return int(sum(1 for c in cdf[:-1] if u >= c))
+
+
 def discretise_filter(num, den, dt):
     """The (Ad, Bd0, Bd1, C, D) that scipy.signal.lsim(interp=True) builds from a transfer function."""
     import scipy.linalg
@@ -162,11 +181,16 @@ class CompiledConfig:
         if config_kw is not None:
             apply_overrides(self.cfg, copy.deepcopy(config_kw))
         sim_config_kw = dict(sim_config_kw or {})
+        # the dict form of turbulence_intensity (per-env levels) replaces PyFly's string leaf instead of descending into it
+        turb_mix = sim_config_kw.pop("turbulence_intensity") if isinstance(sim_config_kw.get("turbulence_intensity"),
+                                                                         dict) else None
         sim_config_kw.update({"actuation": {"inputs": [a["name"] for a in self.cfg["action"]["states"]]}})
         sim_config_kw["turbulence_sim_length"] = self.cfg["steps_max"]
         with open(sim_config_path or DEFAULT_SIM_CONFIG) as f:
             self.sim_cfg = json.load(f)
         _set_sim_config_attrs(self.sim_cfg, copy.deepcopy(sim_config_kw))
+        if turb_mix is not None:
+            self.sim_cfg["turbulence_intensity"] = copy.deepcopy(turb_mix)
         with open(sim_parameter_path or DEFAULT_SIM_PARAMS) as f:
             self.params = {k: v for k, v in json.load(f).items() if not k.startswith("_")}
         self.precision = {"fp64": 0, "fp32": 1}[precision]
@@ -201,6 +225,43 @@ class CompiledConfig:
         self._rand_plan()   # raises on simulator-parameter randomisation entries the device path cannot honour
         if self.sim_cfg["turbulence"] and not self.cfg["steps_max"] > 0:
             raise ConfigError("turbulence needs steps_max > 0 (turbulence_sim_length = steps_max, fixed_wing.py:40)")
+        self.turbulence_mix = self._turbulence_mix()
+
+    def _turbulence_mix(self):
+        """sim_config_kw turbulence_intensity = {"values": [level names], "probabilities": [...]} (the reference's
+        values / probabilities syntax for simulator attributes, fixed_wing.py:561-569; omitted probabilities are uniform,
+        as np.random.choice) -> the probabilities of the four levels in TURB_LEVELS order; None for the string form."""
+        spec = self.sim_cfg.get("turbulence_intensity")
+        if not isinstance(spec, dict):
+            return None
+        if not self.sim_cfg["turbulence"]:
+            raise ConfigError("turbulence_intensity {values, probabilities} needs turbulence: True")
+        unknown = set(spec) - {"values", "probabilities"}
+        if unknown or "values" not in spec:
+            raise ConfigError("turbulence_intensity: expected {\"values\": [...], \"probabilities\": [...]}, got keys %s"
+                              % sorted(spec))
+        values = list(spec["values"])
+        if not values:
+            raise ConfigError("turbulence_intensity: values is empty")
+        for v in values:
+            if v not in TURB_LEVELS:
+                raise ConfigError("turbulence_intensity: unknown level %r (levels: %s)" % (v, ", ".join(TURB_LEVELS)))
+        if len(set(values)) != len(values):
+            raise ConfigError("turbulence_intensity: a level is listed twice in %r" % (values,))
+        probs = spec.get("probabilities")
+        if probs is None:
+            probs = [1.0 / len(values)] * len(values)
+        probs = [float(p) for p in probs]
+        if len(probs) != len(values):
+            raise ConfigError("turbulence_intensity: %d values but %d probabilities" % (len(values), len(probs)))
+        if any(not p >= 0 for p in probs):
+            raise ConfigError("turbulence_intensity: negative probability in %r" % (probs,))
+        if not abs(math.fsum(probs) - 1.0) <= 1e-12:
+            raise ConfigError("turbulence_intensity: probabilities sum to %r, not 1" % math.fsum(probs))
+        out = [0.0] * len(TURB_LEVELS)
+        for v, p in zip(values, probs):
+            out[TURB_LEVELS.index(v)] = p
+        return out
 
     # --------------------------------------------------- fixed_wing.py:523-570 (sample_simulator_parameters) as a table
     LIVE_PARAMS = ("mass", "S_wing", "b", "c", "S_prop", "k_motor", "k_T_P", "k_Omega", "C_prop", "e", "M", "a_0", "ar",
@@ -453,7 +514,9 @@ class CompiledConfig:
         s.wind_enabled = 1 if (sc["wind_magnitude_max"] != 0 or sc["wind_magnitude_min"] != 0
                                or sc.get("allow_wind_injection", False)) else 0
         s.turb_noise_scale = math.sqrt(math.pi / sc["dt"])
-        if sc["turbulence"]:
+        if sc["turbulence"] and self.turbulence_mix is not None:
+            self._fill_turbulence_mix(s, P, sc)
+        elif sc["turbulence"]:
             length = sc.get("turbulence_sim_length", 250)
             # PyFly simulates `length` samples on t = linspace(0, length*dt, length): spacing length*dt/(length-1)
             dt_eff = float(np.diff(np.linspace(0, length * sc["dt"], length))[0]) if length > 1 else sc["dt"]
@@ -509,6 +572,50 @@ class CompiledConfig:
         _, slot1, _ = self._rand_slots()
         for i, v in enumerate(slot1):
             s.par_slot1[i] = v
+
+    @staticmethod
+    def turbulence_dt(sc):
+        """The sample spacing of PyFly's Dryden simulation: `length` samples on t = linspace(0, length*dt, length)."""
+        length = sc.get("turbulence_sim_length", 250)
+        return float(np.diff(np.linspace(0, length * sc["dt"], length))[0]) if length > 1 else sc["dt"]
+
+    @staticmethod
+    def compile_turbulence_levels(b, dt):
+        """(Ad, Bd0, Bd1, C, D, stream) of the six shaping filters for light, moderate and severe.  The intensity enters
+        only through the numerators, so Ad / Bd0 / Bd1 (built from the denominators) must come out bitwise equal across
+        the levels: one filter state then serves every level and only the output rows C / D are per level."""
+        out = {}
+        for lvl in TURB_LEVELS[1:]:
+            out[lvl] = [discretise_filter(num, den, dt) + (stream,)
+                        for num, den, stream in dryden_transfer_functions(b, lvl)]
+        ref = out[TURB_LEVELS[1]]
+        for lvl in TURB_LEVELS[2:]:
+            for f, (a, b_) in enumerate(zip(ref, out[lvl])):
+                for k in range(3):
+                    if np.asarray(a[k]).tobytes() != np.asarray(b_[k]).tobytes():
+                        raise ConfigError("Dryden filter %d: the state matrices of %s and %s differ; per-env intensities "
+                                          "need them equal" % (f, TURB_LEVELS[1], lvl))
+        return out
+
+    def _fill_turbulence_mix(self, s, P, sc):
+        """Mixed handle: filt[] holds the shared Ad / Bd0 / Bd1 (its C / D stay zero: the kernels read turb_C / turb_D of
+        the episode's level), turb_C / turb_D one row per level (level 0, none, all zero) and turb_cdf the draw table."""
+        levels = self.compile_turbulence_levels(P["b"], self.turbulence_dt(sc))
+        s.turb_mixed = 1
+        for i, (Ad, Bd0, Bd1, _C, _D, stream) in enumerate(levels[TURB_LEVELS[1]]):
+            f = s.filt[i]
+            f.n, f.stream = Ad.shape[0], stream
+            for a in range(f.n):
+                for b_ in range(f.n):
+                    f.Ad[a * 3 + b_] = float(Ad[a, b_])
+                f.Bd0[a], f.Bd1[a] = float(Bd0[a]), float(Bd1[a])
+        for li, lvl in enumerate(TURB_LEVELS[1:], start=1):
+            for i, (_Ad, _Bd0, _Bd1, C, D, _stream) in enumerate(levels[lvl]):
+                for a in range(len(C)):
+                    s.turb_C[li][i][a] = float(C[a])
+                s.turb_D[li][i] = D
+        for li, c in enumerate(turbulence_cdf(self.turbulence_mix)):
+            s.turb_cdf[li] = c
 
     def _fill_env(self, e):
         cfg = self.cfg

@@ -502,12 +502,18 @@ __device__ __forceinline__ void fw_turb_noise_injected(const fw_sim_t& P, const 
 // advance the six shaping filters by one sample (scipy lsim recurrence) and refresh the gust rows.  The host zero-pads
 // Ad / Bd0 / Bd1 / C of filters of order < 3 (config.py), so the generic loops are fixed-size and everything stays in
 // registers; a fixed shape knows each filter's order and skips the padding (whose states stay exactly zero).
+// A mixed shape (SH::mixed) reads the output rows C / D of the episode's level `tlvl` (1..3) instead of the handle's:
+// the state recurrence does not depend on the intensity, and the operation order is the same as for filt[f].C / D, so
+// an env at level l computes bitwise what a handle of that uniform intensity computes.
 template <class SH>
-__device__ __forceinline__ void fw_turb_advance(const fw_sim_t& P, const FwEnvCtx& c, const double (&unew)[4]) {
+__device__ __forceinline__ void fw_turb_advance(const fw_sim_t& P, const FwEnvCtx& c, const double (&unew)[4],
+                                                int tlvl = 0) {
   const fw_sim_t& Ps = SH::sim(P);
 #pragma unroll
   for (int f = 0; f < FW_N_FILT; ++f) {
     const fw_filter_t& F = P.filt[f];
+    const double* __restrict__ Cf = SH::mixed ? P.turb_C[tlvl][f] : F.C;
+    const double Df = SH::mixed ? P.turb_D[tlvl][f] : F.D;
     const int st = Ps.filt[f].stream;
     const int nf = SH::fixed ? Ps.filt[f].n : FW_FILT_MAXN;
     const double up = c.D(D_TU + st);
@@ -515,7 +521,7 @@ __device__ __forceinline__ void fw_turb_advance(const fw_sim_t& P, const FwEnvCt
     double x[FW_FILT_MAXN], xn[FW_FILT_MAXN];
 #pragma unroll
     for (int a = 0; a < FW_FILT_MAXN; ++a) x[a] = a < nf ? c.D(D_TX + 3 * f + a) : 0.0;
-    double yv = F.D * un;
+    double yv = Df * un;
 #pragma unroll
     for (int b = 0; b < FW_FILT_MAXN; ++b) {
       if (b < nf) {
@@ -524,7 +530,7 @@ __device__ __forceinline__ void fw_turb_advance(const fw_sim_t& P, const FwEnvCt
         for (int a = 0; a < FW_FILT_MAXN; ++a)
           if (a < nf) s += x[a] * F.Ad[a * FW_FILT_MAXN + b];
         xn[b] = s;
-        yv += s * F.C[b];
+        yv += s * Cf[b];
       }
     }
 #pragma unroll
@@ -728,7 +734,22 @@ __device__ __forceinline__ void fw_reset_env_body(const fw_env_t& E, const fw_si
   // Dryden: x = 0, first sample drawn, gust = D*u0
   for (int j = 0; j < 18; ++j) c.D(D_TX + j) = 0.0;
   double gl[3] = {0, 0, 0};
-  if (Ps.turbulence) {
+  // mixed handle: the episode's intensity, the requested level or one draw of its own stream (no other draw moves);
+  // level 0 (none) then takes exactly the path of a handle without turbulence
+  int tlvl = 0;
+  if constexpr (SH::mixed) {
+    const int req = c.I(Ls.tl_row);
+    if (req >= 0) {
+      tlvl = req;
+    } else {
+      const double u = fw_uniform01<SH::fixed>(g, FW_RS_TURBLVL, 0);
+      tlvl = (u >= P.turb_cdf[0]) + (u >= P.turb_cdf[1]) + (u >= P.turb_cdf[2]);   // first l with u < cdf[l]
+    }
+    c.I(Ls.tl_row + 1) = tlvl;
+  }
+  // (the condition is spelled out at both of its uses, not kept in a variable: a handle without per-env levels then
+  // compiles to exactly the code it compiled to before they existed)
+  if (SH::mixed ? tlvl != 0 : Ps.turbulence != 0) {
     double u0[4];
     if (ti.noise) fw_turb_noise_injected(P, ti, c.env, 0, u0);
     else fw_turb_noise_g<SH::fixed>(P, g, 0, u0);
@@ -736,7 +757,8 @@ __device__ __forceinline__ void fw_reset_env_body(const fw_env_t& E, const fw_si
 #pragma unroll
     for (int f = 0; f < FW_N_FILT; ++f) {
       const int st = Ps.filt[f].stream;
-      const double gv = P.filt[f].D * (st == 0 ? u0[0] : (st == 1 ? u0[1] : (st == 2 ? u0[2] : u0[3])));
+      const double Df = SH::mixed ? P.turb_D[tlvl][f] : P.filt[f].D;
+      const double gv = Df * (st == 0 ? u0[0] : (st == 1 ? u0[1] : (st == 2 ? u0[2] : u0[3])));
       c.D(D_GUST + f) = gv;
       if (f < 3) gl[f] = gv;
     }
@@ -834,7 +856,7 @@ __device__ __forceinline__ void fw_reset_env_body(const fw_env_t& E, const fw_si
   flags |= FWF_HIST_VALID;
   flags &= ~(7u << FWF_PREVSHAPE_SHIFT);
   flags &= ~(FWF_EP_SUCCESS | FWF_TURB_INJ);
-  if (ti.noise && Ps.turbulence) flags |= FWF_TURB_INJ;
+  if (ti.noise && (SH::mixed ? tlvl != 0 : Ps.turbulence != 0)) flags |= FWF_TURB_INJ;
   // reward.randomize_scaling (fixed_wing.py:330-334): after the observation and the history rebuild, one uniform draw
   // per factor configured with scaling = [low, high], in factor order
   if (Es.n_scale_rows > 0)

@@ -16,17 +16,24 @@
 #include "layout.h"
 #include "env_shapes_gen.h"
 
+// `mixed`: the configuration flies each env at its own Dryden intensity (fw_sim_t.turb_mixed).  A compile-time property
+// of every shape, so that the per-env level code exists only in the instantiations that need it: the generic kernels
+// come in two instantiations, FwShapeGeneric (one intensity for the whole handle) and FwShapeGenericMixed.
 struct FwShapeGeneric {
   static constexpr bool fixed = false;
+  static constexpr bool mixed = false;
   static constexpr fw_env_t cenv{};
   static __device__ __forceinline__ const fw_env_t& env(const fw_env_t& E) { return E; }
   static __device__ __forceinline__ const fw_sim_t& sim(const fw_sim_t& P) { return P; }
   static __device__ __forceinline__ const FwLayout& lay(const FwLayout& L) { return L; }
 };
+struct FwShapeGenericMixed : FwShapeGeneric {
+  static constexpr bool mixed = true;
+};
 
 constexpr FwLayout fw_shape_layout(const fw_env_t& e, const fw_sim_t& s) {
   FwLayout L{};
-  fw_layout_build(e, s.scale_actions, 0, L);
+  fw_layout_build(e, s.scale_actions, 0, L, s.turb_mixed);
   return L;
 }
 
@@ -36,6 +43,7 @@ constexpr FwLayout fw_shape_layout(const fw_env_t& e, const fw_sim_t& s) {
   __device__ const FwLayout kShapeLay_##NAME = fw_shape_layout(fw_shape_env_##NAME(), fw_shape_sim_##NAME()); \
   struct FwShape_##NAME {                                                                                  \
     static constexpr bool fixed = true;                                                                    \
+    static constexpr bool mixed = fw_shape_sim_##NAME().turb_mixed != 0;                                   \
     static constexpr fw_env_t cenv = fw_shape_env_##NAME();   /* for constant expressions (loop trip counts) */ \
     static __device__ __forceinline__ const fw_env_t& env(const fw_env_t&) { return kShapeEnv_##NAME; }    \
     static __device__ __forceinline__ const fw_sim_t& sim(const fw_sim_t&) { return kShapeSim_##NAME; }    \
@@ -117,7 +125,8 @@ inline bool fw_env_same_shape(const fw_env_t& a, const fw_env_t& b) {
   return true;
 }
 inline bool fw_sim_same_shape(const fw_sim_t& a, const fw_sim_t& b) {
-  if (a.drag_model != b.drag_model || a.turbulence != b.turbulence || a.wind_enabled != b.wind_enabled ||
+  if (a.drag_model != b.drag_model || a.turbulence != b.turbulence || a.turb_mixed != b.turb_mixed ||
+      a.wind_enabled != b.wind_enabled ||
       a.scale_actions != b.scale_actions || a.has_scale_low != b.has_scale_low || a.has_scale_high != b.has_scale_high)
     return false;
   for (int f = 0; f < FW_N_FILT; ++f)

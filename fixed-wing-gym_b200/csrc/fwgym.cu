@@ -474,7 +474,7 @@ template <class SH>
 __device__ __forceinline__ void fw_commit_step(const fw_sim_t& P, const FwEnvCtx& c, const double* __restrict__ cd,
                                                const int32_t* __restrict__ ci, int64_t stride, uint32_t k0, uint32_t k1,
                                                uint32_t genv, const FwTurbInject ti, const double* un_pre,
-                                               int& attempts_out, int& accepted_out) {
+                                               int& attempts_out, int& accepted_out, int tlvl = 0) {
   const fw_sim_t& Ps = SH::sim(P);
 #define FW_CS(SV, X) fw_cond_s<false>(Ps.var[SV].flags, P.var[SV], SV, X, failv)
 #define FW_CSW(SV, X) fw_cond_s<true>(Ps.var[SV].flags, P.var[SV], SV, X, failv)
@@ -537,12 +537,13 @@ __device__ __forceinline__ void fw_commit_step(const fw_sim_t& P, const FwEnvCtx
       c.D(D_ROLL) = roll; c.D(D_PITCH) = pitch; c.D(D_YAW) = yaw;
       c.D(D_VA) = Va; c.D(D_ALPHA) = alpha; c.D(D_BETA) = beta;
       c.D(D_ELEV) = elev; c.D(D_AIL) = ail;
-      if (Ps.turbulence) {   // gust column for the next sim step (cur_sim_step + 1)
+      // gust column for the next sim step (cur_sim_step + 1); a mixed handle's level-0 episodes keep their zero gusts
+      if (SH::mixed ? tlvl != 0 : Ps.turbulence != 0) {
         double un[4];
         if (ti.noise && ((uint32_t)c.I(I_FLAGS) & FWF_TURB_INJ)) fw_turb_noise_injected(P, ti, c.env, c.I(I_STEPS) + 1, un);
         else if (un_pre) { un[0] = un_pre[0]; un[1] = un_pre[1]; un[2] = un_pre[2]; un[3] = un_pre[3]; }
         else fw_turb_noise<SH::fixed>(P, k0, k1, genv, (uint32_t)c.I(I_EPTICK), c.I(I_STEPS) + 1, un);
-        fw_turb_advance<SH>(P, c, un);
+        fw_turb_advance<SH>(P, c, un, tlvl);
       }
     }
   }
@@ -618,7 +619,7 @@ __device__ __forceinline__ void fw_env_step(const fw_env_t& E, const fw_sim_t& P
   FW_SHAPE_REFS;
   FwEnvCtx c{a.d, a.i, L.stride, env};
   fw_commit_step<SH>(P, c, a.cd + env, a.ci + env, L.stride, a.k0, a.k1, a.env_offset + (uint32_t)env, a.ti,
-                     pre.have_un ? pre.un : nullptr, attempts, accepted);
+                     pre.have_un ? pre.un : nullptr, attempts, accepted, SH::mixed ? c.I(Ls.tl_row + 1) : 0);
   failed = c.I(I_STATUS) != 0;
   uint32_t flags = (uint32_t)c.I(I_FLAGS);
   int steps = c.I(I_STEPS);
@@ -929,6 +930,18 @@ fw_reset_kernel(const __grid_constant__ fw_env_t E, const __grid_constant__ fw_s
   fw_reset_env<SH>(E, P, L, c, a.k0, a.k1, a.env_offset + (uint32_t)env, a.init_state, a.init_target, a.n, a.ti, ow);
 }
 
+// Kernel parameters are limited to 32 764 bytes (CUDA 12.1+ on Volta and later).  The configuration travels as
+// __grid_constant__ parameters, so its size is bounded here (the per-level Dryden tables of fw_sim_t count against it);
+// 64 bytes cover the alignment padding between the parameters.
+static_assert(sizeof(fw_env_t) + sizeof(fw_sim_t) + sizeof(FwLayout) + sizeof(FwEnvArgs) + 64 <= 32764,
+              "env kernel parameters exceed the 32 764-byte limit");
+static_assert(sizeof(fw_env_t) + sizeof(fw_sim_t) + sizeof(FwLayout) + sizeof(FwResetArgs) + 64 <= 32764,
+              "reset kernel parameters exceed the 32 764-byte limit");
+static_assert(sizeof(FwSimX) + sizeof(FwDynArgs) + 64 <= 32764, "fp32 dynamics kernel parameters exceed the 32 764-byte limit");
+static_assert(sizeof(fw_sim_t) + sizeof(FwDynArgs) + 64 <= 32764, "fp64 dynamics kernel parameters exceed the 32 764-byte limit");
+// the per-level Dryden tables were appended without moving any later kernel parameter off its 16-byte alignment
+static_assert(sizeof(fw_sim_t) % 32 == 24 && sizeof(FwLayout) % 16 == 8, "see fw_sim_t._pad_turb / FwLayout._pad_tl");
+
 // ---- shape dispatch: index into FW_SHAPE_LIST (fw_find_shape), -1 = generic -----------------------------------------
 // overlap != 0: programmatic dependent launch - the kernel may start while the preceding kernel of the stream (the
 // attempt kernel) is still running; it synchronises on the per-chunk counters
@@ -953,6 +966,7 @@ static cudaError_t launch_env(int shape, int grid, cudaStream_t s, int overlap, 
 #define FW_LAUNCH_SHAPE(NAME) if (shape == idx++) return launch_env_t<FwShape_##NAME>(grid, s, overlap, E, P, L, a);
   FW_SHAPE_LIST(FW_LAUNCH_SHAPE)
 #undef FW_LAUNCH_SHAPE
+  if (P.turb_mixed) return launch_env_t<FwShapeGenericMixed>(grid, s, overlap, E, P, L, a);
   return launch_env_t<FwShapeGeneric>(grid, s, overlap, E, P, L, a);
 }
 static cudaError_t launch_reset(int shape, int grid, cudaStream_t s, const fw_env_t& E, const fw_sim_t& P,
@@ -962,7 +976,8 @@ static cudaError_t launch_reset(int shape, int grid, cudaStream_t s, const fw_en
   if (shape == idx++) { fw_reset_kernel<FwShape_##NAME><<<grid, FW_ENV_BLOCK, 0, s>>>(E, P, L, a); return cudaGetLastError(); }
   FW_SHAPE_LIST(FW_LAUNCH_SHAPE)
 #undef FW_LAUNCH_SHAPE
-  fw_reset_kernel<FwShapeGeneric><<<grid, FW_ENV_BLOCK, 0, s>>>(E, P, L, a);
+  if (P.turb_mixed) fw_reset_kernel<FwShapeGenericMixed><<<grid, FW_ENV_BLOCK, 0, s>>>(E, P, L, a);
+  else fw_reset_kernel<FwShapeGeneric><<<grid, FW_ENV_BLOCK, 0, s>>>(E, P, L, a);
   return cudaGetLastError();
 }
 static const char* shape_name(int shape) {
@@ -1020,6 +1035,13 @@ __global__ void fw_import_kernel(double* d, int32_t* i, int64_t stride, int64_t 
   for (int r = 0; r < rows_d; ++r) d[(int64_t)r * stride + env] = in[(int64_t)r * n + env];
   for (int r = 0; r < rows_i; ++r) i[(int64_t)r * stride + env] = (int32_t)(long long)in[(int64_t)(rows_d + r) * n + env];
 }
+// requested Dryden levels of a mixed handle (fw_set_turbulence_levels); NULL or a value outside -1..3 = -1 (draw)
+__global__ void fw_set_levels_kernel(int32_t* row, int64_t n, const int32_t* __restrict__ levels) {
+  const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (env >= n) return;
+  const int32_t v = levels ? levels[env] : -1;
+  row[env] = (v < -1 || v > 3) ? -1 : v;
+}
 __global__ void fw_gather_i32_kernel(const int32_t* i, int64_t stride, int64_t n, int row, int32_t* out) {
   const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (env < n) out[env] = i[(int64_t)row * stride + env];
@@ -1042,7 +1064,9 @@ __global__ void __launch_bounds__(256) fw_dfma_kernel(double* out, int iters, do
 
 // ------------------------------------------------------------------------------------------------------- host side
 static int make_layout(const fw_config_t& cfg, int64_t n, FwLayout& L) {
-  const int rc = fw_layout_build(cfg.env, cfg.sim.scale_actions, n, L);
+  if (cfg.sim.turb_mixed && !cfg.sim.turbulence)
+    return fail(FW_ERR_CONFIG, "per-env turbulence levels (turb_mixed) need turbulence on");
+  const int rc = fw_layout_build(cfg.env, cfg.sim.scale_actions, n, L, cfg.sim.turb_mixed);
   if (rc) return fail(FW_ERR_CONFIG, "%s", fw_layout_error(rc));
   return FW_OK;
 }
@@ -1237,6 +1261,8 @@ int fw_create(const fw_config_t* cfg, int64_t n_envs, int64_t global_env_offset,
   }
   CK(cudaMemset(h->d, 0, db));
   CK(cudaMemset(h->i, 0, ib));
+  if (h->L.n_tl_rows)   // requested levels start at -1: every env draws its level at each reset
+    CK(cudaMemset(h->i + (size_t)h->L.tl_row * h->L.stride, 0xff, (size_t)h->L.stride * sizeof(int32_t)));
   CK(cudaMemset(h->ctr, 0, CTR_N * sizeof(unsigned long long)));
   CK(cudaMemset(h->msum, 0, FW_N_METRIC_SUMS * sizeof(double)));
   h->generic = needs_generic(h->cfg.sim);
@@ -1375,6 +1401,8 @@ const char* fw_state_row_name(fw_handle h, int64_t r) {
   if (r < h->L.d_rows) return "ring";
   r -= h->L.d_rows;
   if (r < I_GOALRING) return in[r];
+  if (h->L.n_tl_rows && r == h->L.tl_row) return "turb_level_req";
+  if (h->L.n_tl_rows && r == h->L.tl_row + 1) return "turb_level";
   if (r < h->L.i_rows) return in[I_GOALRING];
   return nullptr;
 }
@@ -1643,6 +1671,18 @@ int fw_set_state(fw_handle h, const double* in, void* stream) {
   const int grid = (int)((h->n + 255) / 256);
   fw_import_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->d, h->i, h->L.stride, h->n, h->L.d_rows, h->L.i_rows, in);
   CK(cudaMemsetAsync(h->queue, 0, (size_t)h->q_len * sizeof(int32_t), (cudaStream_t)stream));   // re-arm the step queue
+  CK(cudaGetLastError());
+  return FW_OK;
+}
+
+int fw_set_turbulence_levels(fw_handle h, const int32_t* levels, void* stream) {
+  if (!h) return fail(FW_ERR_ARG, "null handle");
+  if (!h->L.n_tl_rows)
+    return fail(FW_ERR_ARG, "fw_set_turbulence_levels: the handle flies one turbulence intensity (configure "
+                            "turbulence_intensity as {\"values\": [...], \"probabilities\": [...]})");
+  CK(cudaSetDevice(h->device));
+  const int grid = (int)((h->n + 255) / 256);
+  fw_set_levels_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->i + (size_t)h->L.tl_row * h->L.stride, h->n, levels);
   CK(cudaGetLastError());
   return FW_OK;
 }

@@ -67,6 +67,10 @@ struct FwLayout {
   int32_t par_row, n_par_rows;
   // per-env reward scalings (reward.randomize_scaling): n_rs_rows rows starting at rs_row
   int32_t rs_row, n_rs_rows;
+  // per-env Dryden intensity (only when fw_sim_t.turb_mixed): int32 rows tl_row (requested level, -1 = draw at every
+  // reset) and tl_row + 1 (level of the running episode); n_tl_rows = 0 or 2.  (_pad_tl: the struct grows by 16 bytes,
+  // so the kernel parameters after it keep their 16-byte alignment and the compiler its 128-bit constant loads.)
+  int32_t tl_row, n_tl_rows, _pad_tl[2];
 };
 
 // metric accumulators, relative to FwLayout.m_drow (double) / m_irow (int32); k = target index
@@ -80,7 +84,7 @@ enum { EP_RETURN = 0, EP_LENGTH, EP_CV, EP_SUCCESS_ALL, EP_SETTLE_ALL, EP_STF_AL
 // Layout of the variable part.  constexpr so that the SAME function sizes a handle on the host (make_layout, fwgym.cu)
 // and folds the row numbers of a compile-time configuration shape into the specialised env kernels (env_shapes.h).
 // Returns 0 or a 1-based error number (messages: fw_layout_error).
-constexpr int fw_layout_build(const fw_env_t& E, int scale_actions, int64_t n, FwLayout& L) {
+constexpr int fw_layout_build(const fw_env_t& E, int scale_actions, int64_t n, FwLayout& L, int turb_mixed = 0) {
   L = FwLayout{};
   L.n = n;
   L.stride = (n + 31) / 32 * 32;
@@ -131,6 +135,7 @@ constexpr int fw_layout_build(const fw_env_t& E, int scale_actions, int64_t n, F
     L.end_row = row; row += FW_END_WINDOW * E.n_targets;
     L.m_irow = L.i_rows; L.i_rows += MI_GRING + 3 * L.goal_words;
   }
+  if (turb_mixed) { L.tl_row = L.i_rows; L.n_tl_rows = 2; L.i_rows += 2; }
   if (E.n_rand < 0 || E.n_rand > FW_MAX_RAND || E.n_par_rows < 0 || E.n_par_rows > FW_N_PAR) return 6;
   L.par_row = row;
   L.n_par_rows = E.n_par_rows;

@@ -15,6 +15,7 @@
 #define FW_RS_TURB 2    // Dryden white noise; tick = episode tick, index = 2*sim_step + {0,1}
 #define FW_RS_ENV_U 3   // env-side uniform draws in call order (target sampling, init noise)
 #define FW_RS_ENV_N 4   // env-side normal draws in call order (observation noise), two per block
+#define FW_RS_TURBLVL 5 // Dryden intensity of a mixed handle's episode (one uniform at the reset's tick, index 0)
 
 // Two forms of every generator.  INL = false (generic, table-walking env kernels): out of line on purpose, ~100
 // instructions x ~25 call sites would otherwise dominate that kernel's code size.  INL = true (shape-specialised

@@ -103,28 +103,41 @@ def load_test_set(path):
 
 
 def evaluate_on_set(scenarios, config_path, controller="pid", config_kw=None, metrics=DEFAULT_METRICS,
-                    turbulence_intensity="none", device="cuda:0", seed=0, max_steps=None):
+                    turbulence_intensity="none", device="cuda:0", seed=0, max_steps=None, env_offset=0):
     """Run every scenario once (in parallel) under `controller`: "pid", a dict of saved MlpPolicy arrays
     (MlpController), or a callable(vec) -> actions tensor.
-    Returns (res, vec_env): res[metric][state] lists in scenario order, res["rewards"], res["lengths"]."""
-    n = len(scenarios)
+    Returns (res, vec_env): res[metric][state] lists in scenario order, res["rewards"], res["lengths"].
+    `turbulence_intensity`: one level ("none", "light", "moderate", "severe"), or a list of levels: then the S
+    scenarios x L levels fly as ONE batch of L * S envs on a handle with per-env intensities (env j * S + i is scenario i
+    at level j, pinned with set_turbulence_intensity) and the first element of the return value is {level: res}.
+    `env_offset`: global id of the first env (the Philox streams are keyed by it)."""
+    levels = None if isinstance(turbulence_intensity, str) else list(turbulence_intensity)
+    n_scen = len(scenarios)
+    n = n_scen if levels is None else n_scen * len(levels)
     kw = dict(config_kw or {})
     for k, v in EVAL_CONFIG_KW.items():
         kw[k] = v
     if controller == "pid":
         kw["action"] = {"scale_space": False}          # evaluate_controller.py:78-79
-    sim_kw = {"turbulence": turbulence_intensity != "none", "turbulence_intensity": turbulence_intensity}
+    if levels is None:
+        sim_kw = {"turbulence": turbulence_intensity != "none", "turbulence_intensity": turbulence_intensity}
+    else:
+        sim_kw = {"turbulence": True, "turbulence_intensity": {"values": levels}}
     vec = FixedWingVecEnv(config_path, n, device=device, config_kw=kw, sim_config_kw=sim_kw, seed=seed, metrics=True,
-                          auto_reset=True)
+                          auto_reset=True, env_offset=env_offset)
+    if levels is not None:
+        vec.set_turbulence_intensity([lv for lv in levels for _ in range(n_scen)])
+    reps = 1 if levels is None else len(levels)
     skeys = sorted(scenarios[0]["state"].keys())
     state = {}
     for k in skeys:
         v0 = scenarios[0]["state"][k]
         if isinstance(v0, (list, tuple, np.ndarray)):     # "wind": [n, e, d]
-            state[k] = np.array([s["state"][k] for s in scenarios], dtype=np.float64).T
+            state[k] = np.tile(np.array([s["state"][k] for s in scenarios], dtype=np.float64).T, (1, reps))
         else:
-            state[k] = np.array([s["state"][k] for s in scenarios], dtype=np.float64)
-    target = {k: np.array([s["target"][k] for s in scenarios], dtype=np.float64) for k in scenarios[0]["target"]}
+            state[k] = np.tile(np.array([s["state"][k] for s in scenarios], dtype=np.float64), reps)
+    target = {k: np.tile(np.array([s["target"][k] for s in scenarios], dtype=np.float64), reps)
+              for k in scenarios[0]["target"]}
     vec.enable_f64_outputs(True)
     vec.reset(state=state, target=target)
     pid = DevicePID(vec) if controller == "pid" else None
@@ -152,22 +165,28 @@ def evaluate_on_set(scenarios, config_path, controller="pid", config_kw=None, me
             alive = alive & ~fin
             if not alive.any():
                 break
-    cols = vec.episode_columns()
-    rows = ep_rows.cpu().numpy()
+    lengths[alive] = min(t + 1, steps_cap)
+    rows, tr, ln = ep_rows.cpu().numpy(), rew_trace.cpu().numpy(), lengths.cpu().numpy()
+    if levels is None:
+        return _results(vec, metrics, rows, tr, ln), vec
+    return {lv: _results(vec, metrics, rows[j * n_scen:(j + 1) * n_scen], tr[:, j * n_scen:(j + 1) * n_scen],
+                         ln[j * n_scen:(j + 1) * n_scen]) for j, lv in enumerate(levels)}, vec
+
+
+def _results(vec, metrics, rows, tr, ln):
+    """res[metric][state] lists, rewards, lengths and episode rows of one block of envs (in env order)."""
     res = {m: {} for m in metrics}
-    for i in range(n):
+    for i in range(len(ln)):
         if not np.isfinite(rows[i][1]):
-            continue                       # still flying at max_steps: no episode row, length = max_steps below
+            continue                       # still flying at max_steps: no episode row, length = max_steps
         info = vec.episode_info(rows[i])
         for m in metrics:
             for st, val in info.get(m, {}).items():
                 res[m].setdefault(st, []).append(val)
-    lengths[alive] = min(t + 1, steps_cap)
-    tr, ln = rew_trace.cpu().numpy(), lengths.cpu().numpy()
-    res["rewards"] = [tr[:ln[i], i].copy() for i in range(n)]
+    res["rewards"] = [tr[:ln[i], i].copy() for i in range(len(ln))]
     res["lengths"] = ln
-    res["episode_rows"], res["episode_columns"] = rows, cols
-    return res, vec
+    res["episode_rows"], res["episode_columns"] = rows, vec.episode_columns()
+    return res
 
 
 def summarise(res, metrics=DEFAULT_METRICS):

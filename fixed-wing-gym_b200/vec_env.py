@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import _capi
-from .config import CompiledConfig
+from .config import TURB_LEVELS, CompiledConfig
 
 TERM_NAMES = {0: None, 1: "steps", 2: "success", 3: "numeric"}
 N_INIT_ROWS = _capi.DEFINES["FW_N_SV"] + 3
@@ -390,6 +390,56 @@ class FixedWingVecEnv:
             return torch.empty((self.num_envs, 0), dtype=torch.float64, device=self.device)
         return torch.stack(cols, dim=1)
 
+    # ------------------------------------------------------------------------ per-env Dryden turbulence intensity
+    def set_turbulence_intensity(self, levels, indices=None):
+        """Pin the Dryden intensity of envs (all, or `indices`) from their next reset on (explicit or automatic; the
+        running episodes keep theirs).  `levels`: a level name ("none", "light", "moderate", "severe"), a list of names
+        (one per selected env), or an int array / tensor of levels 0..3, where -1 goes back to drawing from the handle's
+        distribution at every reset.  Needs a mixed handle: sim_config_kw turbulence_intensity =
+        {"values": [...], "probabilities": [...]}."""
+        if not self.cc.turbulence_mix:
+            raise _capi.FwError("set_turbulence_intensity needs per-env levels: configure turbulence_intensity as "
+                                "{\"values\": [...], \"probabilities\": [...]}")
+        idx = None if indices is None else torch.as_tensor(np.atleast_1d(indices), dtype=torch.long, device=self.device)
+        count = self.num_envs if idx is None else len(idx)
+
+        def code(name):
+            if name not in TURB_LEVELS:
+                raise ValueError("unknown turbulence level %r (levels: %s)" % (name, ", ".join(TURB_LEVELS)))
+            return TURB_LEVELS.index(name)
+        if isinstance(levels, str):
+            lv = torch.full((count,), code(levels), dtype=torch.int32, device=self.device)
+        elif isinstance(levels, (list, tuple)) and levels and all(isinstance(x, str) for x in levels):
+            lv = torch.as_tensor([code(x) for x in levels], dtype=torch.int32, device=self.device)
+        else:
+            lv = torch.as_tensor(np.asarray(levels.cpu() if torch.is_tensor(levels) else levels), device=self.device)
+            if lv.dtype.is_floating_point or lv.dtype == torch.bool:
+                raise ValueError("turbulence levels must be names or integers -1..3")
+            lv = lv.to(torch.int32).reshape(-1)
+            if lv.numel() == 1 and count != 1:
+                lv = lv.expand(count)
+            if bool(((lv < -1) | (lv > 3)).any()):
+                raise ValueError("turbulence levels must be in -1..3")
+        if lv.numel() != count:
+            raise ValueError("%d turbulence levels for %d envs" % (lv.numel(), count))
+        req = self.get_rows(self.state_rows().index("turb_level_req"), 1)[0].to(torch.int32)
+        if idx is None:
+            req[:] = lv
+        else:
+            req[idx] = lv
+        _capi.check(self._lib.fw_set_turbulence_levels(self._h, self._ptr(req), self._stream()))
+        self._turb_req_keepalive = req
+
+    def turbulence_levels(self):
+        """Device int32 [N]: the Dryden level of every env's running episode (0 none, 1 light, 2 moderate, 3 severe).
+        A handle without per-env levels reports its single intensity for every env."""
+        rows = self.state_rows()
+        if "turb_level" in rows:
+            return self.get_rows(rows.index("turb_level"), 1)[0].to(torch.int32)
+        sc = self.cc.sim_cfg
+        lvl = TURB_LEVELS.index(sc.get("turbulence_intensity") or "light") if sc["turbulence"] else 0
+        return torch.full((self.num_envs,), lvl, dtype=torch.int32, device=self.device)
+
     def kernel_variant(self):
         """Which kernel instantiations the configuration selected, e.g. "dyn=shipped env=default_turb"."""
         return self._lib.fw_kernel_variant(self._h).decode()
@@ -429,6 +479,10 @@ class FixedWingVecEnv:
             return [int(sc[i]) for i in ids]
         if name == "simulator":
             return [SimulatorView(self)] * n
+        if name == "turbulence_intensity":
+            lv = self.turbulence_levels().cpu().numpy()
+            ids = range(self.num_envs) if indices is None else np.atleast_1d(indices)
+            return [TURB_LEVELS[int(lv[i])] for i in ids]
         return [getattr(self, name)] * n
 
     def set_attr(self, name, value, indices=None):

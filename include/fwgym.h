@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define FW_ABI_VERSION 10
+#define FW_ABI_VERSION 11
 
 /* ---------------------------------------------------------------------------------------------- limits */
 #define FW_MAX_OBS_VARS 32
@@ -36,6 +36,7 @@ extern "C" {
 #define FW_FILT_MAXN 3
 #define FW_N_PAR 53           /* == FW_PAR_N below (model parameters that can differ per env) */
 #define FW_MAX_RAND 64        /* entries of simulator-parameter randomisation per reset */
+#define FW_N_TURB_LEVELS 4    /* Dryden intensities of a mixed handle: 0 none, 1 light, 2 moderate, 3 severe */
 
 /* PyFly state-variable ids (order of oracle/pyfly_restated.py REQUIRED_VARIABLES + elevons) */
 enum fw_sv {
@@ -171,6 +172,18 @@ typedef struct {
   /* per-env model parameters (simulator-parameter randomisation): par_slot1[id] = 1 + row (relative to the handle's
    * parameter rows) holding that parameter for every env, 0 = the same for all envs (the value above) */
   int32_t par_slot1[FW_N_PAR];
+  /* per-env Dryden intensity ("mixed" handle, sim_config_kw turbulence_intensity = {"values", "probabilities"}).  Ad /
+   * Bd0 / Bd1 of filt[] do not depend on the intensity; the output rows C / D do, one set per level (level 0 = none is
+   * all zero).  An env's level is chosen at its reset: its requested level (fw_set_turbulence_levels) when >= 0, else
+   * the first l with u < turb_cdf[l] for one uniform u of Philox stream FW_RS_TURBLVL.  0 everywhere when not mixed. */
+  int32_t turb_mixed, _pad;
+  double turb_cdf[FW_N_TURB_LEVELS];
+  double turb_C[FW_N_TURB_LEVELS][FW_N_FILT][FW_FILT_MAXN];
+  double turb_D[FW_N_TURB_LEVELS][FW_N_FILT];
+  /* keeps sizeof(fw_sim_t) congruent to its earlier size (ABI 10) modulo 32, so every kernel parameter after it, also
+   * behind the float image of the fp32 dynamics kernels (1.5x), keeps its 16-byte alignment and the compiler its
+   * 128-bit constant loads: the kernels of existing configurations compile to the same instructions */
+  double _pad_turb[3];
 } fw_sim_t;
 
 /* One draw of FixedWingAircraft.sample_simulator_parameters (fixed_wing.py:523-570), in the reference's order.
@@ -292,6 +305,13 @@ int fw_host_close(fw_handle h);
 int fw_host_submit(fw_handle h, const float* actions_host, void* stream, int* slot_out);
 int fw_host_wait(fw_handle h, int slot, const float** obs, const float** rew, const uint8_t** done,
                  const int32_t** term);
+
+/* Per-env Dryden intensity of a mixed handle (fw_sim_t.turb_mixed): levels = device int32 [N], -1 = draw from the
+ * handle's distribution at every reset, 0..3 = pinned (none, light, moderate, severe), any other value counts as -1;
+ * NULL sets every env to -1.  Takes
+ * effect at each env's next reset (explicit or automatic).  FW_ERR_ARG on a handle that is not mixed.  The requested
+ * and active levels are the state rows "turb_level_req" / "turb_level" (fw_get_state / fw_set_state). */
+int fw_set_turbulence_levels(fw_handle h, const int32_t* levels, void* stream);
 
 /* Rows [row0, row0 + nrows) of the state matrix below: device double [nrows, N] (e.g. the three target rows without
  * exporting the whole state). */
