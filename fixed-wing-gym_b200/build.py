@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc", "fwgym.cu")
 OUT = os.path.join(HERE, "libfwgym.so")
-DEPS = [os.path.join(HERE, "csrc", f) for f in ("fwgym.cu", "attempt_pair.cuh", "dynamics.cuh", "env.cuh", "philox.cuh", "layout.h", "fwmath.cuh", "env_shapes.h",
+DEPS = [os.path.join(HERE, "csrc", f) for f in ("fwgym.cu", "dynamics.cuh", "env.cuh", "philox.cuh", "layout.h", "fwmath.cuh", "env_shapes.h",
                                                     "env_shapes_gen.h")] + [
     os.path.join(HERE, "..", "include", "fwgym.h")]
 

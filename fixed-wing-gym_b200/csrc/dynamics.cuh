@@ -421,16 +421,12 @@ __device__ __forceinline__ constexpr int fw_kc_to_ode(int kc) { return kc < 7 ? 
 // conflict-free.
 template <typename T, int BLOCK> struct FwKStore {
   T* base;
-#ifndef FW_K_SINGLE
   // components in pairs, [slot][pair][thread][2]: the unrolled stage code reads / writes two components per 16-byte
   // access (LDS.128 / STS.128, 512 B per warp instruction, conflict-free) - half the shared-memory instructions of the
-  // [slot][component][thread] layout (round 2: dynamics kernels 143.2 -> 139.2 us; -DFW_K_SINGLE restores it for A/B)
+  // [slot][component][thread] layout (round 2: dynamics kernels 143.2 -> 139.2 us)
   __device__ __forceinline__ T& at(int slot, int kc) {
     return base[((slot * (FW_N_KC / 2) + (kc >> 1)) * BLOCK + threadIdx.x) * 2 + (kc & 1)];
   }
-#else
-  __device__ __forceinline__ T& at(int slot, int kc) { return base[(slot * FW_N_KC + kc) * BLOCK + threadIdx.x]; }
-#endif
 };
 
 // Stage state of stage S_ for the 16 stored components: ys = y + h * sum_{j < S_} a_{S_ j} K_j, accumulated exactly as
@@ -564,28 +560,11 @@ __device__ __forceinline__ void fw_ivp_attempt(const fw_sim_t& P, const PAR& PP,
   T accB[3], accE[3];    // running B-row / E-row sums of the position components (never stored as K stages)
 #pragma unroll
   for (int j = 0; j < 3; ++j) { accB[j] = fw_dpA<T>(6, 0) * S.k0pos[j]; accE[j] = fw_dpE<T>(0) * S.k0pos[j]; }
-#ifdef FW_FLAT_PASS
-  // experiment build: the six stages as ONE straight-line block (six copies of the right-hand side); a constraint
-  // violation is recorded (first stage wins, as the raise would) and acted on after the last stage instead of branching
-  // out, so that the scheduler may fill the tail of one stage's dependency chain with the next stage's partial sums
-  uint32_t failmask_first = 0u;
-#pragma unroll
-#else
 #pragma unroll 1
-#endif
   for (int s = 1; s <= 6; ++s) {
     T ys[FW_N_ODE], f[FW_N_ODE];
     {
       // y_s = y + h * sum_j a_sj K_j, accumulated as y += (h a_sj) K_j (one fma per term, no separate scaling pass)
-#ifdef FW_COMBINE_LOOP   // experiment build: the former run-time loop over the terms
-#pragma unroll
-      for (int kc = 0; kc < FW_N_KC; ++kc) ys[fw_kc_to_ode(kc)] = S.y[fw_kc_to_ode(kc)];
-      for (int j = 0; j < s; ++j) {
-        const T ha = h * fw_dpA<T>(s, j);
-#pragma unroll
-        for (int kc = 0; kc < FW_N_KC; ++kc) ys[fw_kc_to_ode(kc)] = fma(ha, K.at(j, kc), ys[fw_kc_to_ode(kc)]);
-      }
-#else
       switch (s) {
         case 1: fw_stage_state<T, BLOCK, 1>(S.y, h, K, ys); break;
         case 2: fw_stage_state<T, BLOCK, 2>(S.y, h, K, ys); break;
@@ -594,27 +573,17 @@ __device__ __forceinline__ void fw_ivp_attempt(const fw_sim_t& P, const PAR& PP,
         case 5: fw_stage_state<T, BLOCK, 5>(S.y, h, K, ys); break;
         default: fw_stage_state<T, BLOCK, 6>(S.y, h, K, ys); break;
       }
-#endif
       // position stage states are never read by the RHS; y_new[pos] is formed from accB when s == 6
 #pragma unroll
       for (int j = 0; j < 3; ++j) ys[7 + j] = S.y[7 + j] + h * accB[j];
     }
     uint32_t failmask = 0u;
     fw_rhs<T, Spec>(P, PP, in, ys, f, failmask);
-#ifdef FW_FLAT_PASS
-    failmask_first = failmask_first ? failmask_first : failmask;
-    if (s == 6 && failmask_first) {
-      S.fail = fw_fail_code<T>(failmask_first);
-      S.status = FW_STATUS_FINISHED;
-      return;
-    }
-#else
     if (failmask) {
       S.fail = fw_fail_code<T>(failmask);
       S.status = FW_STATUS_FINISHED;
       return;
     }
-#endif
     if (s < 6) {
 #pragma unroll
       for (int kc = 0; kc < FW_N_KC; ++kc) K.at(s, kc) = f[fw_kc_to_ode(kc)];

@@ -68,10 +68,7 @@ struct fw_handle_s {
   int32_t* long_list;            // [stride]
   int32_t* queue;                // [Q_N]
   int attempt_grid;              // persistent warps of the attempt kernel (resident capacity of the device)
-  int pair;                      // fp64 attempt kernel with two warps per 32 aircraft (attempt_pair.cuh; FWGYM_PAIR=1, off by default: measured slower)
-  int pair_grid;                 // its persistent blocks
   double long_div, long_h;       // priority threshold on the initial step size: long_h = dt / long_div
-  double long_omega;             // priority threshold on max |omega| in rad/s (FWGYM_LONG_OMEGA, 0 = off)
   std::vector<cudaEvent_t> ev;   // 3 events per profiled step: before dyn, between, after env
   // host-buffer pipeline (fw_host_*): `depth` slots of device staging + pinned host result buffers, copy streams
   struct HostSlot {
@@ -158,15 +155,16 @@ struct FwDynArgs {
   int32_t* long_list;  // [stride] aircraft to start first
   int32_t* q;          // [Q_N + chunks] queue counters + per-chunk finished counters; all zero between steps (fw_init_kernel)
   double long_h;       // initial step sizes below this go on the priority list
-  double long_omega;   // ... and aircraft whose largest body rate (rad/s) exceeds this
   int32_t par_row;     // first per-env model-parameter row of d (FwSpecRand)
   int32_t n_par_rows;
   const int32_t* order;   // experiment hook (fw_debug_set_order): adoption order of the natural queue, NULL = identity
   int32_t pdl;            // the attempt kernel was launched as a programmatic dependent of the init kernel
-  int32_t pair;           // host only: launch fw_attempt_pair_kernel with pair_grid blocks
-  int32_t pair_grid;
-  int32_t pair_mix;       // alternate which warp of a block plays role T (FWGYM_PAIR_MIX, default on)
+  // ptxas allocates the attempt kernels' registers differently when this block changes size (at 120 or 128 bytes: fp64
+  // FwSpecRand 253 -> 254 registers, fp32 FwSpecShipped 127 -> 128, fp32 FwSpecRand spills 60/56 -> 66/68 bytes):
+  // padded to the 136 bytes they were tuned at
+  int32_t _pad[5];
 };
+static_assert(sizeof(FwDynArgs) == 136, "see FwDynArgs._pad");
 
 // ---- action -> actuator commands (fixed_wing.py:349-354,439-459; Actuation.set_and_constrain_commands) ----
 __device__ __forceinline__ void fw_commands(const fw_sim_t& P, const FwDynArgs& a, const FwEnvCtx& c, double (&cmd)[3]) {
@@ -214,11 +212,7 @@ template <typename T, class Spec>
 #ifndef FW_INIT_MIN_BLOCKS
 #define FW_INIT_MIN_BLOCKS 8   // 128 registers: one wave at 65536 envs (1024 blocks on 148 x 8 slots); 4 -> 8: init 18 -> 13 us
 #endif
-#ifdef FW_INIT_MAXNREG   // experiment build: a register cap instead of launch bounds
-__global__ void __maxnreg__(FW_INIT_MAXNREG)
-#else
 __global__ void __launch_bounds__(FW_INIT_BLOCK, FW_INIT_MIN_BLOCKS)
-#endif
 fw_init_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const FwDynArgs a) {
   const fw_sim_t& P = fw_sim_of(Px);
   FW_TL_BEGIN(0);
@@ -253,12 +247,9 @@ fw_init_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const FwDy
     for (int kc = 0; kc < FW_N_KC; ++kc) cd[(CY_K0 + kc) * a.stride] = (double)f0[fw_kc_to_ode(kc)];
 #pragma unroll
     for (int j = 0; j < 3; ++j) { cd[(CY_KP + j) * a.stride] = (double)f0[7 + j]; cd[(CY_CMD + j) * a.stride] = cmd[j]; }
-    // Priority start (DESIGN.md 4.4): a tiny first step (the 1e-6 start after a reset) or, when FWGYM_LONG_OMEGA is
-    // set, fast body rates (85 % of the aircraft that go on to need >= 12 attempts rotate faster than 3 rad/s about some
-    // axis at the start of the step, 17 % of all do; measured: no gain, off by default).  Membership is carried by the
+    // Priority start (DESIGN.md 4.4): a tiny first step (the 1e-6 start after a reset).  Membership is carried by the
     // SIGN of the parked step size, so the attempt kernel's natural-order visit can skip list members without a load.
-    const double wmax = fmax(fabs((double)y[4]), fmax(fabs((double)y[5]), fabs((double)y[6])));
-    is_long = !failv && (double)h_abs > 0.0 && ((double)h_abs < a.long_h || wmax > a.long_omega);
+    is_long = !failv && (double)h_abs > 0.0 && (double)h_abs < a.long_h;
     cd[CY_H * a.stride] = is_long ? -(double)h_abs : (double)h_abs;
     ci[CI_FAIL * a.stride] = failv;     // != 0: ConstraintException inside RK45.__init__; nothing left to integrate
     ci[CI_ATTEMPTS * a.stride] = 0;
@@ -284,11 +275,7 @@ fw_init_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const FwDy
 
 // fp32 aircraft need half the registers and half the K-stage shared memory: twice the resident warps
 template <typename T, class Spec>
-#ifdef FW_DYN_MAXNREG   // experiment build: a register cap instead of launch bounds (e.g. 224 = 9 warps per SM)
-__global__ void __maxnreg__(sizeof(T) == 4 ? 128 : FW_DYN_MAXNREG)
-#else
 __global__ void __launch_bounds__(FW_DYN_BLOCK, sizeof(T) == 4 ? FW_DYN_MIN_BLOCKS_F32 : FW_DYN_MIN_BLOCKS)
-#endif
 fw_attempt_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const FwDynArgs a) {
   const fw_sim_t& P = fw_sim_of(Px);
   FW_TL_BEGIN(1);
@@ -317,14 +304,7 @@ fw_attempt_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const F
   for (int j = 0; j < 3; ++j) { S.k0pos[j] = 0; in.cmd[j] = 0; in.gl[j] = 0; in.ga[j] = 0; in.wind[j] = 0; }
   bool long_left = n_long > 0, nat_left = true;
   unsigned long long passes = 0, lane_attempts = 0;
-#ifdef FW_TIME_SEGMENTS
-  long long tseg_refill = 0, tseg_park = 0;
-  const long long tseg_start = clock64();
-#endif
   for (;;) {
-#ifdef FW_TIME_SEGMENTS
-    const long long tseg0 = clock64();
-#endif
     // ---- lanes without an aircraft adopt the next waiting ones (priority list first) ----
     const unsigned idle = __ballot_sync(full, S.status != FW_STATUS_RUNNING);
     if (idle && (long_left || nat_left)) {
@@ -362,14 +342,9 @@ fw_attempt_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const F
           // skipped: aircraft that raised inside RK45.__init__ (the init kernel parked that result), and the
           // natural-order visit of an aircraft that is on the priority list
           const bool skip = failv != 0 || (!from_long && h0s < 0.0);
-#ifndef FW_REFILL_LAZY
           // this lane holds no aircraft, so its registers and K slot 0 are free: every load of the candidate is issued
           // before `skip` (which depends on two of them) is known - one dependent L2 round trip less per refill
-          // (-DFW_REFILL_LAZY: load only what will be used, as before)
           {
-#else
-          if (!skip) {
-#endif
             par_base = a.d + (int64_t)a.par_row * a.stride + e;
             if constexpr (Spec::rand)
               for (int r = 0; r < a.n_par_rows; ++r) par_cache[r * 32] = (T)par_base[(int64_t)r * a.stride];
@@ -391,25 +366,16 @@ fw_attempt_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const F
       }
     }
     const unsigned running = __ballot_sync(full, S.status == FW_STATUS_RUNNING);
-#ifdef FW_TIME_SEGMENTS
-    tseg_refill += clock64() - tseg0;
-#endif
     if (!running) {
       if (!long_left && !nat_left) break;
       continue;   // everything adopted in this round was a skip; draw again
     }
     // ---- one dopri5 step attempt for every lane that holds an aircraft ----
     ++passes;
-#ifdef FW_TIME_SEGMENTS
-    long long tseg1 = 0;
-#endif
     if (S.status == FW_STATUS_RUNNING) {
       ++lane_attempts;
       const FwPar<T, Spec::rand ? FW_PAR_SMEM : FW_PAR_CONST> PP{P, par_base, a.stride, par_cache};
       fw_ivp_attempt<T, Spec, FW_DYN_BLOCK>(P, PP, in, S, K);
-#ifdef FW_TIME_SEGMENTS
-      tseg1 = clock64();
-#endif
       if (S.status != FW_STATUS_RUNNING) {   // env step finished (or raised): park the result for the env kernel
         double* cd = a.cd + env;
         int32_t* ci = a.ci + env;
@@ -418,23 +384,11 @@ fw_attempt_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const F
         ci[CI_FAIL * a.stride] = S.fail;
         ci[CI_ATTEMPTS * a.stride] = S.attempts;
         ci[CI_ACCEPTED * a.stride] = S.accepted;
-#ifndef FW_PARK_NO_FENCE   // experiment build (valid with FWGYM_OVERLAP=0 only): what the release fence costs
         __threadfence();                               // results before the count (release)
-#endif
         atomicAdd(FW_CHUNK_DONE(a.q, env), 1);
       }
     }
-#ifdef FW_TIME_SEGMENTS
-    __syncwarp();
-    tseg1 = __shfl_sync(full, tseg1, __ffs(running) - 1);
-    tseg_park += clock64() - tseg1;
-#endif
   }
-#ifdef FW_TIME_SEGMENTS   // experiment build: the divergence counters carry cycle sums instead (scripts/gpu_segments.sh)
-  passes = (unsigned long long)tseg_refill;
-  lane_attempts = lane == 0 ? (unsigned long long)(clock64() - tseg_start) : 0ull;
-  if (lane == 0) atomicAdd(a.ctr + CTR_WATCHDOG, (unsigned long long)tseg_park);
-#endif
   // ---- counters: warp passes (cost) and lane attempts (useful work) ----
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) lane_attempts += __shfl_xor_sync(full, lane_attempts, o);
@@ -444,8 +398,6 @@ fw_attempt_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const F
   }
   FW_TL_END(1);
 }
-
-#include "attempt_pair.cuh"   // fw_attempt_pair_kernel: two warps per 32 aircraft (fp64, FwSpecShipped / FwSpecGeneric)
 
 // ---- PyFly._set_states_from_ode_solution(save=True) + airspeed factors + next gust column (env kernel prologue) ----
 // PyFly Variable.apply_conditions with the variable's condition FLAGS taken from the shape (a literal in a fixed
@@ -774,7 +726,6 @@ fw_env_kernel(const __grid_constant__ fw_env_t E, const __grid_constant__ fw_sim
   FwEnvPre<NZ> pre;
   pre.have_un = false;
   pre.nz = 0;
-#ifndef FW_ENV_NO_PREDRAW   // (experiment build: draw in place, as before round 2)
   if constexpr (SH::fixed) {
     const fw_sim_t& Ps = SH::sim(P);
     if (env < a.n) {
@@ -793,7 +744,6 @@ fw_env_kernel(const __grid_constant__ fw_env_t E, const __grid_constant__ fw_sim
     pre.have_un = Ps.turbulence != 0;
     pre.nz = NZ;
   }
-#endif
   // Wait until every aircraft of this block's chunk has been parked by the dynamics kernels (acquire side of the
   // release in fw_attempt_kernel).  One polling thread per block; the others sleep on the barrier.  The attempt kernel
   // never waits for anything, so this cannot deadlock; the watchdog turns a lost update into an error flag
@@ -1114,21 +1064,6 @@ static cudaError_t launch_dyn(const fw_sim_t& sim_in, const FwDynArgs& da, int a
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   const int64_t warps = (da.n + FW_DYN_BLOCK - 1) / FW_DYN_BLOCK;
-  if constexpr (sizeof(T) == 8 && !Spec::rand) {
-    if (da.pair) {
-      cudaLaunchConfig_t lc = {};
-      lc.gridDim = dim3((unsigned)(warps < da.pair_grid ? warps : da.pair_grid));
-      lc.blockDim = dim3(FW_PAIR_THREADS);
-      lc.dynamicSmemBytes = (size_t)FW_PAIR_SMEM_BYTES;
-      lc.stream = s;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      at[0].val.programmaticStreamSerializationAllowed = 1;
-      lc.attrs = at;
-      lc.numAttrs = da.pdl ? 1 : 0;
-      return cudaLaunchKernelEx(&lc, fw_attempt_pair_kernel<Spec>, sim, da);
-    }
-  }
   const int smem = fw_attempt_smem<T, Spec>(da.n_par_rows);
   const int grid = (int)(warps < attempt_grid ? warps : attempt_grid);
   if (!da.pdl) {
@@ -1149,7 +1084,7 @@ static cudaError_t launch_dyn(const fw_sim_t& sim_in, const FwDynArgs& da, int a
 }
 // per device (called from fw_create): opt in to the K-stage shared memory and size the persistent grid
 template <typename T, class Spec>
-static cudaError_t prepare_dyn(int sm_count, int n_par_rows, int* grid_out, int* pair_grid_out) {
+static cudaError_t prepare_dyn(int sm_count, int n_par_rows, int* grid_out) {
   const int smem = fw_attempt_smem<T, Spec>(n_par_rows);
   cudaError_t e = cudaFuncSetAttribute(fw_attempt_kernel<T, Spec>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;
@@ -1157,18 +1092,6 @@ static cudaError_t prepare_dyn(int sm_count, int n_par_rows, int* grid_out, int*
   e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fw_attempt_kernel<T, Spec>, FW_DYN_BLOCK, smem);
   if (e != cudaSuccess) return e;
   if (grid_out) *grid_out = per_sm * sm_count;
-  if constexpr (sizeof(T) == 8 && !Spec::rand) {
-    if (pair_grid_out) {
-      e = cudaFuncSetAttribute(fw_attempt_pair_kernel<Spec>, cudaFuncAttributeMaxDynamicSharedMemorySize, FW_PAIR_SMEM_BYTES);
-      if (e != cudaSuccess) return e;
-      e = cudaFuncSetAttribute(fw_attempt_pair_kernel<Spec>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-      if (e != cudaSuccess) return e;
-      int pb = 0;
-      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&pb, fw_attempt_pair_kernel<Spec>, FW_PAIR_THREADS, FW_PAIR_SMEM_BYTES);
-      if (e != cudaSuccess) return e;
-      *pair_grid_out = pb * sm_count;
-    }
-  } else if (pair_grid_out) *pair_grid_out = 0;
   return cudaSuccess;
 }
 
@@ -1183,15 +1106,15 @@ static cudaError_t launch_dyn_any(int precision, int spec, const fw_sim_t& sim, 
   if (spec == 1) return launch_dyn<float, FwSpecGeneric>(sim, da, grid, s);
   return launch_dyn<float, FwSpecRand>(sim, da, grid, s);
 }
-static cudaError_t prepare_dyn_any(int precision, int spec, int sms, int n_par_rows, int* grid_out, int* pair_grid_out) {
+static cudaError_t prepare_dyn_any(int precision, int spec, int sms, int n_par_rows, int* grid_out) {
   if (precision == 0) {
-    if (spec == 0) return prepare_dyn<double, FwSpecShipped>(sms, n_par_rows, grid_out, pair_grid_out);
-    if (spec == 1) return prepare_dyn<double, FwSpecGeneric>(sms, n_par_rows, grid_out, pair_grid_out);
-    return prepare_dyn<double, FwSpecRand>(sms, n_par_rows, grid_out, pair_grid_out);
+    if (spec == 0) return prepare_dyn<double, FwSpecShipped>(sms, n_par_rows, grid_out);
+    if (spec == 1) return prepare_dyn<double, FwSpecGeneric>(sms, n_par_rows, grid_out);
+    return prepare_dyn<double, FwSpecRand>(sms, n_par_rows, grid_out);
   }
-  if (spec == 0) return prepare_dyn<float, FwSpecShipped>(sms, n_par_rows, grid_out, pair_grid_out);
-  if (spec == 1) return prepare_dyn<float, FwSpecGeneric>(sms, n_par_rows, grid_out, pair_grid_out);
-  return prepare_dyn<float, FwSpecRand>(sms, n_par_rows, grid_out, pair_grid_out);
+  if (spec == 0) return prepare_dyn<float, FwSpecShipped>(sms, n_par_rows, grid_out);
+  if (spec == 1) return prepare_dyn<float, FwSpecGeneric>(sms, n_par_rows, grid_out);
+  return prepare_dyn<float, FwSpecRand>(sms, n_par_rows, grid_out);
 }
 
 extern "C" {
@@ -1255,9 +1178,6 @@ int fw_create(const fw_config_t* cfg, int64_t n_envs, int64_t global_env_offset,
     const char* e = getenv("FWGYM_LONG_DIV");
     h->long_div = e ? atof(e) : 32.0;
     h->long_h = h->long_div > 0 ? h->cfg.sim.dt / h->long_div : 0.0;
-    const char* w = getenv("FWGYM_LONG_OMEGA");
-    h->long_omega = w ? atof(w) : 0.0;      // off by default: measured 207.1 (3 rad/s) / 208.0 (5) vs 208.5 us per step
-    if (!(h->long_omega > 0)) h->long_omega = 1e300;
   }
   CK(cudaMemset(h->d, 0, db));
   CK(cudaMemset(h->i, 0, ib));
@@ -1281,14 +1201,10 @@ int fw_create(const fw_config_t* cfg, int64_t n_envs, int64_t global_env_offset,
     CK(cudaGetDeviceProperties(&prop, device));
     const int sms = prop.multiProcessorCount;
     int g = 0;
-    int pg = 0;
-    CK(prepare_dyn_any(h->cfg.precision, h->generic, sms, h->L.n_par_rows, &g, &pg));
+    CK(prepare_dyn_any(h->cfg.precision, h->generic, sms, h->L.n_par_rows, &g));
     const char* e = getenv("FWGYM_ATTEMPT_WARPS_PER_SM");
-    if (e && atoi(e) > 0) { g = atoi(e) * sms; if (pg > 0) pg = atoi(e) * sms; }
+    if (e && atoi(e) > 0) g = atoi(e) * sms;
     h->attempt_grid = g > 0 ? g : sms;
-    h->pair_grid = pg;
-    const char* pe = getenv("FWGYM_PAIR");
-    h->pair = (pg > 0 && pe && atoi(pe) != 0) ? 1 : 0;   // opt-in: measured slower than one thread per aircraft (DESIGN.md 4.4)
   }
   *out = h;
   return FW_OK;
@@ -1331,12 +1247,9 @@ int fw_set_config(fw_handle h, const fw_config_t* cfg) {
     cudaDeviceProp prop;
     CK(cudaSetDevice(h->device));
     CK(cudaGetDeviceProperties(&prop, h->device));
-    int g = 0, pg = 0;
-    CK(prepare_dyn_any(h->cfg.precision, h->generic, prop.multiProcessorCount, h->L.n_par_rows, &g, &pg));
+    int g = 0;
+    CK(prepare_dyn_any(h->cfg.precision, h->generic, prop.multiProcessorCount, h->L.n_par_rows, &g));
     if (g > 0) h->attempt_grid = g;
-    h->pair_grid = pg;
-    const char* pe = getenv("FWGYM_PAIR");
-    h->pair = (pg > 0 && pe && atoi(pe) != 0) ? 1 : 0;   // opt-in: measured slower than one thread per aircraft (DESIGN.md 4.4)
   }
   h->long_h = h->long_div > 0 ? h->cfg.sim.dt / h->long_div : 0.0;
   return FW_OK;
@@ -1379,7 +1292,6 @@ const char* fw_kernel_variant(fw_handle h) {
            shape_name(h->shape));
   return buf;
 }
-int fw_attempt_warps_per_group(fw_handle h) { return h ? (h->pair ? 2 : 1) : 0; }
 int64_t fw_state_rows(fw_handle h) { return h ? h->L.d_rows + h->L.i_rows : 0; }
 
 const char* fw_state_row_name(fw_handle h, int64_t r) {
@@ -1457,8 +1369,7 @@ static int step_impl(fw_handle h, const void* actions, int actions_f64, float* o
   cudaStream_t s = (cudaStream_t)stream;
   const uint32_t k0 = (uint32_t)h->seed, k1 = (uint32_t)(h->seed >> 32);
   FwDynArgs da{h->d, h->i, h->L.stride, h->n, actions, actions_f64, h->ctr, h->carry_d, h->carry_i, h->long_list,
-               h->queue, h->long_h, h->long_omega, h->L.par_row, h->L.n_par_rows, h->order, h->pdl_dyn, h->pair,
-               h->pair_grid, getenv("FWGYM_PAIR_MIX") ? atoi(getenv("FWGYM_PAIR_MIX")) : 1};
+               h->queue, h->long_h, h->L.par_row, h->L.n_par_rows, h->order, h->pdl_dyn};
   cudaEvent_t pe[3] = {nullptr, nullptr, nullptr};
   if (h->profiling) {
     for (int k = 0; k < 3; ++k) { CK(cudaEventCreate(&pe[k])); h->ev.push_back(pe[k]); }

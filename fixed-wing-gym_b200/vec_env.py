@@ -444,10 +444,6 @@ class FixedWingVecEnv:
         """Which kernel instantiations the configuration selected, e.g. "dyn=shipped env=default_turb"."""
         return self._lib.fw_kernel_variant(self._h).decode()
 
-    def attempt_warps_per_group(self):
-        """2: the fp64 attempt kernel runs two warps per 32 aircraft (csrc/attempt_pair.cuh); 1: one thread per aircraft."""
-        return self._lib.fw_attempt_warps_per_group(self._h)
-
     def set_profiling(self, on=True):
         _capi.check(self._lib.fw_set_profiling(self._h, 1 if on else 0))
 

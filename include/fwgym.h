@@ -374,11 +374,6 @@ int fw_launches_per_step(fw_handle h);
  * (dynamics.cuh "kernel specialisation", env_shapes.h).  Valid until the next call on the calling thread. */
 const char* fw_kernel_variant(fw_handle h);
 
-/* Warps that share one group of 32 aircraft in the dopri5 attempt kernel: 1 = one thread per aircraft (default),
- * 2 = the two-warp kernel of csrc/attempt_pair.cuh; fp64 without per-env model parameters, opt-in with FWGYM_PAIR=1:
- * parity-tested, measured slower, DESIGN.md 4.4. */
-int fw_attempt_warps_per_group(fw_handle h);
-
 /* Experiment hook (scheduling studies, DESIGN.md 4.4): `order` is a device int32 [N] permutation of the env ids, the
  * order in which the attempt kernel's warps adopt aircraft (NULL restores the natural order).  Results do not depend
  * on it; the time does.  The buffer must stay valid while it is set. */

@@ -1,4 +1,4 @@
-"""Lane reuse in the persistent attempt kernels (DESIGN.md §4.2, csrc/fwgym.cu fw_attempt_kernel, csrc/attempt_pair.cuh).
+"""Lane reuse in the persistent attempt kernel (DESIGN.md §4.2, csrc/fwgym.cu fw_attempt_kernel).
 
 A lane whose aircraft finished its env step parks the result and adopts the next waiting aircraft (priority list, then
 natural order), reloading everything the aircraft's step depends on.  Below ~38 k envs (fp64: 8 resident warps per SM on
@@ -22,7 +22,7 @@ import parity_utils as pu
 TOL = 1e-9
 SEED = 20261017
 BENCH = dict(config="fixed_wing_config.json", config_kw=CONFIG_KW, sim_kw=SIM_KW)
-SWITCHES = ("FWGYM_ATTEMPT_WARPS_PER_SM", "FWGYM_LONG_DIV", "FWGYM_PAIR")
+SWITCHES = ("FWGYM_ATTEMPT_WARPS_PER_SM", "FWGYM_LONG_DIV")
 ONE_WARP_PER_SM = {"FWGYM_ATTEMPT_WARPS_PER_SM": 1}
 TERM_NUMERIC = 3
 
@@ -41,8 +41,6 @@ def make_vec(c, n, monkeypatch, precision="fp64", **switches):
     finally:
         for k in SWITCHES:
             monkeypatch.delenv(k, raising=False)
-    if "FWGYM_PAIR" in switches:
-        assert v.attempt_warps_per_group() == 2
     return v
 
 
@@ -94,13 +92,11 @@ def first_difference(what, x, y, rows=None):
 # 1. lane-assignment invariance, bitwise
 # ---------------------------------------------------------------------------------------------------------------------
 VARIANTS = {
-    "bench": (BENCH, 65536, "fp64", {}),
-    "bench_ragged": (BENCH, 65491, "fp64", {}),
-    "bench_fp32": (BENCH, 65536, "fp32", {}),           # default fp32 grid: 16 warps per SM = 75 776 lanes, no reuse in A
-    "wind": (CASES["wind"], 65536, "fp64", {}),          # FwSpecGeneric: steady wind reloaded on adoption
-    "param_rand_uniform": (CASES["param_rand_uniform"], 65536, "fp64", {}),   # FwSpecRand: parameter cache refilled
-    "bench_pair": (BENCH, 65536, "fp64", {"FWGYM_PAIR": 1}),
-    "wind_pair": (CASES["wind"], 65536, "fp64", {"FWGYM_PAIR": 1}),
+    "bench": (BENCH, 65536, "fp64"),
+    "bench_ragged": (BENCH, 65491, "fp64"),
+    "bench_fp32": (BENCH, 65536, "fp32"),           # default fp32 grid: 16 warps per SM = 75 776 lanes, no reuse in A
+    "wind": (CASES["wind"], 65536, "fp64"),          # FwSpecGeneric: steady wind reloaded on adoption
+    "param_rand_uniform": (CASES["param_rand_uniform"], 65536, "fp64"),   # FwSpecRand: parameter cache refilled
 }
 INVARIANCE_STEPS = 230      # the post-reset transient + 200 steps of the stationary episode mix
 SAME_COUNTERS = ("env_steps", "attempts", "accepted", "failures", "resets", "rhs_evals")
@@ -113,7 +109,7 @@ def test_lane_assignment_invariance(built_lib, variant, monkeypatch):
     order; B default, a fresh random order every step; C one warp per SM with every aircraft whose first step is
     below dt on the priority list; D one warp per SM, empty priority list, reversed order.  After every step B, C and
     D equal A bitwise in the float32 outputs, the attempt counts and the whole state matrix."""
-    c, n, precision, extra = VARIANTS[variant]
+    c, n, precision = VARIANTS[variant]
     lanes = 32 * torch.cuda.get_device_properties(0).multi_processor_count   # one warp per SM
     assert n >= 4 * lanes, "C and D must reuse lanes: %d envs on %d lanes" % (n, lanes)
     gen = torch.Generator(device="cuda")
@@ -124,7 +120,7 @@ def test_lane_assignment_invariance(built_lib, variant, monkeypatch):
     handles = []
     try:
         for name, sw, kind in setups:
-            v = make_vec(c, n, monkeypatch, precision=precision, **dict(extra, **sw))
+            v = make_vec(c, n, monkeypatch, precision=precision, **sw)
             handles.append((name, Order(v, kind, gen)))
         rows = handles[0][1].vec.state_rows()
         obs0 = [o.vec.reset().clone() for _, o in handles]
@@ -304,22 +300,17 @@ def test_bench_workload_sampled_oracle(built_lib, monkeypatch):
     sampled_oracle_parity(BENCH, 65536, 250, monkeypatch, bench_sample, {}, False, "bench workload, full size")
 
 
-REUSE_CASES = {
-    "wind": (CASES["wind"], {}),
-    "wind_pair": (CASES["wind"], {"FWGYM_PAIR": 1}),
-    "param_rand_uniform": (CASES["param_rand_uniform"], {}),
-}
+REUSE_CASES = ("wind", "param_rand_uniform")
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("case", list(REUSE_CASES))
+@pytest.mark.parametrize("case", REUSE_CASES)
 def test_reuse_heavy_sampled_oracle(built_lib, case, monkeypatch):
-    """The FwSpecGeneric (steady wind; one-warp and two-warp kernels) and FwSpecRand instantiations with ~3.5 aircraft
+    """The FwSpecGeneric (steady wind) and FwSpecRand instantiations with ~3.5 aircraft
     per lane per step: 16 384 envs on one warp per SM, every aircraft whose first step is below dt on the priority
     list, a random adoption order every step; 60 steps against the oracle on 128 sampled envs."""
-    c, extra = REUSE_CASES[case]
-    switches = dict(ONE_WARP_PER_SM, FWGYM_LONG_DIV=1, **extra)
-    sampled_oracle_parity(c, 16384, 60, monkeypatch, reuse_sample, switches, True, "reuse-heavy %s" % case)
+    switches = dict(ONE_WARP_PER_SM, FWGYM_LONG_DIV=1)
+    sampled_oracle_parity(CASES[case], 16384, 60, monkeypatch, reuse_sample, switches, True, "reuse-heavy %s" % case)
 
 
 def test_bench_sample_is_distinct_and_complete():

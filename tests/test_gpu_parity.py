@@ -68,21 +68,6 @@ def test_generic_kernel_instantiation(built_lib, name, monkeypatch):
     test_golden_fixture(built_lib, name)
 
 
-@pytest.mark.parametrize("name", ["default", "turb_noise", "failure", "wind", "poly_drag", "target_sinusoidal"])
-def test_two_warp_attempt_kernel(built_lib, name, monkeypatch):
-    """fw_attempt_pair_kernel (csrc/attempt_pair.cuh: two warps share 32 aircraft, SURVEY §7 option (ii)) is opt-in
-    (FWGYM_PAIR=1; measured slower than one thread per aircraft, DESIGN.md 4.4) and held to the same fixtures:
-    states <= 1e-9, done flags and dopri5 attempt counts bit-exact."""
-    vec = make_vec(CASES[name])
-    assert vec.attempt_warps_per_group() == 1
-    vec.close()
-    monkeypatch.setenv("FWGYM_PAIR", "1")
-    vec = make_vec(CASES[name])
-    assert vec.attempt_warps_per_group() == 2
-    vec.close()
-    test_golden_fixture(built_lib, name)
-
-
 def test_kernel_variant_selection(built_lib):
     """The host picks the specialised instantiations exactly for the configurations whose structure they were
     generated from; numbers (noise level, constraint values, curriculum level) do not change the choice."""

@@ -41,20 +41,10 @@ def sim_kw_at(c, level):
     return kw
 
 
-def make_vec(c, n, level, monkeypatch=None, precision="fp64", env_offset=0, pair=False):
+def make_vec(c, n, level, precision="fp64", env_offset=0):
     from fwgym_b200 import FixedWingVecEnv
-    if monkeypatch is not None:
-        monkeypatch.delenv("FWGYM_PAIR", raising=False)
-        if pair:
-            monkeypatch.setenv("FWGYM_PAIR", "1")
-    try:
-        v = FixedWingVecEnv(harness.config_path(c["config"]), n, config_kw=c["config_kw"],
-                            sim_config_kw=sim_kw_at(c, level), seed=SEED, precision=precision, env_offset=env_offset)
-    finally:
-        if monkeypatch is not None:
-            monkeypatch.delenv("FWGYM_PAIR", raising=False)
-    if pair:
-        assert v.attempt_warps_per_group() == 2
+    v = FixedWingVecEnv(harness.config_path(c["config"]), n, config_kw=c["config_kw"],
+                        sim_config_kw=sim_kw_at(c, level), seed=SEED, precision=precision, env_offset=env_offset)
     v.enable_f64_outputs(True)
     return v
 
@@ -104,33 +94,31 @@ def pinned_levels(n, pattern):
 # 1. pinned levels are bitwise the uniform handles
 # ---------------------------------------------------------------------------------------------------------------------
 PINNED = {
-    "bench_4096_mod4": (BENCH, 4096, "fp64", "mod4", False),
-    "bench_4096_random": (BENCH, 4096, "fp64", "random", False),
-    "bench_65536_mod4": (BENCH, 65536, "fp64", "mod4", False),
-    "bench_65536_fp32_random": (BENCH, 65536, "fp32", "random", False),
-    "bench_4096_fp32_mod4": (BENCH, 4096, "fp32", "mod4", False),
-    "wind_mod4": (CASES["wind"], 4096, "fp64", "mod4", False),
-    "wind_random": (CASES["wind"], 4096, "fp64", "random", False),
-    "bench_pair_random": (BENCH, 4096, "fp64", "random", True),
-    "wind_pair_mod4": (CASES["wind"], 4096, "fp64", "mod4", True),
+    "bench_4096_mod4": (BENCH, 4096, "fp64", "mod4"),
+    "bench_4096_random": (BENCH, 4096, "fp64", "random"),
+    "bench_65536_mod4": (BENCH, 65536, "fp64", "mod4"),
+    "bench_65536_fp32_random": (BENCH, 65536, "fp32", "random"),
+    "bench_4096_fp32_mod4": (BENCH, 4096, "fp32", "mod4"),
+    "wind_mod4": (CASES["wind"], 4096, "fp64", "mod4"),
+    "wind_random": (CASES["wind"], 4096, "fp64", "random"),
 }
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", list(PINNED))
-def test_pinned_levels_equal_uniform_handles(built_lib, case, monkeypatch):
+def test_pinned_levels_equal_uniform_handles(built_lib, case):
     """A mixed handle whose envs are pinned to levels (env % 4, or a seeded random assignment) against four uniform
     handles (turbulence off, light, moderate, severe) with the same seed, N and offset, 300 steps with auto-resets on the
     same actions: every env's outputs bitwise equal to those of the handle of its level after every step, and all its
     state rows (except the two level rows) at the end."""
-    c, n, prec, pattern, pair = PINNED[case]
+    c, n, prec, pattern = PINNED[case]
     lv = pinned_levels(n, pattern)
     handles = []
     try:
-        mixed = make_vec(c, n, ALL4, monkeypatch, prec, pair=pair)
+        mixed = make_vec(c, n, ALL4, prec)
         handles.append(mixed)
         mixed.set_turbulence_intensity(lv)
-        uni = [make_vec(c, n, name, monkeypatch, prec, pair=pair) for name in LEVELS]
+        uni = [make_vec(c, n, name, prec) for name in LEVELS]
         handles += uni
         if c is BENCH:
             assert mixed.kernel_variant().endswith("env=default_turb_mixed"), mixed.kernel_variant()
