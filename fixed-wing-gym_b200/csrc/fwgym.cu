@@ -24,15 +24,12 @@
 #include "env.cuh"
 
 #define FW_DYN_BLOCK 32
-#ifndef FW_DYN_MIN_BLOCKS_F32
 #define FW_DYN_MIN_BLOCKS_F32 16
-#endif
-#ifndef FW_DYN_MIN_BLOCKS
 #define FW_DYN_MIN_BLOCKS 8
-#endif
-#ifndef FW_ENV_BLOCK
 #define FW_ENV_BLOCK 128
-#endif
+#define FW_ENV_MIN_BLOCKS 4
+#define FW_INIT_BLOCK 64
+#define FW_INIT_MIN_BLOCKS 8   // 128 registers: one wave at 65536 envs (1024 blocks on 148 x 8 slots); 4 -> 8: init 18 -> 13 us
 
 enum { CTR_ENV_STEPS = 0, CTR_ATTEMPTS, CTR_ACCEPTED, CTR_WARP_MAX, CTR_WARP_STEPS, CTR_FAILURES, CTR_RESETS, CTR_WATCHDOG, CTR_N };
 enum { MS_EPISODES = 0, MS_SUCCESS, MS_RETURN, MS_LENGTH, MS_FAILURES, MS_STEPS_TERM, MS_SUCCESS_TERM, MS_GOAL_STEPS };
@@ -50,10 +47,8 @@ struct fw_handle_s {
   cudaStream_t last_stream;
   int profiling;
   int generic;                   // dynamics instantiation: 0 FwSpecShipped, 1 FwSpecGeneric, 2 FwSpecRand (dynamics.cuh)
-  int overlap;                   // launch the env kernel as a programmatic dependent of the attempt kernel
   int64_t q_len;                 // ints in `queue`: Q_N + chunks
   const int32_t* order;          // fw_debug_set_order
-  int pdl_dyn;                   // attempt kernel launched as a programmatic dependent of the init kernel (FWGYM_PDL_DYN)
   int shape;                     // env / reset kernel instantiation: index into FW_SHAPE_LIST, -1 generic (env_shapes.h)
   double* ep_out;                // caller's episode-metric buffer (fw_set_episode_out)
   const double* turb_noise;      // caller's injected Dryden noise [4, turb_len, n] (fw_reset), NULL: Philox streams
@@ -158,11 +153,10 @@ struct FwDynArgs {
   int32_t par_row;     // first per-env model-parameter row of d (FwSpecRand)
   int32_t n_par_rows;
   const int32_t* order;   // experiment hook (fw_debug_set_order): adoption order of the natural queue, NULL = identity
-  int32_t pdl;            // the attempt kernel was launched as a programmatic dependent of the init kernel
   // ptxas allocates the attempt kernels' registers differently when this block changes size (at 120 or 128 bytes: fp64
   // FwSpecRand 253 -> 254 registers, fp32 FwSpecShipped 127 -> 128, fp32 FwSpecRand spills 60/56 -> 66/68 bytes):
   // padded to the 136 bytes they were tuned at
-  int32_t _pad[5];
+  int32_t _pad[6];
 };
 static_assert(sizeof(FwDynArgs) == 136, "see FwDynArgs._pad");
 
@@ -205,13 +199,7 @@ __device__ __forceinline__ void fw_load_gusts(const fw_sim_t& P, const FwEnvCtx&
   }
 }
 
-#ifndef FW_INIT_BLOCK
-#define FW_INIT_BLOCK 64
-#endif
 template <typename T, class Spec>
-#ifndef FW_INIT_MIN_BLOCKS
-#define FW_INIT_MIN_BLOCKS 8   // 128 registers: one wave at 65536 envs (1024 blocks on 148 x 8 slots); 4 -> 8: init 18 -> 13 us
-#endif
 __global__ void __launch_bounds__(FW_INIT_BLOCK, FW_INIT_MIN_BLOCKS)
 fw_init_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const FwDynArgs a) {
   const fw_sim_t& P = fw_sim_of(Px);
@@ -222,9 +210,9 @@ fw_init_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const FwDy
   // Queue words are zeroed by the kernels instead of a memset node per step (one launch gap less): the two cursors,
   // which only the attempt kernel uses, here; the priority-list length and the chunk counters by the env kernel of the
   // previous step once it has consumed them (fw_create, a full fw_reset and fw_set_state zero everything).
-  // (a.pdl) let the attempt kernel's warps take their places on the SMs as this kernel's blocks retire; they wait for
-  // this grid's completion (griddepcontrol.wait) before they read anything
-  if (a.pdl) asm volatile("griddepcontrol.launch_dependents;");
+  // Let the attempt kernel's warps take their places on the SMs as this kernel's blocks retire; they wait for this
+  // grid's completion (griddepcontrol.wait) before they read anything
+  asm volatile("griddepcontrol.launch_dependents;");
   if (blockIdx.x == 0 && threadIdx.x == 0) { a.q[Q_LONG_CURSOR] = 0; a.q[Q_NAT_CURSOR] = 0; }
   if (valid) {
     FwEnvCtx c{a.d, a.i, a.stride, env};
@@ -283,7 +271,7 @@ fw_attempt_kernel(const __grid_constant__ typename FwSimArg<T>::type Px, const F
   FwKStore<T, FW_DYN_BLOCK> K{reinterpret_cast<T*>(smem_raw)};
   // Every warp of this (fully resident) grid is on an SM by now: let the env kernel's blocks queue up behind us.  They
   // synchronise on the per-chunk counters below, not on this kernel's completion.
-  if (a.pdl) asm volatile("griddepcontrol.wait;" ::: "memory");   // the init kernel has completed and its writes are visible
+  asm volatile("griddepcontrol.wait;" ::: "memory");   // the init kernel has completed and its writes are visible
   // (The priority-list length is read first and the release depends on it: env block 0 zeroes it for the next step.)
   const int n_long = a.q[Q_LONG_COUNT];     // final: the init kernel has completed
   asm volatile("griddepcontrol.launch_dependents;" :: "r"(n_long) : "memory");
@@ -711,9 +699,6 @@ __device__ __forceinline__ void fw_flush_metrics(const FwEnvArgs& a, double (&m)
   }
 }
 
-#ifndef FW_ENV_MIN_BLOCKS
-#define FW_ENV_MIN_BLOCKS 4
-#endif
 template <class SH>
 __global__ void __launch_bounds__(FW_ENV_BLOCK, FW_ENV_MIN_BLOCKS)
 fw_env_kernel(const __grid_constant__ fw_env_t E, const __grid_constant__ fw_sim_t P, const __grid_constant__ FwLayout L,
@@ -1066,10 +1051,6 @@ static cudaError_t launch_dyn(const fw_sim_t& sim_in, const FwDynArgs& da, int a
   const int64_t warps = (da.n + FW_DYN_BLOCK - 1) / FW_DYN_BLOCK;
   const int smem = fw_attempt_smem<T, Spec>(da.n_par_rows);
   const int grid = (int)(warps < attempt_grid ? warps : attempt_grid);
-  if (!da.pdl) {
-    fw_attempt_kernel<T, Spec><<<grid, FW_DYN_BLOCK, smem, s>>>(sim, da);
-    return cudaGetLastError();
-  }
   cudaLaunchConfig_t lc = {};
   lc.gridDim = dim3((unsigned)grid);
   lc.blockDim = dim3(FW_DYN_BLOCK);
@@ -1117,6 +1098,18 @@ static cudaError_t prepare_dyn_any(int precision, int spec, int sms, int n_par_r
   return prepare_dyn<float, FwSpecRand>(sms, n_par_rows, grid_out);
 }
 
+// persistent grid of the handle's attempt kernel: its resident capacity on the device, or FWGYM_ATTEMPT_WARPS_PER_SM
+// warps per SM; one warp per SM if the occupancy query reports none
+static int size_attempt_grid(fw_handle h) {
+  int sms = 0, g = 0;
+  CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
+  CK(prepare_dyn_any(h->cfg.precision, h->generic, sms, h->L.n_par_rows, &g));
+  const char* e = getenv("FWGYM_ATTEMPT_WARPS_PER_SM");
+  if (e && atoi(e) > 0) g = atoi(e) * sms;
+  h->attempt_grid = g > 0 ? g : sms;
+  return FW_OK;
+}
+
 extern "C" {
 
 static void host_free(fw_handle h);
@@ -1125,49 +1118,25 @@ const char* fw_last_error(void) { return g_err; }
 int fw_abi_version(void) { return FW_ABI_VERSION; }
 int64_t fw_config_sizeof(void) { return (int64_t)sizeof(fw_config_t); }
 
-int fw_create(const fw_config_t* cfg, int64_t n_envs, int64_t global_env_offset, int device, fw_handle* out) {
-  if (!cfg || !out || n_envs <= 0) return fail(FW_ERR_ARG, "fw_create: bad argument");
-  if (cfg->abi_version != FW_ABI_VERSION) return fail(FW_ERR_ABI, "fw_create: config ABI version mismatch");
-  CK(cudaSetDevice(device));
-  fw_handle_s* h = new (std::nothrow) fw_handle_s();
-  if (!h) return fail(FW_ERR_ALLOC, "out of host memory");
-  h->cfg = *cfg;
-  h->device = device;
-  h->n = n_envs;
-  h->offset = global_env_offset;
-  h->seed = 0;
-  h->last_stream = nullptr;
-  h->profiling = 0;
-  h->ep_out = nullptr;
-  h->turb_noise = nullptr;
-  h->turb_len = 0;
-  h->err_flag_host = nullptr;
-  h->err_flag_dev = nullptr;
-  h->spin_limit = 1u << 22;   // x 256 ns: ~1 s
-  h->starve_next = 0;
-  int rc = make_layout(h->cfg, n_envs, h->L);
-  if (rc) { delete h; return rc; }
+// buffers and launch choices of a value-initialised handle; on failure fw_create hands the partly built handle to
+// fw_destroy
+static int init_handle(fw_handle h) {
+  int rc = make_layout(h->cfg, h->n, h->L);
+  if (rc) return rc;
   const size_t db = (size_t)h->L.d_rows * h->L.stride * sizeof(double);
   const size_t ib = (size_t)h->L.i_rows * h->L.stride * sizeof(int32_t);
   if (cudaMalloc(&h->d, db) != cudaSuccess || cudaMalloc(&h->i, ib) != cudaSuccess ||
       cudaMalloc(&h->ctr, CTR_N * sizeof(unsigned long long)) != cudaSuccess ||
-      cudaMalloc(&h->msum, FW_N_METRIC_SUMS * sizeof(double)) != cudaSuccess) {
-    delete h;
+      cudaMalloc(&h->msum, FW_N_METRIC_SUMS * sizeof(double)) != cudaSuccess)
     return fail(FW_ERR_ALLOC, "cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
-  }
-  h->carry_d = nullptr; h->carry_i = nullptr; h->long_list = nullptr; h->queue = nullptr;
   if (cudaMalloc(&h->carry_d, (size_t)CY_ROWS * h->L.stride * sizeof(double)) != cudaSuccess ||
       cudaMalloc(&h->carry_i, (size_t)CI_ROWS * h->L.stride * sizeof(int32_t)) != cudaSuccess ||
       cudaMalloc(&h->long_list, (size_t)h->L.stride * sizeof(int32_t)) != cudaSuccess ||
-      cudaMalloc(&h->queue, (size_t)(h->q_len = Q_N + (h->L.stride + FW_ENV_BLOCK - 1) / FW_ENV_BLOCK) * sizeof(int32_t)) != cudaSuccess) {
-    delete h;
+      cudaMalloc(&h->queue, (size_t)(h->q_len = Q_N + (h->L.stride + FW_ENV_BLOCK - 1) / FW_ENV_BLOCK) * sizeof(int32_t)) != cudaSuccess)
     return fail(FW_ERR_ALLOC, "cudaMalloc (carry) failed: %s", cudaGetErrorString(cudaGetLastError()));
-  }
   if (cudaHostAlloc(&h->err_flag_host, sizeof(int), cudaHostAllocMapped) != cudaSuccess ||
-      cudaHostGetDevicePointer(&h->err_flag_dev, h->err_flag_host, 0) != cudaSuccess) {
-    delete h;
+      cudaHostGetDevicePointer(&h->err_flag_dev, h->err_flag_host, 0) != cudaSuccess)
     return fail(FW_ERR_ALLOC, "cudaHostAlloc (error flag) failed: %s", cudaGetErrorString(cudaGetLastError()));
-  }
   *h->err_flag_host = 0;
   CK(cudaMemset(h->queue, 0, (size_t)h->q_len * sizeof(int32_t)));   // from here on the kernels keep it zeroed (fw_init_kernel)
   CK(cudaMemset(h->carry_d, 0, (size_t)CY_ROWS * h->L.stride * sizeof(double)));
@@ -1187,29 +1156,27 @@ int fw_create(const fw_config_t* cfg, int64_t n_envs, int64_t global_env_offset,
   CK(cudaMemset(h->msum, 0, FW_N_METRIC_SUMS * sizeof(double)));
   h->generic = needs_generic(h->cfg.sim);
   h->shape = pick_shape(h->cfg);
-  h->order = nullptr;
-  {
-    const char* e = getenv("FWGYM_PDL_DYN");
-    h->pdl_dyn = e ? atoi(e) : 1;
-  }
-  {
-    const char* e = getenv("FWGYM_OVERLAP");
-    h->overlap = e ? atoi(e) : 1;
-  }
-  {
-    cudaDeviceProp prop;
-    CK(cudaGetDeviceProperties(&prop, device));
-    const int sms = prop.multiProcessorCount;
-    int g = 0;
-    CK(prepare_dyn_any(h->cfg.precision, h->generic, sms, h->L.n_par_rows, &g));
-    const char* e = getenv("FWGYM_ATTEMPT_WARPS_PER_SM");
-    if (e && atoi(e) > 0) g = atoi(e) * sms;
-    h->attempt_grid = g > 0 ? g : sms;
-  }
+  return size_attempt_grid(h);
+}
+
+int fw_create(const fw_config_t* cfg, int64_t n_envs, int64_t global_env_offset, int device, fw_handle* out) {
+  if (!cfg || !out || n_envs <= 0) return fail(FW_ERR_ARG, "fw_create: bad argument");
+  if (cfg->abi_version != FW_ABI_VERSION) return fail(FW_ERR_ABI, "fw_create: config ABI version mismatch");
+  CK(cudaSetDevice(device));
+  fw_handle_s* h = new (std::nothrow) fw_handle_s();
+  if (!h) return fail(FW_ERR_ALLOC, "out of host memory");
+  h->cfg = *cfg;
+  h->device = device;
+  h->n = n_envs;
+  h->offset = global_env_offset;
+  h->spin_limit = 1u << 22;   // x 256 ns: ~1 s
+  const int rc = init_handle(h);
+  if (rc) { fw_destroy(h); return rc; }
   *out = h;
   return FW_OK;
 }
 
+// also frees the partly built handle of a failed fw_create: any of its buffers may still be null
 int fw_destroy(fw_handle h) {
   if (!h) return FW_OK;
   cudaSetDevice(h->device);
@@ -1244,12 +1211,9 @@ int fw_set_config(fw_handle h, const fw_config_t* cfg) {
   h->shape = pick_shape(h->cfg);
   if (needs_generic(h->cfg.sim) != h->generic) {
     h->generic = needs_generic(h->cfg.sim);
-    cudaDeviceProp prop;
     CK(cudaSetDevice(h->device));
-    CK(cudaGetDeviceProperties(&prop, h->device));
-    int g = 0;
-    CK(prepare_dyn_any(h->cfg.precision, h->generic, prop.multiProcessorCount, h->L.n_par_rows, &g));
-    if (g > 0) h->attempt_grid = g;
+    rc = size_attempt_grid(h);
+    if (rc) return rc;
   }
   h->long_h = h->long_div > 0 ? h->cfg.sim.dt / h->long_div : 0.0;
   return FW_OK;
@@ -1369,7 +1333,7 @@ static int step_impl(fw_handle h, const void* actions, int actions_f64, float* o
   cudaStream_t s = (cudaStream_t)stream;
   const uint32_t k0 = (uint32_t)h->seed, k1 = (uint32_t)(h->seed >> 32);
   FwDynArgs da{h->d, h->i, h->L.stride, h->n, actions, actions_f64, h->ctr, h->carry_d, h->carry_i, h->long_list,
-               h->queue, h->long_h, h->L.par_row, h->L.n_par_rows, h->order, h->pdl_dyn};
+               h->queue, h->long_h, h->L.par_row, h->L.n_par_rows, h->order};
   cudaEvent_t pe[3] = {nullptr, nullptr, nullptr};
   if (h->profiling) {
     for (int k = 0; k < 3; ++k) { CK(cudaEventCreate(&pe[k])); h->ev.push_back(pe[k]); }
@@ -1385,7 +1349,7 @@ static int step_impl(fw_handle h, const void* actions, int actions_f64, float* o
   h->starve_next = 0;
   const int egrid = (int)((h->n + FW_ENV_BLOCK - 1) / FW_ENV_BLOCK);
   // with per-kernel profiling on, an event sits between the two kernels, so they are serialised anyway
-  CK(launch_env(h->shape, egrid, s, h->overlap && !h->profiling, h->cfg.env, h->cfg.sim, h->L, ea));
+  CK(launch_env(h->shape, egrid, s, !h->profiling, h->cfg.env, h->cfg.sim, h->L, ea));
   if (h->profiling) CK(cudaEventRecord(pe[2], s));
   h->last_stream = s;
   return FW_OK;
@@ -1431,7 +1395,7 @@ int fw_host_open_ex(fw_handle h, int depth, int zero_copy) {
     if (!ok ||
         cudaEventCreateWithFlags(&r.e_in, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&r.e_step, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&r.e_out, cudaEventDisableTiming | (getenv("FWGYM_HOST_BLOCKING") ? cudaEventBlockingSync : 0)) != cudaSuccess) {
+        cudaEventCreateWithFlags(&r.e_out, cudaEventDisableTiming) != cudaSuccess) {
       const char* msg = cudaGetErrorString(cudaGetLastError());
       host_free(h);
       return fail(FW_ERR_ALLOC, "fw_host_open: allocation failed: %s", msg);

@@ -1,5 +1,5 @@
 #!/bin/bash
-# A/B library variants on the bench workload, interleaved twice: scripts/gpu_ab.sh base fused fused@FWGYM_OWN_FRACTION=0.5 ...
+# A/B library variants on the bench workload, interleaved twice: scripts/gpu_ab.sh base base@FWGYM_LONG_DIV=0 ...
 # (names under build/variants, scripts/build_variant.sh; NAME@VAR=VALUE sets an environment variable for that arm)
 for rep in $(seq 1 ${REPS:-2}); do
 for arm in "$@"; do

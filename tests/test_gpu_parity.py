@@ -127,7 +127,7 @@ def test_ragged_env_counts(built_lib, n):
     assert out["done_mismatch"] == 0 and out["k_mismatch"] == 0
     # free-running (device and oracle each continue from their OWN state), under turbulence: observations / rewards hold
     # the per-step bar; a raw simulator state near a zero crossing of one sensitive aircraft showed 1.7e-9 for one step
-    # (absolute 1.7e-12, env 3 of 197 - not in the ragged part; scripts/gpu_debug_ragged.py), hence the rollout bar there
+    # (absolute 1.7e-12, env 3 of 197 - not in the ragged part), hence the rollout bar there
     assert max(out["obs"]) <= TOL and max(out["rew"]) <= TOL and max(out["state"]) <= 1e-7, out
     ctr = vec.counters()
     assert ctr["env_steps"] == n * steps and ctr["watchdog"] == 0
@@ -266,17 +266,17 @@ def test_scenario_injection(built_lib):
         assert pu.rel_err(vec._rew64.cpu().numpy(), np.array([r[1] for r in res]), 1e-3).max() <= TOL
 
 
-def test_overlapped_env_kernel_is_bitwise_identical(built_lib, monkeypatch):
+def test_overlapped_env_kernel_is_bitwise_identical(built_lib):
     """The env kernel normally runs as a programmatic dependent of the attempt kernel (its blocks start while the
     attempt kernel's tail is still running and wait on per-chunk completion counters).  Serialised launches
-    (FWGYM_OVERLAP=0) must give bitwise identical states, and no block may ever have given up waiting."""
+    (per-kernel profiling on) must give bitwise identical states, and no block may ever have given up waiting."""
     c = CASES["turb_noise"]
     n = 4096 + 77      # several chunks per SM and a ragged last chunk
     acts = torch.rand((12, n, 3), dtype=torch.float64, device="cuda") * 2 - 1
     states = []
-    for overlap in ("1", "0"):
-        monkeypatch.setenv("FWGYM_OVERLAP", overlap)
+    for serial in (False, True):
         vec = make_vec(c, n=n, seed=33)
+        vec.set_profiling(serial)
         vec.reset()
         for a in acts:
             vec.step_tensors(a)
