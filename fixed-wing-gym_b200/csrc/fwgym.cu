@@ -34,6 +34,9 @@
 enum { CTR_ENV_STEPS = 0, CTR_ATTEMPTS, CTR_ACCEPTED, CTR_WARP_MAX, CTR_WARP_STEPS, CTR_FAILURES, CTR_RESETS, CTR_WATCHDOG, CTR_N };
 enum { MS_EPISODES = 0, MS_SUCCESS, MS_RETURN, MS_LENGTH, MS_FAILURES, MS_STEPS_TERM, MS_SUCCESS_TERM, MS_GOAL_STEPS };
 
+struct FwDynEntry;     // kernel instantiation tables ("kernel instantiations" below)
+struct FwShapeEntry;
+
 struct fw_handle_s {
   fw_config_t cfg;
   FwLayout L;
@@ -46,10 +49,10 @@ struct fw_handle_s {
   double* msum;              // FW_N_METRIC_SUMS
   cudaStream_t last_stream;
   int profiling;
-  int generic;                   // dynamics instantiation: 0 FwSpecShipped, 1 FwSpecGeneric, 2 FwSpecRand (dynamics.cuh)
+  const FwDynEntry* dyn;         // dynamics kernel instantiation (select_kernels)
   int64_t q_len;                 // ints in `queue`: Q_N + chunks
   const int32_t* order;          // fw_debug_set_order
-  int shape;                     // env / reset kernel instantiation: index into FW_SHAPE_LIST, -1 generic (env_shapes.h)
+  const FwShapeEntry* shape;     // env / reset kernel instantiation (select_kernels)
   double* ep_out;                // caller's episode-metric buffer (fw_set_episode_out)
   const double* turb_noise;      // caller's injected Dryden noise [4, turb_len, n] (fw_reset), NULL: Philox streams
   int64_t turb_len;
@@ -91,9 +94,10 @@ static int fail(int code, const char* fmt, const char* a = "") {
   } while (0)
 
 // sticky watchdog error (fw_env_kernel): the flag lives in mapped pinned memory, so this is a plain host load
+static bool poisoned(fw_handle h) { return *reinterpret_cast<volatile int*>(h->err_flag_host) != 0; }
 #define CK_POISON(h)                                                                                             \
   do {                                                                                                           \
-    if (*reinterpret_cast<volatile int*>((h)->err_flag_host))                                                    \
+    if (poisoned(h))                                                                                             \
       return fail(FW_ERR_WATCHDOG, "an env-kernel block gave up waiting for its aircraft (fw_counters().watchdog): "  \
                                    "state of its envs was not advanced; call fw_reset (all envs) or fw_set_state%s", ""); \
   } while (0)
@@ -877,57 +881,6 @@ static_assert(sizeof(fw_sim_t) + sizeof(FwDynArgs) + 64 <= 32764, "fp64 dynamics
 // the per-level Dryden tables were appended without moving any later kernel parameter off its 16-byte alignment
 static_assert(sizeof(fw_sim_t) % 32 == 24 && sizeof(FwLayout) % 16 == 8, "see fw_sim_t._pad_turb / FwLayout._pad_tl");
 
-// ---- shape dispatch: index into FW_SHAPE_LIST (fw_find_shape), -1 = generic -----------------------------------------
-// overlap != 0: programmatic dependent launch - the kernel may start while the preceding kernel of the stream (the
-// attempt kernel) is still running; it synchronises on the per-chunk counters
-template <class SH>
-static cudaError_t launch_env_t(int grid, cudaStream_t s, int overlap, const fw_env_t& E, const fw_sim_t& P,
-                                const FwLayout& L, const FwEnvArgs& a) {
-  cudaLaunchConfig_t lc = {};
-  lc.gridDim = dim3((unsigned)grid);
-  lc.blockDim = dim3(FW_ENV_BLOCK);
-  lc.dynamicSmemBytes = a.stage_obs ? (size_t)FW_ENV_BLOCK * a.obs_dim * sizeof(float) : 0;
-  lc.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  lc.attrs = at;
-  lc.numAttrs = overlap ? 1 : 0;
-  return cudaLaunchKernelEx(&lc, fw_env_kernel<SH>, E, P, L, a);
-}
-static cudaError_t launch_env(int shape, int grid, cudaStream_t s, int overlap, const fw_env_t& E, const fw_sim_t& P,
-                              const FwLayout& L, const FwEnvArgs& a) {
-  int idx = 0;
-#define FW_LAUNCH_SHAPE(NAME) if (shape == idx++) return launch_env_t<FwShape_##NAME>(grid, s, overlap, E, P, L, a);
-  FW_SHAPE_LIST(FW_LAUNCH_SHAPE)
-#undef FW_LAUNCH_SHAPE
-  if (P.turb_mixed) return launch_env_t<FwShapeGenericMixed>(grid, s, overlap, E, P, L, a);
-  return launch_env_t<FwShapeGeneric>(grid, s, overlap, E, P, L, a);
-}
-static cudaError_t launch_reset(int shape, int grid, cudaStream_t s, const fw_env_t& E, const fw_sim_t& P,
-                                const FwLayout& L, const FwResetArgs& a) {
-  int idx = 0;
-#define FW_LAUNCH_SHAPE(NAME)                                                           \
-  if (shape == idx++) { fw_reset_kernel<FwShape_##NAME><<<grid, FW_ENV_BLOCK, 0, s>>>(E, P, L, a); return cudaGetLastError(); }
-  FW_SHAPE_LIST(FW_LAUNCH_SHAPE)
-#undef FW_LAUNCH_SHAPE
-  if (P.turb_mixed) fw_reset_kernel<FwShapeGenericMixed><<<grid, FW_ENV_BLOCK, 0, s>>>(E, P, L, a);
-  else fw_reset_kernel<FwShapeGeneric><<<grid, FW_ENV_BLOCK, 0, s>>>(E, P, L, a);
-  return cudaGetLastError();
-}
-static const char* shape_name(int shape) {
-  int idx = 0;
-#define FW_NAME_SHAPE(NAME) if (shape == idx++) return #NAME;
-  FW_SHAPE_LIST(FW_NAME_SHAPE)
-#undef FW_NAME_SHAPE
-  return "generic";
-}
-static int pick_shape(const fw_config_t& cfg) {
-  const char* force = getenv("FWGYM_FORCE_GENERIC");
-  if (force && force[0] == '1') return -1;
-  return fw_find_shape(cfg.env, cfg.sim);
-}
-
 // ---- PID baseline controller (pyfly/pid_controller.py; evaluate_controller.py:141-151) ---------------------------
 __global__ void fw_pid_kernel(const double* __restrict__ d, int64_t stride, int64_t n, const fw_pid_gains_t g, double dt,
                               int k_roll, int k_pitch, int k_va, double* __restrict__ integ,
@@ -955,14 +908,7 @@ __global__ void fw_pid_kernel(const double* __restrict__ d, int64_t stride, int6
   actions[env * 3 + 2] = dt_;
 }
 
-// ---- state export / import: [rows_d + rows_i, N] doubles -----------------------------------------------------
-__global__ void fw_export_kernel(const double* d, const int32_t* i, int64_t stride, int64_t n, int rows_d, int rows_i,
-                                 double* out) {
-  const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (env >= n) return;
-  for (int r = 0; r < rows_d; ++r) out[(int64_t)r * n + env] = d[(int64_t)r * stride + env];
-  for (int r = 0; r < rows_i; ++r) out[(int64_t)(rows_d + r) * n + env] = (double)i[(int64_t)r * stride + env];
-}
+// ---- state import: [rows_d + rows_i, N] doubles (export: fw_export_rows_kernel) -------------------------------
 __global__ void fw_import_kernel(double* d, int32_t* i, int64_t stride, int64_t n, int rows_d, int rows_i,
                                  const double* in) {
   const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -998,35 +944,31 @@ __global__ void __launch_bounds__(256) fw_dfma_kernel(double* out, int iters, do
 }
 
 // ------------------------------------------------------------------------------------------------------- host side
+static int blocks(int64_t n, int per_block) { return (int)((n + per_block - 1) / per_block); }
+
+// pdl: programmatic dependent launch - the kernel may start while the preceding kernel of the stream is still running
+template <typename... P, typename... A>
+static cudaError_t launch(void (*kernel)(P...), int grid, int block, size_t smem, cudaStream_t s, bool pdl,
+                          const A&... args) {
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t lc = {};
+  lc.gridDim = dim3((unsigned)grid);
+  lc.blockDim = dim3((unsigned)block);
+  lc.dynamicSmemBytes = smem;
+  lc.stream = s;
+  lc.attrs = at;
+  lc.numAttrs = pdl ? 1 : 0;
+  return cudaLaunchKernelEx(&lc, kernel, args...);
+}
+
 static int make_layout(const fw_config_t& cfg, int64_t n, FwLayout& L) {
   if (cfg.sim.turb_mixed && !cfg.sim.turbulence)
     return fail(FW_ERR_CONFIG, "per-env turbulence levels (turb_mixed) need turbulence on");
   const int rc = fw_layout_build(cfg.env, cfg.sim.scale_actions, n, L, cfg.sim.turb_mixed);
   if (rc) return fail(FW_ERR_CONFIG, "%s", fw_layout_error(rc));
   return FW_OK;
-}
-
-// Which dynamics-kernel instantiation covers this configuration (dynamics.cuh "kernel specialisation")
-static int needs_generic(const fw_sim_t& S) {
-  static const int rank_sv[FW_R_BETA + 1] = {FW_SV_OMEGA_P, FW_SV_OMEGA_Q, FW_SV_OMEGA_R, FW_SV_VEL_U, FW_SV_VEL_V,
-                                             FW_SV_VEL_W, FW_SV_ELEVON_L, FW_SV_ELEVON_R, FW_SV_THROTTLE,
-                                             FW_SV_AILERON, FW_SV_ELEVATOR, FW_SV_VA, FW_SV_ALPHA, FW_SV_BETA};
-  for (int i = 0; i < FW_PAR_N; ++i)
-    if (S.par_slot1[i]) return 2;   // per-env model parameters: FwSpecRand
-  const char* force = getenv("FWGYM_FORCE_GENERIC");
-  if (force && force[0] == '1') return 1;
-  uint32_t clip = 0, cons = 0;
-  for (int r = 0; r <= FW_R_BETA; ++r) {
-    const uint32_t f = S.var[rank_sv[r]].flags;
-    if (f & (FW_VC_VMIN | FW_VC_VMAX)) clip |= FW_RB(r);
-    if (f & (FW_VC_CMIN | FW_VC_CMAX)) cons |= FW_RB(r);
-  }
-  for (int i = 0; i < FW_N_ACT; ++i)
-    if (S.act_has_dot_max[i]) clip |= FW_RB(FW_R_AD0 + i);
-  if (clip & ~FwSpecShipped::clip) return 1;
-  if (cons & ~FwSpecShipped::cons) return 1;
-  if (S.wind_enabled || S.drag_model != 0) return 1;
-  return 0;
 }
 
 // dynamic shared memory of one attempt warp: 6 K stages x 16 components (+ the parameter cache of FwSpecRand)
@@ -1044,24 +986,12 @@ static cudaError_t launch_dyn(const fw_sim_t& sim_in, const FwDynArgs& da, int a
     const double* src = reinterpret_cast<const double*>(&sim_in);
     for (size_t k = 0; k < sizeof(fw_sim_t) / 8; ++k) sim.F.v[k] = (float)src[k];
   }
-  const int igrid = (int)((da.n + FW_INIT_BLOCK - 1) / FW_INIT_BLOCK);
-  fw_init_kernel<T, Spec><<<igrid, FW_INIT_BLOCK, 0, s>>>(sim, da);
+  fw_init_kernel<T, Spec><<<blocks(da.n, FW_INIT_BLOCK), FW_INIT_BLOCK, 0, s>>>(sim, da);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  const int64_t warps = (da.n + FW_DYN_BLOCK - 1) / FW_DYN_BLOCK;
-  const int smem = fw_attempt_smem<T, Spec>(da.n_par_rows);
-  const int grid = (int)(warps < attempt_grid ? warps : attempt_grid);
-  cudaLaunchConfig_t lc = {};
-  lc.gridDim = dim3((unsigned)grid);
-  lc.blockDim = dim3(FW_DYN_BLOCK);
-  lc.dynamicSmemBytes = (size_t)smem;
-  lc.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  lc.attrs = at;
-  lc.numAttrs = 1;
-  return cudaLaunchKernelEx(&lc, fw_attempt_kernel<T, Spec>, sim, da);
+  const int warps = blocks(da.n, FW_DYN_BLOCK);
+  return launch(fw_attempt_kernel<T, Spec>, warps < attempt_grid ? warps : attempt_grid, FW_DYN_BLOCK,
+                (size_t)fw_attempt_smem<T, Spec>(da.n_par_rows), s, true, sim, da);
 }
 // per device (called from fw_create): opt in to the K-stage shared memory and size the persistent grid
 template <typename T, class Spec>
@@ -1076,26 +1006,66 @@ static cudaError_t prepare_dyn(int sm_count, int n_par_rows, int* grid_out) {
   return cudaSuccess;
 }
 
-// dynamics instantiation by (precision, spec)
-static cudaError_t launch_dyn_any(int precision, int spec, const fw_sim_t& sim, const FwDynArgs& da, int grid, cudaStream_t s) {
-  if (precision == 0) {
-    if (spec == 0) return launch_dyn<double, FwSpecShipped>(sim, da, grid, s);
-    if (spec == 1) return launch_dyn<double, FwSpecGeneric>(sim, da, grid, s);
-    return launch_dyn<double, FwSpecRand>(sim, da, grid, s);
+// ---- kernel instantiations: chosen once per configuration (select_kernels), launched through these entries --------
+// name: what fw_kernel_variant reports
+struct FwDynEntry {
+  const char* name;
+  cudaError_t (*launch)(const fw_sim_t& sim, const FwDynArgs& da, int attempt_grid, cudaStream_t s);
+  cudaError_t (*prepare)(int sm_count, int n_par_rows, int* grid_out);
+};
+enum { DYN_SHIPPED = 0, DYN_GENERIC, DYN_RAND };   // dynamics.cuh "kernel specialisation"
+#define FW_DYN_ENTRY(T, SPEC, NAME) {NAME, launch_dyn<T, SPEC>, prepare_dyn<T, SPEC>}
+static const FwDynEntry kDynKernels[2][3] = {   // [fw_config_t.precision: fp64, fp32][DYN_*]
+    {FW_DYN_ENTRY(double, FwSpecShipped, "shipped"), FW_DYN_ENTRY(double, FwSpecGeneric, "generic"),
+     FW_DYN_ENTRY(double, FwSpecRand, "rand")},
+    {FW_DYN_ENTRY(float, FwSpecShipped, "shipped"), FW_DYN_ENTRY(float, FwSpecGeneric, "generic"),
+     FW_DYN_ENTRY(float, FwSpecRand, "rand")}};
+#undef FW_DYN_ENTRY
+
+struct FwShapeEntry {
+  const char* name;
+  void (*env)(fw_env_t, fw_sim_t, FwLayout, FwEnvArgs);
+  void (*reset)(fw_env_t, fw_sim_t, FwLayout, FwResetArgs);
+};
+// FW_SHAPE_LIST in fw_find_shape's order, then the two table-walking instantiations (env_shapes.h)
+#define FW_SHAPE_ENTRY(NAME) {#NAME, fw_env_kernel<FwShape_##NAME>, fw_reset_kernel<FwShape_##NAME>},
+static const FwShapeEntry kShapeKernels[] = {
+    FW_SHAPE_LIST(FW_SHAPE_ENTRY)
+    {"generic", fw_env_kernel<FwShapeGeneric>, fw_reset_kernel<FwShapeGeneric>},
+    {"generic", fw_env_kernel<FwShapeGenericMixed>, fw_reset_kernel<FwShapeGenericMixed>}};
+#undef FW_SHAPE_ENTRY
+static constexpr int kShapeGeneric = sizeof(kShapeKernels) / sizeof(kShapeKernels[0]) - 2;
+
+struct FwKernels {
+  const FwDynEntry* dyn;
+  const FwShapeEntry* shape;
+};
+// The leanest instantiations that cover this configuration.  FWGYM_FORCE_GENERIC=1 selects the table-walking kernels
+// even for a shipped configuration; per-env model parameters still need FwSpecRand.
+static FwKernels select_kernels(const fw_config_t& cfg) {
+  static const int rank_sv[FW_R_BETA + 1] = {FW_SV_OMEGA_P, FW_SV_OMEGA_Q, FW_SV_OMEGA_R, FW_SV_VEL_U, FW_SV_VEL_V,
+                                             FW_SV_VEL_W, FW_SV_ELEVON_L, FW_SV_ELEVON_R, FW_SV_THROTTLE,
+                                             FW_SV_AILERON, FW_SV_ELEVATOR, FW_SV_VA, FW_SV_ALPHA, FW_SV_BETA};
+  const fw_sim_t& S = cfg.sim;
+  const char* force_env = getenv("FWGYM_FORCE_GENERIC");
+  const bool force = force_env && force_env[0] == '1';
+  bool rand = false;   // per-env model parameters
+  for (int i = 0; i < FW_PAR_N; ++i)
+    if (S.par_slot1[i]) rand = true;
+  uint32_t clip = 0, cons = 0;
+  for (int r = 0; r <= FW_R_BETA; ++r) {
+    const uint32_t f = S.var[rank_sv[r]].flags;
+    if (f & (FW_VC_VMIN | FW_VC_VMAX)) clip |= FW_RB(r);
+    if (f & (FW_VC_CMIN | FW_VC_CMAX)) cons |= FW_RB(r);
   }
-  if (spec == 0) return launch_dyn<float, FwSpecShipped>(sim, da, grid, s);
-  if (spec == 1) return launch_dyn<float, FwSpecGeneric>(sim, da, grid, s);
-  return launch_dyn<float, FwSpecRand>(sim, da, grid, s);
-}
-static cudaError_t prepare_dyn_any(int precision, int spec, int sms, int n_par_rows, int* grid_out) {
-  if (precision == 0) {
-    if (spec == 0) return prepare_dyn<double, FwSpecShipped>(sms, n_par_rows, grid_out);
-    if (spec == 1) return prepare_dyn<double, FwSpecGeneric>(sms, n_par_rows, grid_out);
-    return prepare_dyn<double, FwSpecRand>(sms, n_par_rows, grid_out);
-  }
-  if (spec == 0) return prepare_dyn<float, FwSpecShipped>(sms, n_par_rows, grid_out);
-  if (spec == 1) return prepare_dyn<float, FwSpecGeneric>(sms, n_par_rows, grid_out);
-  return prepare_dyn<float, FwSpecRand>(sms, n_par_rows, grid_out);
+  for (int i = 0; i < FW_N_ACT; ++i)
+    if (S.act_has_dot_max[i]) clip |= FW_RB(FW_R_AD0 + i);
+  const bool shipped_covers = !(clip & ~FwSpecShipped::clip) && !(cons & ~FwSpecShipped::cons) && !S.wind_enabled &&
+                              S.drag_model == 0;
+  const int spec = rand ? DYN_RAND : (force || !shipped_covers) ? DYN_GENERIC : DYN_SHIPPED;
+  const int shape = force ? -1 : fw_find_shape(cfg.env, cfg.sim);
+  return {&kDynKernels[cfg.precision != 0][spec],
+          &kShapeKernels[shape >= 0 ? shape : kShapeGeneric + (S.turb_mixed != 0)]};
 }
 
 // persistent grid of the handle's attempt kernel: its resident capacity on the device, or FWGYM_ATTEMPT_WARPS_PER_SM
@@ -1103,11 +1073,16 @@ static cudaError_t prepare_dyn_any(int precision, int spec, int sms, int n_par_r
 static int size_attempt_grid(fw_handle h) {
   int sms = 0, g = 0;
   CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-  CK(prepare_dyn_any(h->cfg.precision, h->generic, sms, h->L.n_par_rows, &g));
+  CK(h->dyn->prepare(sms, h->L.n_par_rows, &g));
   const char* e = getenv("FWGYM_ATTEMPT_WARPS_PER_SM");
   if (e && atoi(e) > 0) g = atoi(e) * sms;
   h->attempt_grid = g > 0 ? g : sms;
   return FW_OK;
+}
+
+template <typename T>
+static bool alloc_zeroed(T** p, size_t count) {
+  return cudaMalloc(p, count * sizeof(T)) == cudaSuccess && cudaMemset(*p, 0, count * sizeof(T)) == cudaSuccess;
 }
 
 extern "C" {
@@ -1123,39 +1098,29 @@ int64_t fw_config_sizeof(void) { return (int64_t)sizeof(fw_config_t); }
 static int init_handle(fw_handle h) {
   int rc = make_layout(h->cfg, h->n, h->L);
   if (rc) return rc;
-  const size_t db = (size_t)h->L.d_rows * h->L.stride * sizeof(double);
-  const size_t ib = (size_t)h->L.i_rows * h->L.stride * sizeof(int32_t);
-  if (cudaMalloc(&h->d, db) != cudaSuccess || cudaMalloc(&h->i, ib) != cudaSuccess ||
-      cudaMalloc(&h->ctr, CTR_N * sizeof(unsigned long long)) != cudaSuccess ||
-      cudaMalloc(&h->msum, FW_N_METRIC_SUMS * sizeof(double)) != cudaSuccess)
+  const size_t st = (size_t)h->L.stride;
+  h->q_len = Q_N + blocks(h->L.stride, FW_ENV_BLOCK);
+  if (!alloc_zeroed(&h->d, h->L.d_rows * st) || !alloc_zeroed(&h->i, h->L.i_rows * st) ||
+      !alloc_zeroed(&h->ctr, CTR_N) || !alloc_zeroed(&h->msum, FW_N_METRIC_SUMS))
     return fail(FW_ERR_ALLOC, "cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
-  if (cudaMalloc(&h->carry_d, (size_t)CY_ROWS * h->L.stride * sizeof(double)) != cudaSuccess ||
-      cudaMalloc(&h->carry_i, (size_t)CI_ROWS * h->L.stride * sizeof(int32_t)) != cudaSuccess ||
-      cudaMalloc(&h->long_list, (size_t)h->L.stride * sizeof(int32_t)) != cudaSuccess ||
-      cudaMalloc(&h->queue, (size_t)(h->q_len = Q_N + (h->L.stride + FW_ENV_BLOCK - 1) / FW_ENV_BLOCK) * sizeof(int32_t)) != cudaSuccess)
+  // from here on the kernels keep the queue zeroed (fw_init_kernel)
+  if (!alloc_zeroed(&h->carry_d, CY_ROWS * st) || !alloc_zeroed(&h->carry_i, CI_ROWS * st) ||
+      !alloc_zeroed(&h->long_list, st) || !alloc_zeroed(&h->queue, (size_t)h->q_len))
     return fail(FW_ERR_ALLOC, "cudaMalloc (carry) failed: %s", cudaGetErrorString(cudaGetLastError()));
   if (cudaHostAlloc(&h->err_flag_host, sizeof(int), cudaHostAllocMapped) != cudaSuccess ||
       cudaHostGetDevicePointer(&h->err_flag_dev, h->err_flag_host, 0) != cudaSuccess)
     return fail(FW_ERR_ALLOC, "cudaHostAlloc (error flag) failed: %s", cudaGetErrorString(cudaGetLastError()));
   *h->err_flag_host = 0;
-  CK(cudaMemset(h->queue, 0, (size_t)h->q_len * sizeof(int32_t)));   // from here on the kernels keep it zeroed (fw_init_kernel)
-  CK(cudaMemset(h->carry_d, 0, (size_t)CY_ROWS * h->L.stride * sizeof(double)));
-  CK(cudaMemset(h->carry_i, 0, (size_t)CI_ROWS * h->L.stride * sizeof(int32_t)));
-  {
-    // aircraft whose first dopri5 step is below dt / FWGYM_LONG_DIV need the most attempts (e.g. the 1e-6 start after
-    // a reset): they are started first so that they do not become the tail of the attempt kernel
-    const char* e = getenv("FWGYM_LONG_DIV");
-    h->long_div = e ? atof(e) : 32.0;
-    h->long_h = h->long_div > 0 ? h->cfg.sim.dt / h->long_div : 0.0;
-  }
-  CK(cudaMemset(h->d, 0, db));
-  CK(cudaMemset(h->i, 0, ib));
   if (h->L.n_tl_rows)   // requested levels start at -1: every env draws its level at each reset
-    CK(cudaMemset(h->i + (size_t)h->L.tl_row * h->L.stride, 0xff, (size_t)h->L.stride * sizeof(int32_t)));
-  CK(cudaMemset(h->ctr, 0, CTR_N * sizeof(unsigned long long)));
-  CK(cudaMemset(h->msum, 0, FW_N_METRIC_SUMS * sizeof(double)));
-  h->generic = needs_generic(h->cfg.sim);
-  h->shape = pick_shape(h->cfg);
+    CK(cudaMemset(h->i + (size_t)h->L.tl_row * st, 0xff, st * sizeof(int32_t)));
+  // aircraft whose first dopri5 step is below dt / FWGYM_LONG_DIV need the most attempts (e.g. the 1e-6 start after a
+  // reset): they are started first so that they do not become the tail of the attempt kernel
+  const char* e = getenv("FWGYM_LONG_DIV");
+  h->long_div = e ? atof(e) : 32.0;
+  h->long_h = h->long_div > 0 ? h->cfg.sim.dt / h->long_div : 0.0;
+  const FwKernels k = select_kernels(h->cfg);
+  h->dyn = k.dyn;
+  h->shape = k.shape;
   return size_attempt_grid(h);
 }
 
@@ -1208,9 +1173,10 @@ int fw_set_config(fw_handle h, const fw_config_t* cfg) {
   if (L.d_rows != h->L.d_rows || memcmp(&L, &h->L, sizeof(L)) != 0)
     return fail(FW_ERR_CONFIG, "fw_set_config: new config changes the state layout; create a new handle");
   h->cfg = *cfg;
-  h->shape = pick_shape(h->cfg);
-  if (needs_generic(h->cfg.sim) != h->generic) {
-    h->generic = needs_generic(h->cfg.sim);
+  const FwKernels k = select_kernels(h->cfg);
+  h->shape = k.shape;
+  if (k.dyn != h->dyn) {
+    h->dyn = k.dyn;
     CK(cudaSetDevice(h->device));
     rc = size_attempt_grid(h);
     if (rc) return rc;
@@ -1233,9 +1199,8 @@ int fw_pid_step(fw_handle h, const fw_pid_gains_t* gains, double* integ, const u
   if (k_roll < 0 || k_pitch < 0 || k_va < 0)
     return fail(FW_ERR_CONFIG, "fw_pid_step: the PID controller needs roll, pitch and Va targets");
   CK(cudaSetDevice(h->device));
-  const int grid = (int)((h->n + 127) / 128);
-  fw_pid_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(h->d, h->L.stride, h->n, *gains, h->cfg.sim.dt, k_roll, k_pitch,
-                                                        k_va, integ, reset_mask, actions_out);
+  fw_pid_kernel<<<blocks(h->n, 128), 128, 0, (cudaStream_t)stream>>>(h->d, h->L.stride, h->n, *gains, h->cfg.sim.dt,
+                                                                     k_roll, k_pitch, k_va, integ, reset_mask, actions_out);
   CK(cudaGetLastError());
   return FW_OK;
 }
@@ -1252,8 +1217,7 @@ int fw_launches_per_step(fw_handle h) { return h ? 3 : 0; }
 const char* fw_kernel_variant(fw_handle h) {
   static thread_local char buf[96];
   if (!h) return "";
-  snprintf(buf, sizeof(buf), "dyn=%s env=%s", h->generic == 2 ? "rand" : (h->generic ? "generic" : "shipped"),
-           shape_name(h->shape));
+  snprintf(buf, sizeof(buf), "dyn=%s env=%s", h->dyn->name, h->shape->name);
   return buf;
 }
 int64_t fw_state_rows(fw_handle h) { return h ? h->L.d_rows + h->L.i_rows : 0; }
@@ -1283,16 +1247,28 @@ const char* fw_state_row_name(fw_handle h, int64_t r) {
   return nullptr;
 }
 
+// A full reset and fw_set_state recover from a watchdog error and re-arm the step queue (the kernels keep it zeroed
+// between steps; this covers a step that was abandoned half-way, e.g. after an error)
+static int recover_and_rearm(fw_handle h, cudaStream_t s) {
+  if (poisoned(h)) {
+    CK(cudaDeviceSynchronize());   // nothing of the abandoned step may still be running
+    *h->err_flag_host = 0;
+  }
+  CK(cudaMemsetAsync(h->queue, 0, (size_t)h->q_len * sizeof(int32_t), s));
+  return FW_OK;
+}
+
 int fw_reset(fw_handle h, const uint8_t* mask, const double* init_state, const double* init_target,
              const double* turb_noise, int64_t turb_len, float* obs_out, double* obs64_out, void* stream) {
   if (!h) return fail(FW_ERR_ARG, "null handle");
   if (turb_noise && turb_len <= 0) return fail(FW_ERR_ARG, "fw_reset: turb_noise needs turb_len > 0");
   CK(cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
-  if (*reinterpret_cast<volatile int*>(h->err_flag_host)) {
-    if (mask) CK_POISON(h);                    // only a FULL reset recovers from a watchdog error
-    CK(cudaDeviceSynchronize());               // nothing of the abandoned step may still be running
-    *h->err_flag_host = 0;
+  if (mask) {
+    CK_POISON(h);   // only a FULL reset recovers from a watchdog error
+  } else {
+    const int rc = recover_and_rearm(h, s);
+    if (rc) return rc;
   }
   // injected Dryden noise: kept for the episodes that start here (a partial reset without noise keeps the buffer the
   // other envs may still be reading; a full reset without noise drops it)
@@ -1301,24 +1277,10 @@ int fw_reset(fw_handle h, const uint8_t* mask, const double* init_state, const d
   FwResetArgs a{h->d, h->i, h->n, mask, init_state, init_target, (uint32_t)h->seed, (uint32_t)(h->seed >> 32),
                 (uint32_t)h->offset, obs_out, obs64_out, fw_obs_dim(h), h->ctr,
                 FwTurbInject{turb_noise, turb_len, h->n}};
-  const int grid = (int)((h->n + FW_ENV_BLOCK - 1) / FW_ENV_BLOCK);
-  CK(launch_reset(h->shape, grid, s, h->cfg.env, h->cfg.sim, h->L, a));
-  // a full reset also re-arms the step queue (the kernels keep it zeroed between steps; this covers a step that was
-  // abandoned half-way, e.g. after an error)
-  if (!mask) CK(cudaMemsetAsync(h->queue, 0, (size_t)h->q_len * sizeof(int32_t), s));
+  h->shape->reset<<<blocks(h->n, FW_ENV_BLOCK), FW_ENV_BLOCK, 0, s>>>(h->cfg.env, h->cfg.sim, h->L, a);
+  CK(cudaGetLastError());
   h->last_stream = s;
   return FW_OK;
-}
-
-static int step_impl(fw_handle h, const void* actions, int actions_f64, float* obs_out, float* rew_out, uint8_t* done_out,
-                     int32_t* term_out, double* obs64_out, double* rew64_out, float* term_obs_out, int auto_reset,
-                     void* stream, int stage_obs);
-
-int fw_step(fw_handle h, const void* actions, int actions_f64, float* obs_out, float* rew_out, uint8_t* done_out,
-            int32_t* term_out, double* obs64_out, double* rew64_out, float* term_obs_out, int auto_reset,
-            void* stream) {
-  return step_impl(h, actions, actions_f64, obs_out, rew_out, done_out, term_out, obs64_out, rew64_out, term_obs_out,
-                   auto_reset, stream, 0);
 }
 
 // stage_obs: obs_out is mapped pinned HOST memory (fw_host_open zero-copy mode): observations leave the env kernel as
@@ -1339,7 +1301,7 @@ static int step_impl(fw_handle h, const void* actions, int actions_f64, float* o
     for (int k = 0; k < 3; ++k) { CK(cudaEventCreate(&pe[k])); h->ev.push_back(pe[k]); }
     CK(cudaEventRecord(pe[0], s));
   }
-  CK(launch_dyn_any(h->cfg.precision, h->generic, h->cfg.sim, da, h->attempt_grid, s));
+  CK(h->dyn->launch(h->cfg.sim, da, h->attempt_grid, s));
   if (h->profiling) CK(cudaEventRecord(pe[1], s));
   FwEnvArgs ea{h->d, h->i, h->n, actions, actions_f64, k0, k1, (uint32_t)h->offset, obs_out, rew_out, done_out,
                term_out, obs64_out, rew64_out, term_obs_out, auto_reset, fw_obs_dim(h), h->ctr, h->msum, h->carry_d,
@@ -1347,12 +1309,21 @@ static int step_impl(fw_handle h, const void* actions, int actions_f64, float* o
                h->err_flag_dev, h->spin_limit, h->starve_next,
                (stage_obs && obs_out && (size_t)FW_ENV_BLOCK * fw_obs_dim(h) * sizeof(float) <= 48 * 1024) ? 1 : 0};
   h->starve_next = 0;
-  const int egrid = (int)((h->n + FW_ENV_BLOCK - 1) / FW_ENV_BLOCK);
-  // with per-kernel profiling on, an event sits between the two kernels, so they are serialised anyway
-  CK(launch_env(h->shape, egrid, s, !h->profiling, h->cfg.env, h->cfg.sim, h->L, ea));
+  // a programmatic dependent of the attempt kernel: it synchronises on the per-chunk counters.  With per-kernel
+  // profiling on, an event sits between the two kernels, so they are serialised anyway.
+  CK(launch(h->shape->env, blocks(h->n, FW_ENV_BLOCK), FW_ENV_BLOCK,
+            ea.stage_obs ? (size_t)FW_ENV_BLOCK * ea.obs_dim * sizeof(float) : 0, s, !h->profiling, h->cfg.env,
+            h->cfg.sim, h->L, ea));
   if (h->profiling) CK(cudaEventRecord(pe[2], s));
   h->last_stream = s;
   return FW_OK;
+}
+
+int fw_step(fw_handle h, const void* actions, int actions_f64, float* obs_out, float* rew_out, uint8_t* done_out,
+            int32_t* term_out, double* obs64_out, double* rew64_out, float* term_obs_out, int auto_reset,
+            void* stream) {
+  return step_impl(h, actions, actions_f64, obs_out, rew_out, done_out, term_out, obs64_out, rew64_out, term_obs_out,
+                   auto_reset, stream, 0);
 }
 
 // ---- host-buffer stepping ---------------------------------------------------------------------------------------
@@ -1369,6 +1340,13 @@ static void host_free(fw_handle h) {
   h->hs.clear();
 }
 
+// results of a step in one block [obs | reward | termination code | done]: one device -> host copy per step
+static void carve_results(float* obs, size_t n, size_t od, float** rew, int32_t** term, uint8_t** done) {
+  *rew = obs + n * od;
+  *term = reinterpret_cast<int32_t*>(*rew + n);
+  *done = reinterpret_cast<uint8_t*>(*term + n);
+}
+
 int fw_host_open(fw_handle h, int depth) { return fw_host_open_ex(h, depth, 0); }
 
 int fw_host_open_ex(fw_handle h, int depth, int zero_copy) {
@@ -1383,7 +1361,6 @@ int fw_host_open_ex(fw_handle h, int depth, int zero_copy) {
     fw_handle_s::HostSlot sl = {};
     h->hs.push_back(sl);
     fw_handle_s::HostSlot& r = h->hs.back();
-    // results of a step in one block [obs | reward | termination code | done]: one device -> host copy per step
     r.out_bytes = n * (od * sizeof(float) + sizeof(float) + sizeof(int32_t) + 1);
     r.zero_copy = zero_copy ? 1 : 0;
     bool ok = cudaMalloc(&r.d_act, n * FW_N_ACT * sizeof(float)) == cudaSuccess;
@@ -1400,10 +1377,8 @@ int fw_host_open_ex(fw_handle h, int depth, int zero_copy) {
       host_free(h);
       return fail(FW_ERR_ALLOC, "fw_host_open: allocation failed: %s", msg);
     }
-    r.d_rew = r.d_obs + n * od; r.d_term = reinterpret_cast<int32_t*>(r.d_rew + n);
-    r.d_done = reinterpret_cast<uint8_t*>(r.d_term + n);
-    r.h_rew = r.h_obs + n * od; r.h_term = reinterpret_cast<int32_t*>(r.h_rew + n);
-    r.h_done = reinterpret_cast<uint8_t*>(r.h_term + n);
+    carve_results(r.d_obs, n, od, &r.d_rew, &r.d_term, &r.d_done);
+    carve_results(r.h_obs, n, od, &r.h_rew, &r.h_term, &r.h_done);
   }
   return FW_OK;
 }
@@ -1514,8 +1489,8 @@ int fw_get_rows(fw_handle h, int64_t row0, int64_t nrows, double* out, void* str
   if (!h || !out) return fail(FW_ERR_ARG, "null argument");
   if (row0 < 0 || nrows < 0 || row0 + nrows > h->L.d_rows + h->L.i_rows) return fail(FW_ERR_ARG, "fw_get_rows: row range");
   CK(cudaSetDevice(h->device));
-  const int grid = (int)((h->n + 255) / 256);
-  fw_export_rows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->d, h->i, h->L.stride, h->n, h->L.d_rows, row0, nrows, out);
+  fw_export_rows_kernel<<<blocks(h->n, 256), 256, 0, (cudaStream_t)stream>>>(h->d, h->i, h->L.stride, h->n, h->L.d_rows,
+                                                                             row0, nrows, out);
   CK(cudaGetLastError());
   return FW_OK;
 }
@@ -1528,24 +1503,16 @@ int fw_debug_watchdog(fw_handle h, uint32_t spin_limit, int starve) {
 }
 
 int fw_get_state(fw_handle h, double* out, void* stream) {
-  if (!h || !out) return fail(FW_ERR_ARG, "null argument");
-  CK(cudaSetDevice(h->device));
-  const int grid = (int)((h->n + 255) / 256);
-  fw_export_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->d, h->i, h->L.stride, h->n, h->L.d_rows, h->L.i_rows, out);
-  CK(cudaGetLastError());
-  return FW_OK;
+  return fw_get_rows(h, 0, fw_state_rows(h), out, stream);
 }
 
 int fw_set_state(fw_handle h, const double* in, void* stream) {
   if (!h || !in) return fail(FW_ERR_ARG, "null argument");
   CK(cudaSetDevice(h->device));
-  if (*reinterpret_cast<volatile int*>(h->err_flag_host)) {   // restoring a checkpoint recovers from a watchdog error
-    CK(cudaDeviceSynchronize());
-    *h->err_flag_host = 0;
-  }
-  const int grid = (int)((h->n + 255) / 256);
-  fw_import_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->d, h->i, h->L.stride, h->n, h->L.d_rows, h->L.i_rows, in);
-  CK(cudaMemsetAsync(h->queue, 0, (size_t)h->q_len * sizeof(int32_t), (cudaStream_t)stream));   // re-arm the step queue
+  const int rc = recover_and_rearm(h, (cudaStream_t)stream);
+  if (rc) return rc;
+  fw_import_kernel<<<blocks(h->n, 256), 256, 0, (cudaStream_t)stream>>>(h->d, h->i, h->L.stride, h->n, h->L.d_rows,
+                                                                        h->L.i_rows, in);
   CK(cudaGetLastError());
   return FW_OK;
 }
@@ -1556,8 +1523,7 @@ int fw_set_turbulence_levels(fw_handle h, const int32_t* levels, void* stream) {
     return fail(FW_ERR_ARG, "fw_set_turbulence_levels: the handle flies one turbulence intensity (configure "
                             "turbulence_intensity as {\"values\": [...], \"probabilities\": [...]})");
   CK(cudaSetDevice(h->device));
-  const int grid = (int)((h->n + 255) / 256);
-  fw_set_levels_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->i + (size_t)h->L.tl_row * h->L.stride, h->n, levels);
+  fw_set_levels_kernel<<<blocks(h->n, 256), 256, 0, (cudaStream_t)stream>>>(h->i + (size_t)h->L.tl_row * h->L.stride, h->n, levels);
   CK(cudaGetLastError());
   return FW_OK;
 }
@@ -1565,10 +1531,9 @@ int fw_set_turbulence_levels(fw_handle h, const int32_t* levels, void* stream) {
 int fw_last_attempts(fw_handle h, int32_t* out, void* stream) {
   if (!h || !out) return fail(FW_ERR_ARG, "null argument");
   CK(cudaSetDevice(h->device));
-  const int grid = (int)((h->n + 255) / 256);
   // the carry row, not I_LASTK: an env that finished in the step was reset on the spot (I_LASTK = 0), the carry row still
   // holds the attempts of the step that ended its episode (incl. the attempt a ConstraintException cut short)
-  fw_gather_i32_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->carry_i, h->L.stride, h->n, CI_ATTEMPTS, out);
+  fw_gather_i32_kernel<<<blocks(h->n, 256), 256, 0, (cudaStream_t)stream>>>(h->carry_i, h->L.stride, h->n, CI_ATTEMPTS, out);
   CK(cudaGetLastError());
   return FW_OK;
 }

@@ -370,7 +370,7 @@ int64_t fw_num_envs(fw_handle h);
 int fw_obs_dim(fw_handle h);
 /* Kernel launches one fw_step issues: init, attempt and env kernel. */
 int fw_launches_per_step(fw_handle h);
-/* Which kernel instantiations this handle's configuration selected: "dyn=<shipped|generic> env=<shape name|generic>"
+/* Which kernel instantiations this handle's configuration selected: "dyn=<shipped|generic|rand> env=<shape name|generic>"
  * (dynamics.cuh "kernel specialisation", env_shapes.h).  Valid until the next call on the calling thread. */
 const char* fw_kernel_variant(fw_handle h);
 
