@@ -29,6 +29,8 @@ if __name__ == "__main__":
     ap.add_argument("--env-config-path", help="env configuration JSON (default: the examples configuration)")
     ap.add_argument("--turbulence-intensity", nargs="+", default=["none"], choices=["none", "light", "moderate", "severe"],
                     help="one or more levels; several levels run as one batch (a result table per level)")
+    ap.add_argument("--num-envs", type=int, help="fly the scenarios on this many envs, each taking scenario after "
+                    "scenario (default: one env per scenario and level)")
     ap.add_argument("--save", help="write the result dictionary to this .npy")
     a = ap.parse_args()
     if not a.use_pid and not a.model_path:
@@ -42,7 +44,8 @@ if __name__ == "__main__":
     controller = "pid" if a.use_pid else dict(np.load(a.model_path))
     levels = a.turbulence_intensity
     res, vec = evaluate.evaluate_on_set(scenarios, cfg, controller=controller,
-                                        turbulence_intensity=levels[0] if len(levels) == 1 else levels)
+                                        turbulence_intensity=levels[0] if len(levels) == 1 else levels,
+                                        num_envs=a.num_envs)
     by_level = {levels[0]: res} if len(levels) == 1 else res
     saved = {}
     for lv, r in by_level.items():

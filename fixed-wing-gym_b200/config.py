@@ -174,7 +174,7 @@ class CompiledConfig:
     """Holds the (mutable) parsed JSON configs, mirrors FixedWingAircraft's derived attributes and produces the POD."""
 
     def __init__(self, config_path=None, sim_config_path=None, sim_parameter_path=None, config_kw=None,
-                 sim_config_kw=None, precision="fp64", metrics=False):
+                 sim_config_kw=None, precision="fp64", metrics=False, scenario_bank=False):
         config_path = config_path or DEFAULT_ENV_CONFIG
         with open(config_path) as f:
             self.cfg = json.load(f)
@@ -195,6 +195,7 @@ class CompiledConfig:
             self.params = {k: v for k, v in json.load(f).items() if not k.startswith("_")}
         self.precision = {"fp64": 0, "fp32": 1}[precision]
         self.metrics = bool(metrics)   # stream the get_metric quantities on the device (fixed_wing.py:1095-1162)
+        self.scenario_bank = bool(scenario_bank)   # keep the scenario-bank rows (fw_set_bank)
         self.state = {v["name"]: SimVariable(v) for v in self.sim_cfg["variables"]}
         self.dt = self.sim_cfg["dt"]
         self._check_supported()
@@ -756,3 +757,4 @@ class CompiledConfig:
                 F.has_max, F.max = 1, float(comp["max"])
             F.sign = float(np.sign(comp.get("sign", -1)))
         e.n_scale_rows = n_scale
+        e.bank_enabled = 1 if self.scenario_bank else 0

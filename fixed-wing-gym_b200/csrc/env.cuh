@@ -499,6 +499,26 @@ __device__ __forceinline__ void fw_turb_noise_injected(const fw_sim_t& P, const 
   for (int j = 0; j < 4; ++j) u[j] = ti.noise[((int64_t)j * ti.len + col) * ti.n + env] * P.turb_noise_scale;
 }
 
+// Scenario bank as the kernels see it (fw_set_bank, include/fwgym.h fw_bank_t); n = 0: none attached
+struct FwBank {
+  const double* init_state;   // [FW_N_SV + 3, n]
+  const double* init_target;  // [FW_MAX_TARGETS, n]
+  const int32_t* turb_level;  // [n]
+  int64_t n, stride;
+  int32_t cycle, _pad;
+  int32_t* term;              // result rows [n] (all optional)
+  int32_t* length;
+  double* ret;
+  double* episode;            // [n, ep_dim]
+  int32_t* episodes;
+  int32_t* successes;
+};
+// the scenario after `cur` for the same env: + stride, modulo n when cycling, else saturating at n (past the bank)
+__device__ __forceinline__ int32_t fw_bank_advance(const FwBank& b, int32_t cur) {
+  const int64_t nx = (int64_t)cur + b.stride;
+  return (int32_t)(b.cycle ? nx % b.n : (nx < b.n ? nx : b.n));
+}
+
 // advance the six shaping filters by one sample (scipy lsim recurrence) and refresh the gust rows.  The host zero-pads
 // Ad / Bd0 / Bd1 / C of filters of order < 3 (config.py), so the generic loops are fixed-size and everything stays in
 // registers; a fixed shape knows each filter's order and skips the padding (whose states stay exactly zero).
@@ -679,18 +699,38 @@ __device__ __forceinline__ void fw_reset_env_body(const fw_env_t& E, const fw_si
                                                   uint32_t k0, uint32_t k1, uint32_t genv,
                                                   const double* __restrict__ init_state,
                                                   const double* __restrict__ init_target, int64_t in_stride,
-                                                  const FwTurbInject ti, const FwObsWriter& out) {
+                                                  const FwTurbInject ti, const FwObsWriter& out,
+                                                  const FwBank bank = FwBank{}) {
   FW_SHAPE_REFS;
   const uint32_t tick = (uint32_t)c.I(I_TICK);
-  if constexpr (COOP) __syncwarp();     // every lane has read the counter before any lane overwrites it
+  // scenario bank: a reset that injects nothing starts the env's next scenario while there is one (-1: none)
+  int32_t scen = -1;
+  if constexpr (SH::bank) {
+    const int32_t cur = c.I(Ls.bank_row);
+    if (!init_state && !init_target && cur < bank.n) scen = cur;
+  }
+  if constexpr (COOP) __syncwarp();     // every lane has read the counters before any lane overwrites them
   c.I(I_TICK) = (int32_t)(tick + 1u);
   c.I(I_EPTICK) = (int32_t)tick;
+  int64_t col = c.env;                  // column of init_state / init_target (bank shapes)
+  if constexpr (SH::bank) {
+    if (scen >= 0) {
+      c.I(Ls.bank_row) = fw_bank_advance(bank, scen);
+      init_state = bank.init_state;
+      init_target = bank.init_target;
+      in_stride = bank.n;
+      col = scen;
+    }
+    c.I(Ls.bank_row + 1) = scen;
+  }
   FwRng g{k0, k1, genv, tick};
   if constexpr (COOP) fw_rng_fill_bank(g);
   int dummy = 0;
   auto given = [&](int r, double& v) -> bool {
     if (!init_state) return false;
-    v = init_state[(int64_t)r * in_stride + c.env];
+    // (a bank shape reads the scenario's column; the others keep the code they had before the bank existed)
+    if constexpr (SH::bank) v = init_state[(int64_t)r * in_stride + col];
+    else v = init_state[(int64_t)r * in_stride + c.env];
     return !isnan(v);
   };
   auto init_var = [&](int sv) -> double {
@@ -738,7 +778,13 @@ __device__ __forceinline__ void fw_reset_env_body(const fw_env_t& E, const fw_si
   // level 0 (none) then takes exactly the path of a handle without turbulence
   int tlvl = 0;
   if constexpr (SH::mixed) {
-    const int req = c.I(Ls.tl_row);
+    int req = c.I(Ls.tl_row);
+    if constexpr (SH::bank) {   // the scenario's level column pins the episode's level
+      if (scen >= 0 && bank.turb_level) {
+        const int bl = bank.turb_level[scen];
+        if (bl >= 0 && bl < FW_N_TURB_LEVELS) req = bl;
+      }
+    }
     if (req >= 0) {
       tlvl = req;
     } else {
@@ -821,7 +867,9 @@ __device__ __forceinline__ void fw_reset_env_body(const fw_env_t& E, const fw_si
   fw_sample_target<SH>(E, c, rng, flags, 0);
   if (init_target) {
     for (int k = 0; k < Es.n_targets; ++k) {
-      const double v = init_target[(int64_t)k * in_stride + c.env];
+      double v;
+      if constexpr (SH::bank) v = init_target[(int64_t)k * in_stride + col];
+      else v = init_target[(int64_t)k * in_stride + c.env];
       if (isnan(v)) continue;
       const int cls = fw_tcls(flags, k);
       if (cls != 0 && cls != 3) flags &= ~(3u << (FWF_TCLS_SHIFT + 2 * k));
@@ -876,4 +924,13 @@ __device__ __noinline__ void fw_reset_env(const fw_env_t& E, const fw_sim_t& P, 
                                           const double* __restrict__ init_target, int64_t in_stride,
                                           const FwTurbInject ti, const FwObsWriter& out) {
   fw_reset_env_body<SH, false>(E, P, L, c, k0, k1, genv, init_state, init_target, in_stride, ti, out);
+}
+// ... and its twin for bank shapes (the bank by value: see fw_turb_noise_injected)
+template <class SH>
+__device__ __noinline__ void fw_reset_env_bank(const fw_env_t& E, const fw_sim_t& P, const FwLayout& L, const FwEnvCtx& c,
+                                               uint32_t k0, uint32_t k1, uint32_t genv,
+                                               const double* __restrict__ init_state,
+                                               const double* __restrict__ init_target, int64_t in_stride,
+                                               const FwTurbInject ti, const FwObsWriter& out, const FwBank bank) {
+  fw_reset_env_body<SH, false>(E, P, L, c, k0, k1, genv, init_state, init_target, in_stride, ti, out, bank);
 }

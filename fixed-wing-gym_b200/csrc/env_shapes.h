@@ -19,9 +19,14 @@
 // `mixed`: the configuration flies each env at its own Dryden intensity (fw_sim_t.turb_mixed).  A compile-time property
 // of every shape, so that the per-env level code exists only in the instantiations that need it: the generic kernels
 // come in two instantiations, FwShapeGeneric (one intensity for the whole handle) and FwShapeGenericMixed.
+//
+// `bank`: the handle keeps the scenario-bank rows (fw_env_t.bank_enabled, fw_set_bank).  Also compile-time, so that the
+// instantiations without it compile to exactly the code they compiled to before the bank existed: two more generic
+// instantiations, FwShapeGenericBank and FwShapeGenericMixedBank.
 struct FwShapeGeneric {
   static constexpr bool fixed = false;
   static constexpr bool mixed = false;
+  static constexpr bool bank = false;
   static constexpr fw_env_t cenv{};
   static __device__ __forceinline__ const fw_env_t& env(const fw_env_t& E) { return E; }
   static __device__ __forceinline__ const fw_sim_t& sim(const fw_sim_t& P) { return P; }
@@ -29,6 +34,13 @@ struct FwShapeGeneric {
 };
 struct FwShapeGenericMixed : FwShapeGeneric {
   static constexpr bool mixed = true;
+};
+struct FwShapeGenericBank : FwShapeGeneric {
+  static constexpr bool bank = true;
+};
+struct FwShapeGenericMixedBank : FwShapeGeneric {
+  static constexpr bool mixed = true;
+  static constexpr bool bank = true;
 };
 
 constexpr FwLayout fw_shape_layout(const fw_env_t& e, const fw_sim_t& s) {
@@ -44,6 +56,7 @@ constexpr FwLayout fw_shape_layout(const fw_env_t& e, const fw_sim_t& s) {
   struct FwShape_##NAME {                                                                                  \
     static constexpr bool fixed = true;                                                                    \
     static constexpr bool mixed = fw_shape_sim_##NAME().turb_mixed != 0;                                   \
+    static constexpr bool bank = fw_shape_env_##NAME().bank_enabled != 0;                                  \
     static constexpr fw_env_t cenv = fw_shape_env_##NAME();   /* for constant expressions (loop trip counts) */ \
     static __device__ __forceinline__ const fw_env_t& env(const fw_env_t&) { return kShapeEnv_##NAME; }    \
     static __device__ __forceinline__ const fw_sim_t& sim(const fw_sim_t&) { return kShapeSim_##NAME; }    \
@@ -100,7 +113,7 @@ inline bool fw_env_same_shape(const fw_env_t& a, const fw_env_t& b) {
       a.streak_req != b.streak_req || a.n_factors != b.n_factors ||
       a.potential != b.potential || a.step_fail_timesteps != b.step_fail_timesteps || a.n_terms != b.n_terms ||
       a.metrics_enabled != b.metrics_enabled || a.n_rand != b.n_rand || a.n_par_rows != b.n_par_rows ||
-      a.n_scale_rows != b.n_scale_rows)
+      a.n_scale_rows != b.n_scale_rows || a.bank_enabled != b.bank_enabled)
     return false;
   for (int v = 0; v < a.obs_nvar; ++v) {
     const fw_obs_var_t &x = a.obs[v], &y = b.obs[v];

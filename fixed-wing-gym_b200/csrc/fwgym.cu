@@ -56,6 +56,7 @@ struct fw_handle_s {
   double* ep_out;                // caller's episode-metric buffer (fw_set_episode_out)
   const double* turb_noise;      // caller's injected Dryden noise [4, turb_len, n] (fw_reset), NULL: Philox streams
   int64_t turb_len;
+  FwBank bank;                   // attached scenario bank (fw_set_bank; n = 0: none)
   int* err_flag_host;            // mapped pinned word the env kernel raises when a block's chunk wait times out
   int* err_flag_dev;             //   (device alias); non-zero = the handle refuses to step (FW_ERR_WATCHDOG)
   uint32_t spin_limit;           // polls before an env block gives up (fw_debug_watchdog; default ~1 s)
@@ -531,6 +532,7 @@ struct FwEnvArgs {
   uint32_t spin_limit;
   int32_t starve;      // test hook (fw_debug_watchdog)
   int32_t stage_obs;   // float32 observations through a shared-memory tile (dynamic smem: FW_ENV_BLOCK * obs_dim floats)
+  FwBank bank;         // scenario bank (bank shapes only; appended: no earlier parameter moves)
 };
 
 // Env-side work of one env step for env `env` (fixed_wing.py:338-437 after the simulator call).  Episode-metric
@@ -678,6 +680,23 @@ __device__ __forceinline__ void fw_env_step(const fw_env_t& E, const fw_sim_t& P
     if (term == FW_TERM_STEPS) m[MS_STEPS_TERM] += 1.0;
     if (term == FW_TERM_SUCCESS) m[MS_SUCCESS_TERM] += 1.0;
   }
+  if constexpr (SH::bank) {   // a banked episode ended: its scenario's result rows (never at or beyond n)
+    if (done) {
+      const int32_t scen = c.I(Ls.bank_row + 1);
+      if (scen >= 0) {
+        const FwBank& b = a.bank;
+        if (scen < b.n) {
+          if (b.term) b.term[scen] = term;
+          if (b.length) b.length[scen] = steps;
+          if (b.ret) b.ret[scen] = epret;
+          if (Ls.met && b.episode) fw_metrics_finish(E, P, L, c, hist_len, steps, epret, b.episode + scen * (int64_t)a.ep_dim);
+          if (b.episodes) atomicAdd(b.episodes + scen, 1);
+          if (b.successes && (flags & FWF_EP_SUCCESS)) atomicAdd(b.successes + scen, 1);
+        }
+        c.I(Ls.bank_row + 1) = -1;
+      }
+    }
+  }
   if (do_reset) n_reset += 1;
   need_reset = do_reset;   // the reset itself is run by the whole warp together (fw_env_kernel)
 }
@@ -801,8 +820,12 @@ fw_env_kernel(const __grid_constant__ fw_env_t E, const __grid_constant__ fw_sim
       FwObsWriter ow{a.stage_obs ? fw_env_tile : a.obs_out, a.obs64_out, env_l * (int64_t)a.obs_dim,
                      a.stage_obs ? (int64_t)tid_l * a.obs_dim : (int64_t)-1};
       ow.commit = lane == leader;
-      fw_reset_env_body<SH, true>(E, P, L, c, a.k0, a.k1, a.env_offset + (uint32_t)env_l, nullptr, nullptr, 0,
-                                  FwTurbInject{nullptr, 0, 0}, ow);
+      if constexpr (SH::bank)
+        fw_reset_env_body<SH, true>(E, P, L, c, a.k0, a.k1, a.env_offset + (uint32_t)env_l, nullptr, nullptr, 0,
+                                    FwTurbInject{nullptr, 0, 0}, ow, a.bank);
+      else
+        fw_reset_env_body<SH, true>(E, P, L, c, a.k0, a.k1, a.env_offset + (uint32_t)env_l, nullptr, nullptr, 0,
+                                    FwTurbInject{nullptr, 0, 0}, ow);
       __syncwarp();
     }
   }
@@ -855,6 +878,12 @@ struct FwResetArgs {
   unsigned long long* ctr;
   FwTurbInject ti;
 };
+// the explicit reset of a bank shape: the same arguments and the scenario bank (a struct of its own, so that the reset
+// kernels of the other shapes keep their parameter block and their code)
+struct FwResetBankArgs {
+  FwResetArgs r;
+  FwBank bank;
+};
 
 template <class SH>
 __global__ void __launch_bounds__(FW_ENV_BLOCK)
@@ -868,18 +897,32 @@ fw_reset_kernel(const __grid_constant__ fw_env_t E, const __grid_constant__ fw_s
   atomicAdd(a.ctr + CTR_RESETS, 1ull);
   fw_reset_env<SH>(E, P, L, c, a.k0, a.k1, a.env_offset + (uint32_t)env, a.init_state, a.init_target, a.n, a.ti, ow);
 }
+template <class SH>
+__global__ void __launch_bounds__(FW_ENV_BLOCK)
+fw_reset_bank_kernel(const __grid_constant__ fw_env_t E, const __grid_constant__ fw_sim_t P,
+                     const __grid_constant__ FwLayout L, const FwResetBankArgs ab) {
+  const FwResetArgs& a = ab.r;
+  const int64_t env = (int64_t)blockIdx.x * FW_ENV_BLOCK + threadIdx.x;
+  if (env >= a.n) return;
+  if (a.mask && !a.mask[env]) return;
+  FwEnvCtx c{a.d, a.i, L.stride, env};
+  FwObsWriter ow{a.obs_out, a.obs64_out, env * (int64_t)a.obs_dim, -1};
+  atomicAdd(a.ctr + CTR_RESETS, 1ull);
+  fw_reset_env_bank<SH>(E, P, L, c, a.k0, a.k1, a.env_offset + (uint32_t)env, a.init_state, a.init_target, a.n, a.ti, ow,
+                        ab.bank);
+}
 
 // Kernel parameters are limited to 32 764 bytes (CUDA 12.1+ on Volta and later).  The configuration travels as
 // __grid_constant__ parameters, so its size is bounded here (the per-level Dryden tables of fw_sim_t count against it);
 // 64 bytes cover the alignment padding between the parameters.
 static_assert(sizeof(fw_env_t) + sizeof(fw_sim_t) + sizeof(FwLayout) + sizeof(FwEnvArgs) + 64 <= 32764,
               "env kernel parameters exceed the 32 764-byte limit");
-static_assert(sizeof(fw_env_t) + sizeof(fw_sim_t) + sizeof(FwLayout) + sizeof(FwResetArgs) + 64 <= 32764,
+static_assert(sizeof(fw_env_t) + sizeof(fw_sim_t) + sizeof(FwLayout) + sizeof(FwResetBankArgs) + 64 <= 32764,
               "reset kernel parameters exceed the 32 764-byte limit");
 static_assert(sizeof(FwSimX) + sizeof(FwDynArgs) + 64 <= 32764, "fp32 dynamics kernel parameters exceed the 32 764-byte limit");
 static_assert(sizeof(fw_sim_t) + sizeof(FwDynArgs) + 64 <= 32764, "fp64 dynamics kernel parameters exceed the 32 764-byte limit");
 // the per-level Dryden tables were appended without moving any later kernel parameter off its 16-byte alignment
-static_assert(sizeof(fw_sim_t) % 32 == 24 && sizeof(FwLayout) % 16 == 8, "see fw_sim_t._pad_turb / FwLayout._pad_tl");
+static_assert(sizeof(fw_sim_t) % 32 == 24 && sizeof(FwLayout) % 16 == 8, "see fw_sim_t._pad_turb / FwLayout.bank_row");
 
 // ---- PID baseline controller (pyfly/pid_controller.py; evaluate_controller.py:141-151) ---------------------------
 __global__ void fw_pid_kernel(const double* __restrict__ d, int64_t stride, int64_t n, const fw_pid_gains_t g, double dt,
@@ -922,6 +965,15 @@ __global__ void fw_set_levels_kernel(int32_t* row, int64_t n, const int32_t* __r
   if (env >= n) return;
   const int32_t v = levels ? levels[env] : -1;
   row[env] = (v < -1 || v > 3) ? -1 : v;
+}
+// scenario-bank cursors at attach: bank_next = first + e (mod n when cycling, else at most n), no running scenario
+__global__ void fw_bank_attach_kernel(int32_t* next, int32_t* scen, int64_t n_envs, int64_t first, int64_t n_scen,
+                                      int cycle) {
+  const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (env >= n_envs) return;
+  const int64_t c = first + env;
+  next[env] = (int32_t)(n_scen <= 0 ? 0 : cycle ? c % n_scen : (c < n_scen ? c : n_scen));
+  scen[env] = -1;
 }
 __global__ void fw_gather_i32_kernel(const int32_t* i, int64_t stride, int64_t n, int row, int32_t* out) {
   const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1022,19 +1074,30 @@ static const FwDynEntry kDynKernels[2][3] = {   // [fw_config_t.precision: fp64,
      FW_DYN_ENTRY(float, FwSpecRand, "rand")}};
 #undef FW_DYN_ENTRY
 
+using FwResetKernel = void (*)(fw_env_t, fw_sim_t, FwLayout, FwResetArgs);
+using FwResetBankKernel = void (*)(fw_env_t, fw_sim_t, FwLayout, FwResetBankArgs);
 struct FwShapeEntry {
   const char* name;
   void (*env)(fw_env_t, fw_sim_t, FwLayout, FwEnvArgs);
-  void (*reset)(fw_env_t, fw_sim_t, FwLayout, FwResetArgs);
+  FwResetKernel reset;             // shapes without a bank
+  FwResetBankKernel reset_bank;    // bank shapes
 };
-// FW_SHAPE_LIST in fw_find_shape's order, then the two table-walking instantiations (env_shapes.h)
-#define FW_SHAPE_ENTRY(NAME) {#NAME, fw_env_kernel<FwShape_##NAME>, fw_reset_kernel<FwShape_##NAME>},
+template <class SH>
+constexpr FwShapeEntry fw_shape_entry(const char* name) {
+  if constexpr (SH::bank) return {name, fw_env_kernel<SH>, nullptr, fw_reset_bank_kernel<SH>};
+  else return {name, fw_env_kernel<SH>, fw_reset_kernel<SH>, nullptr};
+}
+// FW_SHAPE_LIST in fw_find_shape's order, then the four table-walking instantiations (env_shapes.h)
+#define FW_SHAPE_ENTRY(NAME) fw_shape_entry<FwShape_##NAME>(#NAME),
 static const FwShapeEntry kShapeKernels[] = {
     FW_SHAPE_LIST(FW_SHAPE_ENTRY)
-    {"generic", fw_env_kernel<FwShapeGeneric>, fw_reset_kernel<FwShapeGeneric>},
-    {"generic", fw_env_kernel<FwShapeGenericMixed>, fw_reset_kernel<FwShapeGenericMixed>}};
+    fw_shape_entry<FwShapeGeneric>("generic"),
+    fw_shape_entry<FwShapeGenericMixed>("generic"),
+    fw_shape_entry<FwShapeGenericBank>("generic_bank"),
+    fw_shape_entry<FwShapeGenericMixedBank>("generic_bank")};
 #undef FW_SHAPE_ENTRY
-static constexpr int kShapeGeneric = sizeof(kShapeKernels) / sizeof(kShapeKernels[0]) - 2;
+// first of the four table-walking entries: + 1 mixed, + 2 bank
+static constexpr int kShapeGeneric = sizeof(kShapeKernels) / sizeof(kShapeKernels[0]) - 4;
 
 struct FwKernels {
   const FwDynEntry* dyn;
@@ -1065,7 +1128,7 @@ static FwKernels select_kernels(const fw_config_t& cfg) {
   const int spec = rand ? DYN_RAND : (force || !shipped_covers) ? DYN_GENERIC : DYN_SHIPPED;
   const int shape = force ? -1 : fw_find_shape(cfg.env, cfg.sim);
   return {&kDynKernels[cfg.precision != 0][spec],
-          &kShapeKernels[shape >= 0 ? shape : kShapeGeneric + (S.turb_mixed != 0)]};
+          &kShapeKernels[shape >= 0 ? shape : kShapeGeneric + (S.turb_mixed != 0) + 2 * (cfg.env.bank_enabled != 0)]};
 }
 
 // persistent grid of the handle's attempt kernel: its resident capacity on the device, or FWGYM_ATTEMPT_WARPS_PER_SM
@@ -1243,6 +1306,8 @@ const char* fw_state_row_name(fw_handle h, int64_t r) {
   if (r < I_GOALRING) return in[r];
   if (h->L.n_tl_rows && r == h->L.tl_row) return "turb_level_req";
   if (h->L.n_tl_rows && r == h->L.tl_row + 1) return "turb_level";
+  if (h->L.n_bank_rows && r == h->L.bank_row) return "bank_next";
+  if (h->L.n_bank_rows && r == h->L.bank_row + 1) return "bank_scenario";
   if (r < h->L.i_rows) return in[I_GOALRING];
   return nullptr;
 }
@@ -1277,7 +1342,11 @@ int fw_reset(fw_handle h, const uint8_t* mask, const double* init_state, const d
   FwResetArgs a{h->d, h->i, h->n, mask, init_state, init_target, (uint32_t)h->seed, (uint32_t)(h->seed >> 32),
                 (uint32_t)h->offset, obs_out, obs64_out, fw_obs_dim(h), h->ctr,
                 FwTurbInject{turb_noise, turb_len, h->n}};
-  h->shape->reset<<<blocks(h->n, FW_ENV_BLOCK), FW_ENV_BLOCK, 0, s>>>(h->cfg.env, h->cfg.sim, h->L, a);
+  if (h->shape->reset_bank)
+    h->shape->reset_bank<<<blocks(h->n, FW_ENV_BLOCK), FW_ENV_BLOCK, 0, s>>>(h->cfg.env, h->cfg.sim, h->L,
+                                                                             FwResetBankArgs{a, h->bank});
+  else
+    h->shape->reset<<<blocks(h->n, FW_ENV_BLOCK), FW_ENV_BLOCK, 0, s>>>(h->cfg.env, h->cfg.sim, h->L, a);
   CK(cudaGetLastError());
   h->last_stream = s;
   return FW_OK;
@@ -1307,7 +1376,8 @@ static int step_impl(fw_handle h, const void* actions, int actions_f64, float* o
                term_out, obs64_out, rew64_out, term_obs_out, auto_reset, fw_obs_dim(h), h->ctr, h->msum, h->carry_d,
                h->carry_i, h->ep_out, fw_episode_dim(h), h->queue, FwTurbInject{h->turb_noise, h->turb_len, h->n},
                h->err_flag_dev, h->spin_limit, h->starve_next,
-               (stage_obs && obs_out && (size_t)FW_ENV_BLOCK * fw_obs_dim(h) * sizeof(float) <= 48 * 1024) ? 1 : 0};
+               (stage_obs && obs_out && (size_t)FW_ENV_BLOCK * fw_obs_dim(h) * sizeof(float) <= 48 * 1024) ? 1 : 0,
+               h->bank};
   h->starve_next = 0;
   // a programmatic dependent of the attempt kernel: it synchronises on the per-chunk counters.  With per-kernel
   // profiling on, an event sits between the two kernels, so they are serialised anyway.
@@ -1525,6 +1595,33 @@ int fw_set_turbulence_levels(fw_handle h, const int32_t* levels, void* stream) {
   CK(cudaSetDevice(h->device));
   fw_set_levels_kernel<<<blocks(h->n, 256), 256, 0, (cudaStream_t)stream>>>(h->i + (size_t)h->L.tl_row * h->L.stride, h->n, levels);
   CK(cudaGetLastError());
+  return FW_OK;
+}
+
+int fw_set_bank(fw_handle h, const fw_bank_t* b, void* stream) {
+  if (!h) return fail(FW_ERR_ARG, "null handle");
+  if (!h->L.n_bank_rows)
+    return fail(FW_ERR_ARG, "fw_set_bank: the handle was not created with a scenario bank (fw_env_t.bank_enabled)%s", "");
+  FwBank k{};
+  if (b) {
+    if (b->n_scenarios <= 0 || b->n_scenarios > INT32_MAX) return fail(FW_ERR_ARG, "fw_set_bank: n_scenarios out of 1..INT32_MAX%s", "");
+    if (b->first < 0) return fail(FW_ERR_ARG, "fw_set_bank: first < 0%s", "");
+    if (b->stride < h->n) return fail(FW_ERR_ARG, "fw_set_bank: stride < n_envs (two envs could fly one scenario)%s", "");
+    if (b->episode && !h->cfg.env.metrics_enabled)
+      return fail(FW_ERR_ARG, "fw_set_bank: an episode buffer needs metrics enabled in the configuration%s", "");
+    if (b->cycle && (b->term || b->length || b->ret || b->episode))
+      return fail(FW_ERR_ARG, "fw_set_bank: a cycling bank has no per-scenario outcome rows (only the counters)%s", "");
+    if (b->turb_level && !h->L.n_tl_rows)
+      return fail(FW_ERR_ARG, "fw_set_bank: a level column needs a handle with per-env turbulence levels%s", "");
+    k = FwBank{b->init_state, b->init_target, b->turb_level, b->n_scenarios, b->stride, b->cycle ? 1 : 0, 0,
+               b->term, b->length, b->ret, b->episode, b->episodes, b->successes};
+  }
+  CK(cudaSetDevice(h->device));
+  const size_t st = (size_t)h->L.stride;
+  fw_bank_attach_kernel<<<blocks(h->n, 256), 256, 0, (cudaStream_t)stream>>>(
+      h->i + (size_t)h->L.bank_row * st, h->i + (size_t)(h->L.bank_row + 1) * st, h->n, b ? b->first : 0, k.n, k.cycle);
+  CK(cudaGetLastError());
+  h->bank = k;
   return FW_OK;
 }
 

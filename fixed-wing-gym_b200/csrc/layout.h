@@ -68,9 +68,12 @@ struct FwLayout {
   // per-env reward scalings (reward.randomize_scaling): n_rs_rows rows starting at rs_row
   int32_t rs_row, n_rs_rows;
   // per-env Dryden intensity (only when fw_sim_t.turb_mixed): int32 rows tl_row (requested level, -1 = draw at every
-  // reset) and tl_row + 1 (level of the running episode); n_tl_rows = 0 or 2.  (_pad_tl: the struct grows by 16 bytes,
-  // so the kernel parameters after it keep their 16-byte alignment and the compiler its 128-bit constant loads.)
-  int32_t tl_row, n_tl_rows, _pad_tl[2];
+  // reset) and tl_row + 1 (level of the running episode); n_tl_rows = 0 or 2
+  int32_t tl_row, n_tl_rows;
+  // scenario bank (only when fw_env_t.bank_enabled): int32 rows bank_row (scenario id of the next banked episode) and
+  // bank_row + 1 (scenario id of the running episode, -1: not from the bank); n_bank_rows = 0 or 2.  (These two fields
+  // took the place of padding: the struct keeps its size, so no kernel parameter after it moves.)
+  int32_t bank_row, n_bank_rows;
 };
 
 // metric accumulators, relative to FwLayout.m_drow (double) / m_irow (int32); k = target index
@@ -136,6 +139,7 @@ constexpr int fw_layout_build(const fw_env_t& E, int scale_actions, int64_t n, F
     L.m_irow = L.i_rows; L.i_rows += MI_GRING + 3 * L.goal_words;
   }
   if (turb_mixed) { L.tl_row = L.i_rows; L.n_tl_rows = 2; L.i_rows += 2; }
+  if (E.bank_enabled) { L.bank_row = L.i_rows; L.n_bank_rows = 2; L.i_rows += 2; }
   if (E.n_rand < 0 || E.n_rand > FW_MAX_RAND || E.n_par_rows < 0 || E.n_par_rows > FW_N_PAR) return 6;
   L.par_row = row;
   L.n_par_rows = E.n_par_rows;

@@ -103,41 +103,34 @@ def load_test_set(path):
 
 
 def evaluate_on_set(scenarios, config_path, controller="pid", config_kw=None, metrics=DEFAULT_METRICS,
-                    turbulence_intensity="none", device="cuda:0", seed=0, max_steps=None, env_offset=0):
+                    turbulence_intensity="none", device="cuda:0", seed=0, max_steps=None, env_offset=0, num_envs=None,
+                    keep_rewards=True):
     """Run every scenario once (in parallel) under `controller`: "pid", a dict of saved MlpPolicy arrays
     (MlpController), or a callable(vec) -> actions tensor.
     Returns (res, vec_env): res[metric][state] lists in scenario order, res["rewards"], res["lengths"].
     `turbulence_intensity`: one level ("none", "light", "moderate", "severe"), or a list of levels: then the S
     scenarios x L levels fly as ONE batch of L * S envs on a handle with per-env intensities (env j * S + i is scenario i
     at level j, pinned with set_turbulence_intensity) and the first element of the return value is {level: res}.
-    `env_offset`: global id of the first env (the Philox streams are keyed by it)."""
+    `env_offset`: global id of the first env (the Philox streams are keyed by it).
+    `num_envs` < scenarios x levels: fly them through a scenario bank on that many envs instead (the reference's pool
+    of workers that take scenario after scenario, evaluate_controller.py:80-169): every env starts its next scenario
+    when its episode ends, the controller is reset for it, and the results come back in scenario order in the same
+    layout.  Envs are reused, so the reference's carry-overs across episodes apply (the goal-achieved latch of the
+    success reward).  `keep_rewards=False` drops the per-step reward traces (S x steps_max doubles on the device)."""
     levels = None if isinstance(turbulence_intensity, str) else list(turbulence_intensity)
     n_scen = len(scenarios)
     n = n_scen if levels is None else n_scen * len(levels)
-    kw = dict(config_kw or {})
-    for k, v in EVAL_CONFIG_KW.items():
-        kw[k] = v
-    if controller == "pid":
-        kw["action"] = {"scale_space": False}          # evaluate_controller.py:78-79
-    if levels is None:
-        sim_kw = {"turbulence": turbulence_intensity != "none", "turbulence_intensity": turbulence_intensity}
-    else:
-        sim_kw = {"turbulence": True, "turbulence_intensity": {"values": levels}}
+    if num_envs is not None and int(num_envs) < n:
+        if max_steps is not None:
+            raise ValueError("max_steps cuts episodes short; a banked evaluation flies every episode to its end")
+        return _evaluate_banked(scenarios, config_path, controller, config_kw, metrics, levels, turbulence_intensity,
+                                device, seed, env_offset, int(num_envs), keep_rewards)
+    kw, sim_kw = _eval_kw(config_kw, controller, levels, turbulence_intensity)
     vec = FixedWingVecEnv(config_path, n, device=device, config_kw=kw, sim_config_kw=sim_kw, seed=seed, metrics=True,
                           auto_reset=True, env_offset=env_offset)
     if levels is not None:
         vec.set_turbulence_intensity([lv for lv in levels for _ in range(n_scen)])
-    reps = 1 if levels is None else len(levels)
-    skeys = sorted(scenarios[0]["state"].keys())
-    state = {}
-    for k in skeys:
-        v0 = scenarios[0]["state"][k]
-        if isinstance(v0, (list, tuple, np.ndarray)):     # "wind": [n, e, d]
-            state[k] = np.tile(np.array([s["state"][k] for s in scenarios], dtype=np.float64).T, (1, reps))
-        else:
-            state[k] = np.tile(np.array([s["state"][k] for s in scenarios], dtype=np.float64), reps)
-    target = {k: np.tile(np.array([s["target"][k] for s in scenarios], dtype=np.float64), reps)
-              for k in scenarios[0]["target"]}
+    state, target = _scenario_columns(scenarios, 1 if levels is None else len(levels))
     vec.enable_f64_outputs(True)
     vec.reset(state=state, target=target)
     pid = DevicePID(vec) if controller == "pid" else None
@@ -173,6 +166,85 @@ def evaluate_on_set(scenarios, config_path, controller="pid", config_kw=None, me
                          ln[j * n_scen:(j + 1) * n_scen]) for j, lv in enumerate(levels)}, vec
 
 
+def _eval_kw(config_kw, controller, levels, turbulence_intensity):
+    kw = dict(config_kw or {})
+    for k, v in EVAL_CONFIG_KW.items():
+        kw[k] = v
+    if controller == "pid":
+        kw["action"] = {"scale_space": False}          # evaluate_controller.py:78-79
+    if levels is None:
+        sim_kw = {"turbulence": turbulence_intensity != "none", "turbulence_intensity": turbulence_intensity}
+    else:
+        sim_kw = {"turbulence": True, "turbulence_intensity": {"values": levels}}
+    return kw, sim_kw
+
+
+def _scenario_columns(scenarios, reps):
+    """reset(state=, target=) columns of the scenarios, repeated `reps` times (one block per turbulence level)."""
+    state = {}
+    for k in sorted(scenarios[0]["state"].keys()):
+        v0 = scenarios[0]["state"][k]
+        if isinstance(v0, (list, tuple, np.ndarray)):     # "wind": [n, e, d]
+            state[k] = np.tile(np.array([s["state"][k] for s in scenarios], dtype=np.float64).T, (1, reps))
+        else:
+            state[k] = np.tile(np.array([s["state"][k] for s in scenarios], dtype=np.float64), reps)
+    target = {k: np.tile(np.array([s["target"][k] for s in scenarios], dtype=np.float64), reps)
+              for k in scenarios[0]["target"]}
+    return state, target
+
+
+def _evaluate_banked(scenarios, config_path, controller, config_kw, metrics, levels, turbulence_intensity, device, seed,
+                     env_offset, num_envs, keep_rewards):
+    """evaluate_on_set on `num_envs` envs: the S x L scenarios (scenario j * S + i = scenario i at level j) are a
+    scenario bank that the auto-resets consume."""
+    n_scen = len(scenarios)
+    reps = 1 if levels is None else len(levels)
+    total = n_scen * reps
+    kw, sim_kw = _eval_kw(config_kw, controller, levels, turbulence_intensity)
+    vec = FixedWingVecEnv(config_path, num_envs, device=device, config_kw=kw, sim_config_kw=sim_kw, seed=seed,
+                          metrics=True, auto_reset=True, env_offset=env_offset, scenario_bank=True)
+    state, target = _scenario_columns(scenarios, reps)
+    res = vec.set_scenario_bank(state=state, target=target,
+                                turbulence_intensity=None if levels is None else
+                                [lv for lv in levels for _ in range(n_scen)])
+    vec.enable_f64_outputs(True)
+    vec.reset()                                          # env e starts scenario e
+    pid = DevicePID(vec) if controller == "pid" else None
+    if isinstance(controller, dict):
+        controller = MlpController(vec, controller)
+    steps_cap = vec.cc.steps_max
+    d = vec.device
+    rew_trace = torch.full((steps_cap, total), float("nan"), dtype=torch.float64, device=d) if keep_rewards else None
+    ep_t = torch.zeros(num_envs, dtype=torch.long, device=d)      # step of each env's running episode
+    new = torch.ones(num_envs, dtype=torch.bool, device=d)        # the env starts a scenario at this step
+    # every env flies at most ceil(total / num_envs) scenarios of at most steps_max steps each
+    for _ in range(steps_cap * (-(-total // num_envs)) + 1):
+        ids = vec.scenario_ids().long()
+        if pid is not None:
+            actions = pid(new)
+        elif isinstance(controller, MlpController):
+            actions = controller(vec._obs64, new)
+        else:
+            actions = controller(vec)
+        _, _, done, _ = vec.step_tensors(actions)
+        if rew_trace is not None:
+            fly = ids >= 0
+            rew_trace[ep_t[fly], ids[fly]] = vec._rew64[fly]
+        new = done.bool()
+        ep_t = torch.where(new, torch.zeros_like(ep_t), ep_t + 1)
+        if bool((res["length"] >= 0).all()):
+            break
+    else:
+        raise RuntimeError("banked evaluation did not finish every scenario")
+    rows, ln = res["episode"].cpu().numpy(), res["length"].long().cpu().numpy()
+    tr = None if rew_trace is None else rew_trace.cpu().numpy()
+    if levels is None:
+        return _results(vec, metrics, rows, tr, ln), vec
+    return {lv: _results(vec, metrics, rows[j * n_scen:(j + 1) * n_scen],
+                         None if tr is None else tr[:, j * n_scen:(j + 1) * n_scen], ln[j * n_scen:(j + 1) * n_scen])
+            for j, lv in enumerate(levels)}, vec
+
+
 def _results(vec, metrics, rows, tr, ln):
     """res[metric][state] lists, rewards, lengths and episode rows of one block of envs (in env order)."""
     res = {m: {} for m in metrics}
@@ -183,7 +255,7 @@ def _results(vec, metrics, rows, tr, ln):
         for m in metrics:
             for st, val in info.get(m, {}).items():
                 res[m].setdefault(st, []).append(val)
-    res["rewards"] = [tr[:ln[i], i].copy() for i in range(len(ln))]
+    res["rewards"] = None if tr is None else [tr[:ln[i], i].copy() for i in range(len(ln))]
     res["lengths"] = ln
     res["episode_rows"], res["episode_columns"] = rows, vec.episode_columns()
     return res

@@ -12,7 +12,7 @@ import ctypes
 import numpy as np
 import torch
 
-from . import _capi
+from . import _capi, scenario_bank
 from .config import TURB_LEVELS, CompiledConfig
 
 TERM_NAMES = {0: None, 1: "steps", 2: "success", 3: "numeric"}
@@ -86,7 +86,8 @@ class VecInfos:
 class FixedWingVecEnv:
     def __init__(self, config_path=None, num_envs=1, device="cuda:0", sampler=None, sim_config_path=None,
                  sim_parameter_path=None, config_kw=None, sim_config_kw=None, seed=0, precision="fp64",
-                 env_offset=0, auto_reset=True, keep_terminal_obs=False, metrics=False, info_keywords=()):
+                 env_offset=0, auto_reset=True, keep_terminal_obs=False, metrics=False, info_keywords=(),
+                 scenario_bank=False):
         if sampler is not None:
             raise NotImplementedError("adaptive sampler hook is out of scope (SURVEY §2 #18)")
         self._lib = _capi.lib()   # raises if the CUDA extension is not built: no fallback
@@ -99,8 +100,9 @@ class FixedWingVecEnv:
         self.keep_terminal_obs = bool(keep_terminal_obs)
         self.metrics = bool(metrics)
         self.info_keywords = tuple(info_keywords)
+        self.scenario_bank = bool(scenario_bank)   # keep the scenario-bank rows: set_scenario_bank
         self.cc = CompiledConfig(config_path, sim_config_path, sim_parameter_path, config_kw, sim_config_kw, precision,
-                                 metrics=self.metrics)
+                                 metrics=self.metrics, scenario_bank=self.scenario_bank)
         self.cfg = self.cc.cfg
         self.target_names = list(self.cc._target_props_init["states"].keys())
         self.observation_space = Box(self.cc.observation_low, self.cc.observation_high)
@@ -121,6 +123,7 @@ class FixedWingVecEnv:
         self._actions = None
         self._ep_out = None
         self._turb_noise = None
+        self._bank = None
         if self.metrics:
             self.ep_dim = self._lib.fw_episode_dim(self._h)
             self._ep_out = torch.full((n, self.ep_dim), float("nan"), dtype=torch.float64, device=d)
@@ -439,6 +442,72 @@ class FixedWingVecEnv:
         sc = self.cc.sim_cfg
         lvl = TURB_LEVELS.index(sc.get("turbulence_intensity") or "light") if sc["turbulence"] else 0
         return torch.full((self.num_envs,), lvl, dtype=torch.int32, device=self.device)
+
+    # ------------------------------------------------------------------------------------------ scenario banks
+    def set_scenario_bank(self, state=None, target=None, turbulence_intensity=None, first=None, stride=None,
+                          cycle=False):
+        """Attach a bank of S scenarios that the resets of this env consume in order (include/fwgym.h fw_bank_t): every
+        auto-reset, and reset() without state= / target=, starts the env's next scenario - env e flies first + e, then
+        + stride per episode (modulo S with `cycle`) - until the env is past the bank, after which it samples as usual.
+        `state` / `target`: the names reset(state=, target=) takes, one value per scenario (NaN = sample it; a scalar
+        applies to all); `turbulence_intensity`: one level per scenario (mixed handles; -1 = the env's own rule).
+        `first` / `stride` default to 0 / num_envs; sharded ranks pass first = env_offset and stride = the total env
+        count.  Allocates the result rows scenario_results() returns (cycling banks: the counters only).  Takes effect
+        at the envs' next reset.  Attaching clears every env's running scenario id: an episode that is running now (from
+        an earlier bank) finishes, but reports no result anywhere."""
+        if not self.scenario_bank:
+            raise _capi.FwError("construct the env with scenario_bank=True")
+        S, st, tg, lv = scenario_bank.build_tables(state, target, turbulence_intensity, self.target_names,
+                                                   mixed=bool(self.cc.turbulence_mix))
+        first = 0 if first is None else int(first)
+        stride = self.num_envs if stride is None else int(stride)
+        scenario_bank.check_assignment(self.num_envs, S, first, stride)
+        d = self.device
+        keep = {"init_state": None if st is None else torch.as_tensor(st, device=d),
+                "init_target": None if tg is None else torch.as_tensor(tg, device=d),
+                "turb_level": None if lv is None else torch.as_tensor(lv, device=d)}
+        res = {"episodes": torch.zeros(S, dtype=torch.int32, device=d),
+               "successes": torch.zeros(S, dtype=torch.int32, device=d)}
+        if not cycle:
+            res["term"] = torch.full((S,), -1, dtype=torch.int32, device=d)
+            res["length"] = torch.full((S,), -1, dtype=torch.int32, device=d)
+            res["return"] = torch.full((S,), float("nan"), dtype=torch.float64, device=d)
+            if self.metrics:
+                res["episode"] = torch.full((S, self.ep_dim), float("nan"), dtype=torch.float64, device=d)
+        b = _capi.fw_bank_t()
+        b.init_state, b.init_target, b.turb_level = (t.data_ptr() if t is not None else None for t in keep.values())
+        b.n_scenarios, b.first, b.stride, b.cycle = S, first, stride, 1 if cycle else 0
+        for f, k in (("term", "term"), ("length", "length"), ("ret", "return"), ("episode", "episode"),
+                     ("episodes", "episodes"), ("successes", "successes")):
+            if k in res:
+                setattr(b, f, res[k].data_ptr())
+        _capi.check(self._lib.fw_set_bank(self._h, ctypes.byref(b), self._stream()))
+        self._bank = (keep, res)          # the device reads these while the bank is attached
+        self.n_scenarios = S
+        self.config_version += 1          # the bank is a kernel parameter: captured graphs hold the old one
+        return res
+
+    def detach_scenario_bank(self):
+        """Back to sampled resets (the cursors are cleared; running episodes no longer report results)."""
+        _capi.check(self._lib.fw_set_bank(self._h, None, self._stream()))
+        self.config_version += 1
+        self._bank_detached = self._bank   # kept alive until the stream is past the last kernel that read them
+        self._bank = None
+
+    def scenario_results(self):
+        """Device tensors of the attached bank, indexed by scenario id: "term" (FW_TERM_* code, -1 = not flown yet),
+        "length", "return", "episode" ([S, ep_dim] metric rows, metrics=True) and the int32 counters "episodes" /
+        "successes" (a cycling bank has the counters only)."""
+        if self._bank is None:
+            raise _capi.FwError("no scenario bank attached (set_scenario_bank)")
+        return self._bank[1]
+
+    def scenario_ids(self):
+        """Device int32 [N]: the scenario each env's running episode started from, -1 when it was not from the bank."""
+        rows = self.state_rows()
+        if "bank_scenario" not in rows:
+            raise _capi.FwError("construct the env with scenario_bank=True")
+        return self.get_rows(rows.index("bank_scenario"), 1)[0].to(torch.int32)
 
     def kernel_variant(self):
         """Which kernel instantiations the configuration selected, e.g. "dyn=shipped env=default_turb"."""

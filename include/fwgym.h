@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define FW_ABI_VERSION 11
+#define FW_ABI_VERSION 12
 
 /* ---------------------------------------------------------------------------------------------- limits */
 #define FW_MAX_OBS_VARS 32
@@ -220,7 +220,8 @@ typedef struct {
   /* simulator-parameter randomisation at every reset (SURVEY §8f row 4) */
   int32_t n_rand, n_par_rows;     /* draws per reset; per-env parameter rows (randomised + derived) */
   fw_rand_t rand[FW_MAX_RAND];
-  int32_t n_scale_rows, _pad5;    /* per-env reward-scaling rows (reward.randomize_scaling) */
+  int32_t n_scale_rows;           /* per-env reward-scaling rows (reward.randomize_scaling) */
+  int32_t bank_enabled;           /* the handle keeps the scenario-bank rows "bank_next" / "bank_scenario" (fw_set_bank) */
 } fw_env_t;
 
 typedef struct {
@@ -312,6 +313,40 @@ int fw_host_wait(fw_handle h, int slot, const float** obs, const float** rew, co
  * effect at each env's next reset (explicit or automatic).  FW_ERR_ARG on a handle that is not mixed.  The requested
  * and active levels are the state rows "turb_level_req" / "turb_level" (fw_get_state / fw_set_state). */
 int fw_set_turbulence_levels(fw_handle h, const int32_t* levels, void* stream);
+
+/* Scenario bank (handles created with fw_env_t.bank_enabled): a device table of S initial states / targets that resets
+ * consume in order, with one result row per scenario.  Every env keeps two int32 state rows: "bank_next" (scenario id of
+ * its next banked episode) and "bank_scenario" (scenario id of the running episode, -1 when it is not from the bank).
+ * fw_set_bank sets bank_next = first + e for local env e (mod S when `cycle`) and bank_scenario = -1; every reset that
+ * injects nothing (auto-resets, fw_reset with NULL init_state and init_target) while bank_next < S starts scenario
+ * bank_next, exactly as fw_reset would with the scenario's columns as init_state / init_target (NaN = sample it), and
+ * advances bank_next by `stride` (mod S when `cycle`, else saturating at S).  stride >= n_envs keeps any two envs off the
+ * same scenario; sharded ranks pass first = their env offset and stride = the total env count.  An env past the bank
+ * samples from the configured ranges; a reset with init_state or init_target leaves the cursor alone (bank_scenario = -1).
+ * When a banked episode ends (with or without auto_reset) the env kernel writes the optional result rows at index
+ * bank_scenario (only below S), counts it, and sets bank_scenario = -1.  The tables and result buffers must stay valid
+ * while the bank is attached.  The cursor rows are state (fw_get_state / fw_set_state); the pointers are not: to resume a
+ * checkpoint, attach the bank, then fw_set_state. */
+typedef struct {
+  const double* init_state;       /* optional device double [FW_N_SV + 3, S] (rows as fw_reset init_state) */
+  const double* init_target;      /* optional device double [FW_MAX_TARGETS, S] */
+  const int32_t* turb_level;      /* optional device int32 [S] (mixed handles only): >= 0 pins the episode's Dryden level
+                                   * like fw_set_turbulence_levels, -1 keeps the env's own rule */
+  int64_t n_scenarios;            /* S: 1 .. INT32_MAX */
+  int64_t first, stride;          /* assignment: env e flies first + e, then + stride per episode; stride >= n_envs */
+  int32_t cycle;                  /* != 0: the cursor wraps modulo S (no outcome rows allowed, several envs share ids) */
+  int32_t _pad;
+  int32_t* term;                  /* optional device int32 [S]: termination code (FW_TERM_*) */
+  int32_t* length;                /* optional device int32 [S]: episode length in env steps */
+  double* ret;                    /* optional device double [S]: episode return */
+  double* episode;                /* optional device double [S, fw_episode_dim] metric rows (metrics enabled only) */
+  int32_t* episodes;              /* optional device int32 [S]: banked episodes ended per scenario (atomic counts) */
+  int32_t* successes;             /* optional device int32 [S]: of those, episodes whose success streak was reached */
+} fw_bank_t;
+/* Attach (bank != NULL) or detach (NULL) a scenario bank.  FW_ERR_ARG: the handle was not created with bank_enabled,
+ * S <= 0 or S > INT32_MAX, first < 0, stride < n_envs, an episode buffer without metrics, outcome rows (term / length /
+ * ret / episode) together with cycle, or a level column on a handle that is not mixed. */
+int fw_set_bank(fw_handle h, const fw_bank_t* bank, void* stream);
 
 /* Rows [row0, row0 + nrows) of the state matrix below: device double [nrows, N] (e.g. the three target rows without
  * exporting the whole state). */
