@@ -174,7 +174,7 @@ class CompiledConfig:
     """Holds the (mutable) parsed JSON configs, mirrors FixedWingAircraft's derived attributes and produces the POD."""
 
     def __init__(self, config_path=None, sim_config_path=None, sim_parameter_path=None, config_kw=None,
-                 sim_config_kw=None, precision="fp64", metrics=False, scenario_bank=False):
+                 sim_config_kw=None, precision="fp64", metrics=False, scenario_bank=False, aircraft_parameters=()):
         config_path = config_path or DEFAULT_ENV_CONFIG
         with open(config_path) as f:
             self.cfg = json.load(f)
@@ -196,6 +196,7 @@ class CompiledConfig:
         self.precision = {"fp64": 0, "fp32": 1}[precision]
         self.metrics = bool(metrics)   # stream the get_metric quantities on the device (fixed_wing.py:1095-1162)
         self.scenario_bank = bool(scenario_bank)   # keep the scenario-bank rows (fw_set_bank)
+        self.aircraft_parameters = tuple(aircraft_parameters or ())   # per-env aircraft rows (fw_set_aircraft)
         self.state = {v["name"]: SimVariable(v) for v in self.sim_cfg["variables"]}
         self.dt = self.sim_cfg["dt"]
         self._check_supported()
@@ -227,6 +228,25 @@ class CompiledConfig:
         if self.sim_cfg["turbulence"] and not self.cfg["steps_max"] > 0:
             raise ConfigError("turbulence needs steps_max > 0 (turbulence_sim_length = steps_max, fixed_wing.py:40)")
         self.turbulence_mix = self._turbulence_mix()
+        self._check_aircraft()
+
+    def _check_aircraft(self):
+        names = self.aircraft_parameters
+        for n in names:
+            if n not in self.AIRCRAFT_PARAMS:
+                raise ConfigError("aircraft_parameters: %r cannot differ per env (allowed: %s; ar is always b^2 / S_wing)"
+                                  % (n, ", ".join(self.AIRCRAFT_PARAMS)))
+        if len(set(names)) != len(names):
+            raise ConfigError("aircraft_parameters: a name is listed twice in %r" % (names,))
+        if not names:
+            return
+        if any(k != "states" for k in self.cfg["simulator"]):
+            raise ConfigError("aircraft_parameters cannot be combined with simulator-parameter randomisation "
+                              "(simulator.%s): the reference centres those draws on each aircraft's own values"
+                              % next(k for k in self.cfg["simulator"] if k != "states"))
+        if "b" in names and self.sim_cfg["turbulence"]:
+            raise ConfigError("aircraft_parameters: a per-env wingspan b needs turbulence off (the Dryden filters are "
+                              "built from b)")
 
     def _turbulence_mix(self):
         """sim_config_kw turbulence_intensity = {"values": [level names], "probabilities": [...]} (the reference's
@@ -272,6 +292,19 @@ class CompiledConfig:
                    "C_l_p", "C_l_r", "C_l_delta_a", "C_l_delta_r", "C_n_0", "C_n_beta", "C_n_p", "C_n_r",
                    "C_n_delta_a", "C_n_delta_r")
     SIM_ATTRS = ("rho", "g")     # PyFly attributes the right-hand side reads at every evaluation
+    INERTIA = ("Jx", "Jy", "Jz", "Jxz")
+    # what FixedWingVecEnv(aircraft_parameters=) may set per env (include/fwgym.h fw_air)
+    AIRCRAFT_PARAMS = tuple(n for n in LIVE_PARAMS if n != "ar") + SIM_ATTRS + INERTIA
+
+    def air_id(self, name):
+        """aircraft parameter name -> its id (fw_air: a fw_par id, or FW_AIR_JX.. for the inertia)"""
+        if name in self.INERTIA:
+            return _capi.ENUMS["FW_AIR_JX"] + self.INERTIA.index(name)
+        return self.par_id(name)
+
+    def aircraft_nominal(self):
+        """name -> the handle's value of every listed aircraft parameter (what a NaN request flies)"""
+        return {n: float(self.sim_cfg[n] if n in self.SIM_ATTRS else self.params[n]) for n in self.aircraft_parameters}
 
     @staticmethod
     def par_id(name):
@@ -326,7 +359,9 @@ class CompiledConfig:
 
     def _rand_slots(self):
         """-> (plan, slot1 of every fw_par id, number of per-env parameter rows).  A parameter drawn twice keeps one
-        row (the last draw wins, as the reference's dict assignment); derived rows follow the drawn ones."""
+        row (the last draw wins, as the reference's dict assignment); derived rows follow the drawn ones.  Aircraft
+        parameters (never together with a draw) take rows in their listed order, then ar when b or S_wing is listed,
+        then the derived rows, and the FW_N_INERTIA inertia rows last (inertia_slots)."""
         plan = self._rand_plan()
         slot1 = [0] * _capi.ENUMS["FW_PAR_N"]
         n = 0
@@ -335,12 +370,30 @@ class CompiledConfig:
                 n += 1
                 slot1[ent["par"]] = n
         E = _capi.ENUMS
+        for name in self.aircraft_parameters:
+            if name not in self.INERTIA:
+                n += 1
+                slot1[self.par_id(name)] = n
+        if self.aircraft_parameters and (slot1[E["FW_PAR_B"]] or slot1[E["FW_PAR_S_WING"]]):
+            n += 1
+            slot1[E["FW_PAR_AR"]] = n
         for derived, sources in ((E["FW_PAR_INV_MASS"], ("MASS",)), (E["FW_PAR_INV_PI_E_AR"], ("E", "AR")),
                                  (E["FW_PAR_EXP_2MA0"], ("M", "A_0"))):
             if any(slot1[E["FW_PAR_" + s_]] for s_ in sources):
                 n += 1
                 slot1[derived] = n
+        if any(name in self.INERTIA for name in self.aircraft_parameters):
+            n += _capi.DEFINES["FW_N_INERTIA"]
         return plan, slot1, n
+
+    def inertia_slots(self):
+        """slot1 of gammas[1..8], inv_Jy (fw_sim_t.inertia_slot1): the last FW_N_INERTIA parameter rows when an inertia
+        entry is an aircraft parameter, else all 0."""
+        k = _capi.DEFINES["FW_N_INERTIA"]
+        if not any(name in self.INERTIA for name in self.aircraft_parameters):
+            return [0] * k
+        n = self._rand_slots()[2]
+        return list(range(n - k + 1, n + 1))
 
     # ------------------------------------------------------------------------- fixed_wing.py:57-191 (spaces etc.)
     def _limit(self, state_name, side):
@@ -573,6 +626,12 @@ class CompiledConfig:
         _, slot1, _ = self._rand_slots()
         for i, v in enumerate(slot1):
             s.par_slot1[i] = v
+        if self.aircraft_parameters:
+            s.Jx, s.Jz, s.Jxz = float(P["Jx"]), float(P["Jz"]), float(P["Jxz"])
+            for j, name in enumerate(self.aircraft_parameters):
+                s.air_id[j] = self.air_id(name)
+            for k, v in enumerate(self.inertia_slots()):
+                s.inertia_slot1[k] = v
 
     @staticmethod
     def turbulence_dt(sc):
@@ -758,3 +817,4 @@ class CompiledConfig:
             F.sign = float(np.sign(comp.get("sign", -1)))
         e.n_scale_rows = n_scale
         e.bank_enabled = 1 if self.scenario_bank else 0
+        e.n_aircraft = len(self.aircraft_parameters)

@@ -186,26 +186,37 @@ static_assert(FW_PAR_N == FW_N_PAR, "FW_N_PAR in fwgym.h must equal the number o
 //                 them branch-free: 50 warp-uniform branches per RHS would cut it into basic blocks that cannot
 //                 overlap; an unconditional shared-memory read + select keeps it one block.
 enum { FW_PAR_CONST = 0, FW_PAR_GLOBAL = 1, FW_PAR_SMEM = 2 };
+// The inertia terms (FW_N_INERTIA: gammas[1..8], inv_Jy) follow the same rule with P.inertia_slot1[k]: per-env rows only
+// on a handle whose aircraft parameters include the inertia (fw_set_aircraft).
+#define FW_INERTIA(X)                                                                                                 \
+  X(0, gamma1, gammas[1]) X(1, gamma2, gammas[2]) X(2, gamma3, gammas[3]) X(3, gamma4, gammas[4])                    \
+  X(4, gamma5, gammas[5]) X(5, gamma6, gammas[6]) X(6, gamma7, gammas[7]) X(7, gamma8, gammas[8]) X(8, inv_Jy, inv_Jy)
+static_assert(FW_AIR_JX == FW_PAR_N, "fw_air ids follow the fw_par ids");
 template <typename T, int MODE> struct FwPar {
   const fw_sim_t& P;
   const double* base;   // GLOBAL: this aircraft's element of parameter row 0
   int64_t stride;
   const T* cache;       // SMEM: this lane's element of cached row 0 (32 lanes per row)
-#define FW_PAR_GETTER(ID, F)                                                      \
-  __device__ __forceinline__ T F() const {                                        \
+#define FW_PAR_READ(NAME, SLOT1, FIELD)                                           \
+  __device__ __forceinline__ T NAME() const {                                     \
     if constexpr (MODE == FW_PAR_GLOBAL) {                                        \
-      const int s1 = P.par_slot1[FW_PAR_##ID];                                    \
+      const int s1 = SLOT1;                                                       \
       if (s1) return (T)base[(int64_t)(s1 - 1) * stride];                         \
     }                                                                             \
     if constexpr (MODE == FW_PAR_SMEM) {                                          \
-      const int s1 = P.par_slot1[FW_PAR_##ID];                                    \
+      const int s1 = SLOT1;                                                       \
       const T v = cache[(s1 > 0 ? s1 - 1 : 0) * 32];                              \
-      return s1 > 0 ? v : fw_rd<T>(P, P.F);                                       \
+      return s1 > 0 ? v : fw_rd<T>(P, FIELD);                                     \
     }                                                                             \
-    return fw_rd<T>(P, P.F);                                                      \
+    return fw_rd<T>(P, FIELD);                                                    \
   }
+#define FW_PAR_GETTER(ID, F) FW_PAR_READ(F, P.par_slot1[FW_PAR_##ID], P.F)
   FW_LIVE_PARAMS(FW_PAR_GETTER)
 #undef FW_PAR_GETTER
+#define FW_INERTIA_GETTER(K, NAME, F) FW_PAR_READ(NAME, P.inertia_slot1[K], P.F)
+  FW_INERTIA(FW_INERTIA_GETTER)
+#undef FW_INERTIA_GETTER
+#undef FW_PAR_READ
 };
 
 // branch-free condition of the variable of rank R: violated constraints set bit R of failmask.  RAW: no condition
@@ -362,11 +373,9 @@ __device__ __forceinline__ void fw_rhs(const fw_sim_t& P, const PAR& PP, const F
   dy[1] = (T)0.5 * (p * e0 + r * e2 - q * e3);
   dy[2] = (T)0.5 * (q * e0 - r * e1 + p * e3);
   dy[3] = (T)0.5 * (r * e0 + q * e1 - p * e2);
-#define FW_G(k) fw_rd<T>(P, P.gammas[k])
-  dy[4] = FW_G(1) * p * q - FW_G(2) * q * r + FW_G(3) * tl + FW_G(4) * tn;
-  dy[5] = FW_G(5) * p * r - FW_G(6) * (p * p - r * r) + tm * fw_rd<T>(P, P.inv_Jy);
-  dy[6] = FW_G(7) * p * q - FW_G(1) * q * r + FW_G(4) * tl + FW_G(8) * tn;
-#undef FW_G
+  dy[4] = PP.gamma1() * p * q - PP.gamma2() * q * r + PP.gamma3() * tl + PP.gamma4() * tn;
+  dy[5] = PP.gamma5() * p * r - PP.gamma6() * (p * p - r * r) + tm * PP.inv_Jy();
+  dy[6] = PP.gamma7() * p * q - PP.gamma1() * q * r + PP.gamma4() * tl + PP.gamma8() * tn;
   dy[7] = (e1 * e1 + e0 * e0 - e2 * e2 - e3 * e3) * u + 2 * (e1 * e2 - e3 * e0) * v + 2 * (e1 * e3 + e2 * e0) * w;
   dy[8] = 2 * (e1 * e2 + e3 * e0) * u + (e2 * e2 + e0 * e0 - e1 * e1 - e3 * e3) * v + 2 * (e2 * e3 - e1 * e0) * w;
   dy[9] = 2 * (e1 * e3 - e2 * e0) * u + 2 * (e2 * e3 + e1 * e0) * v + (e3 * e3 + e0 * e0 - e1 * e1 - e2 * e2) * w;

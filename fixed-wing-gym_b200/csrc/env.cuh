@@ -512,6 +512,7 @@ struct FwBank {
   double* episode;            // [n, ep_dim]
   int32_t* episodes;
   int32_t* successes;
+  const double* aircraft;     // [n_aircraft, n] (appended: no earlier member moves)
 };
 // the scenario after `cur` for the same env: + stride, modulo n when cycling, else saturating at n (past the bank)
 __device__ __forceinline__ int32_t fw_bank_advance(const FwBank& b, int32_t cur) {
@@ -839,6 +840,10 @@ __device__ __forceinline__ void fw_reset_env_body(const fw_env_t& E, const fw_si
   FwEnvRngT<SH::fixed> rng{g, 0u, 0u, 0.0};
   // sample_simulator_parameters (fixed_wing.py:523-570) runs between simulator.reset and sample_target (:308-310) and
   // draws from the env's generator in table order.  Fixed shapes have no table (n_rand == 0).
+  auto par = [&](int id, double shared) -> double {   // the episode's value of a live parameter
+    const int s1 = P.par_slot1[id];
+    return s1 ? c.D(Ls.par_row + s1 - 1) : shared;
+  };
   if (Es.n_rand > 0) {
     for (int j = 0; j < E.n_rand; ++j) {
       const fw_rand_t& r = E.rand[j];
@@ -853,11 +858,56 @@ __device__ __forceinline__ void fw_reset_env_body(const fw_env_t& E, const fw_si
       }
       if (r.slot1) c.D(Ls.par_row + r.slot1 - 1) = v;
     }
+  }
+  // per-env aircraft (fw_set_aircraft): the episode flies its requests (a banked scenario's finite column entries win),
+  // NaN = nominal.  No draw.  The host refuses aircraft parameters together with randomisation, so each row has one writer.
+  if (Es.n_aircraft > 0) {
+    double jx = P.Jx, jy = P.Jy, jz = P.Jz, jxz = P.Jxz;
+    for (int j = 0; j < E.n_aircraft; ++j) {
+      double v = c.D(Ls.air_row + j);
+      if constexpr (SH::bank) {
+        if (scen >= 0 && bank.aircraft) {
+          const double bv = bank.aircraft[(int64_t)j * bank.n + scen];
+          if (!isnan(bv)) v = bv;
+        }
+      }
+      const int id = P.air_id[j];
+      if (id < FW_PAR_N) {
+        // fw_par ids MASS .. C_N_DELTA_R index the fw_sim_t fields mass .. C_n_delta_r
+        if (isnan(v)) v = id == FW_PAR_RHO ? P.rho : (id == FW_PAR_G ? P.g : (&P.mass)[id]);
+        c.D(Ls.par_row + P.par_slot1[id] - 1) = v;
+      } else if (!isnan(v)) {
+        if (id == FW_AIR_JX) jx = v;
+        if (id == FW_AIR_JY) jy = v;
+        if (id == FW_AIR_JZ) jz = v;
+        if (id == FW_AIR_JXZ) jxz = v;
+      }
+    }
+    // what PyFly derives at construction, in config.py's operation order, correctly rounded and never contracted
+    if (P.par_slot1[FW_PAR_AR]) {   // b or S_wing is listed: ar = b^2 / S_wing (pyfly_restated.py:507)
+      const double b = par(FW_PAR_B, P.b);
+      c.D(Ls.par_row + P.par_slot1[FW_PAR_AR] - 1) = __ddiv_rn(__dmul_rn(b, b), par(FW_PAR_S_WING, P.S_wing));
+    }
+    if (P.inertia_slot1[0]) {
+      // I = [[Jx, 0, -Jxz], [0, Jy, 0], [-Jxz, 0, Jz]]; I02^2 = Jxz^2, |I02| = |Jxz|
+      const double axz = fabs(jxz), xz2 = __dmul_rn(jxz, jxz);
+      const double g0 = __dsub_rn(__dmul_rn(jx, jz), xz2);
+      double gam[FW_N_INERTIA];
+      gam[0] = __ddiv_rn(__dmul_rn(axz, __dadd_rn(__dsub_rn(jx, jy), jz)), g0);
+      gam[1] = __ddiv_rn(__dadd_rn(__dmul_rn(jz, __dsub_rn(jz, jy)), xz2), g0);
+      gam[2] = __ddiv_rn(jz, g0);
+      gam[3] = __ddiv_rn(axz, g0);
+      gam[4] = __ddiv_rn(__dsub_rn(jz, jx), jy);
+      gam[5] = __ddiv_rn(-jxz, jy);
+      gam[6] = __ddiv_rn(__dadd_rn(__dmul_rn(__dsub_rn(jx, jy), jx), xz2), g0);
+      gam[7] = __ddiv_rn(jx, g0);
+      gam[8] = __ddiv_rn(1.0, jy);
+#pragma unroll
+      for (int k = 0; k < FW_N_INERTIA; ++k) c.D(Ls.par_row + P.inertia_slot1[k] - 1) = gam[k];
+    }
+  }
+  if (Es.n_rand > 0 || Es.n_aircraft > 0) {
     // derived rows: what the right-hand side multiplies by instead of dividing / exponentiating at every evaluation
-    auto par = [&](int id, double shared) -> double {
-      const int s1 = P.par_slot1[id];
-      return s1 ? c.D(Ls.par_row + s1 - 1) : shared;
-    };
     if (P.par_slot1[FW_PAR_INV_MASS]) c.D(Ls.par_row + P.par_slot1[FW_PAR_INV_MASS] - 1) = 1.0 / par(FW_PAR_MASS, P.mass);
     if (P.par_slot1[FW_PAR_INV_PI_E_AR])
       c.D(Ls.par_row + P.par_slot1[FW_PAR_INV_PI_E_AR] - 1) = 1.0 / (CUDART_PI * par(FW_PAR_E, P.e) * par(FW_PAR_AR, P.ar));

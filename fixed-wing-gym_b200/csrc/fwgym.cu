@@ -922,7 +922,7 @@ static_assert(sizeof(fw_env_t) + sizeof(fw_sim_t) + sizeof(FwLayout) + sizeof(Fw
 static_assert(sizeof(FwSimX) + sizeof(FwDynArgs) + 64 <= 32764, "fp32 dynamics kernel parameters exceed the 32 764-byte limit");
 static_assert(sizeof(fw_sim_t) + sizeof(FwDynArgs) + 64 <= 32764, "fp64 dynamics kernel parameters exceed the 32 764-byte limit");
 // the per-level Dryden tables were appended without moving any later kernel parameter off its 16-byte alignment
-static_assert(sizeof(fw_sim_t) % 32 == 24 && sizeof(FwLayout) % 16 == 8, "see fw_sim_t._pad_turb / FwLayout.bank_row");
+static_assert(sizeof(fw_sim_t) % 32 == 24 && sizeof(FwLayout) % 16 == 8, "see fw_sim_t._pad_air / FwLayout._pad_air");
 
 // ---- PID baseline controller (pyfly/pid_controller.py; evaluate_controller.py:141-151) ---------------------------
 __global__ void fw_pid_kernel(const double* __restrict__ d, int64_t stride, int64_t n, const fw_pid_gains_t g, double dt,
@@ -1020,6 +1020,24 @@ static int make_layout(const fw_config_t& cfg, int64_t n, FwLayout& L) {
     return fail(FW_ERR_CONFIG, "per-env turbulence levels (turb_mixed) need turbulence on");
   const int rc = fw_layout_build(cfg.env, cfg.sim.scale_actions, n, L, cfg.sim.turb_mixed);
   if (rc) return fail(FW_ERR_CONFIG, "%s", fw_layout_error(rc));
+  // the reset writes aircraft parameters through these tables without checks of its own
+  const fw_sim_t& S = cfg.sim;
+  const int np = cfg.env.n_par_rows;
+  auto row_ok = [&](int s1) { return s1 >= 1 && s1 <= np; };
+  bool inertia = false;
+  for (int j = 0; j < cfg.env.n_aircraft; ++j) {
+    const int id = S.air_id[j];
+    const bool live = id >= 0 && id < FW_PAR_N && id != FW_PAR_AR && id < FW_PAR_INV_MASS;
+    if (!live && !(id >= FW_AIR_JX && id <= FW_AIR_JXZ))
+      return fail(FW_ERR_CONFIG, "aircraft parameters: bad air_id%s", "");
+    if (live && !row_ok(S.par_slot1[id])) return fail(FW_ERR_CONFIG, "aircraft parameters: a live entry has no parameter row%s", "");
+    inertia |= !live;
+  }
+  for (int k = 0; k < FW_N_INERTIA; ++k)
+    if (S.inertia_slot1[k] ? !(inertia && row_ok(S.inertia_slot1[k])) : inertia)
+      return fail(FW_ERR_CONFIG, "aircraft parameters: per-env inertia needs a parameter row for every inertia term%s", "");
+  if (cfg.env.n_aircraft && cfg.env.n_rand)
+    return fail(FW_ERR_CONFIG, "aircraft parameters together with simulator-parameter randomisation%s", "");
   return FW_OK;
 }
 
@@ -1115,6 +1133,8 @@ static FwKernels select_kernels(const fw_config_t& cfg) {
   bool rand = false;   // per-env model parameters
   for (int i = 0; i < FW_PAR_N; ++i)
     if (S.par_slot1[i]) rand = true;
+  for (int k = 0; k < FW_N_INERTIA; ++k)
+    if (S.inertia_slot1[k]) rand = true;
   uint32_t clip = 0, cons = 0;
   for (int r = 0; r <= FW_R_BETA; ++r) {
     const uint32_t f = S.var[rank_sv[r]].flags;
@@ -1176,6 +1196,8 @@ static int init_handle(fw_handle h) {
   *h->err_flag_host = 0;
   if (h->L.n_tl_rows)   // requested levels start at -1: every env draws its level at each reset
     CK(cudaMemset(h->i + (size_t)h->L.tl_row * st, 0xff, st * sizeof(int32_t)));
+  if (h->L.n_air_rows)  // aircraft requests start as NaN (all bits set): the nominal aircraft
+    CK(cudaMemset(h->d + (size_t)h->L.air_row * st, 0xff, h->L.n_air_rows * st * sizeof(double)));
   // aircraft whose first dopri5 step is below dt / FWGYM_LONG_DIV need the most attempts (e.g. the 1e-6 start after a
   // reset): they are started first so that they do not become the tail of the attempt kernel
   const char* e = getenv("FWGYM_LONG_DIV");
@@ -1301,6 +1323,7 @@ const char* fw_state_row_name(fw_handle h, int64_t r) {
   if (r < D_FIXED) return dn[r];
   if (h->L.n_par_rows > 0 && r >= h->L.par_row && r < h->L.par_row + h->L.n_par_rows) return "param";
   if (h->L.n_rs_rows > 0 && r >= h->L.rs_row && r < h->L.rs_row + h->L.n_rs_rows) return "reward_scaling";
+  if (h->L.n_air_rows > 0 && r >= h->L.air_row && r < h->L.air_row + h->L.n_air_rows) return "aircraft_req";
   if (r < h->L.d_rows) return "ring";
   r -= h->L.d_rows;
   if (r < I_GOALRING) return in[r];
@@ -1598,6 +1621,23 @@ int fw_set_turbulence_levels(fw_handle h, const int32_t* levels, void* stream) {
   return FW_OK;
 }
 
+int fw_set_aircraft(fw_handle h, const double* values, void* stream) {
+  if (!h) return fail(FW_ERR_ARG, "null handle");
+  if (!h->L.n_air_rows)
+    return fail(FW_ERR_ARG, "fw_set_aircraft: the handle has no aircraft parameters (fw_env_t.n_aircraft)%s", "");
+  CK(cudaSetDevice(h->device));
+  const size_t st = (size_t)h->L.stride;
+  double* rows = h->d + (size_t)h->L.air_row * st;
+  if (values)
+    CK(cudaMemcpy2DAsync(rows, st * sizeof(double), values, (size_t)h->n * sizeof(double), (size_t)h->n * sizeof(double),
+                         (size_t)h->L.n_air_rows, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  else
+    CK(cudaMemsetAsync(rows, 0xff, (size_t)h->L.n_air_rows * st * sizeof(double), (cudaStream_t)stream));
+  return FW_OK;
+}
+
+int64_t fw_aircraft_dim(fw_handle h) { return h ? h->L.n_air_rows : 0; }
+
 int fw_set_bank(fw_handle h, const fw_bank_t* b, void* stream) {
   if (!h) return fail(FW_ERR_ARG, "null handle");
   if (!h->L.n_bank_rows)
@@ -1614,7 +1654,7 @@ int fw_set_bank(fw_handle h, const fw_bank_t* b, void* stream) {
     if (b->turb_level && !h->L.n_tl_rows)
       return fail(FW_ERR_ARG, "fw_set_bank: a level column needs a handle with per-env turbulence levels%s", "");
     k = FwBank{b->init_state, b->init_target, b->turb_level, b->n_scenarios, b->stride, b->cycle ? 1 : 0, 0,
-               b->term, b->length, b->ret, b->episode, b->episodes, b->successes};
+               b->term, b->length, b->ret, b->episode, b->episodes, b->successes, nullptr};
   }
   CK(cudaSetDevice(h->device));
   const size_t st = (size_t)h->L.stride;
@@ -1622,6 +1662,15 @@ int fw_set_bank(fw_handle h, const fw_bank_t* b, void* stream) {
       h->i + (size_t)h->L.bank_row * st, h->i + (size_t)(h->L.bank_row + 1) * st, h->n, b ? b->first : 0, k.n, k.cycle);
   CK(cudaGetLastError());
   h->bank = k;
+  return FW_OK;
+}
+
+int fw_set_bank_aircraft(fw_handle h, const double* aircraft) {
+  if (!h) return fail(FW_ERR_ARG, "null handle");
+  if (aircraft && !h->L.n_air_rows)
+    return fail(FW_ERR_ARG, "fw_set_bank_aircraft: an aircraft column needs a handle with aircraft parameters%s", "");
+  if (aircraft && h->bank.n == 0) return fail(FW_ERR_ARG, "fw_set_bank_aircraft: no scenario bank is attached%s", "");
+  h->bank.aircraft = aircraft;
   return FW_OK;
 }
 

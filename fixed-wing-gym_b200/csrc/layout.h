@@ -74,6 +74,10 @@ struct FwLayout {
   // bank_row + 1 (scenario id of the running episode, -1: not from the bank); n_bank_rows = 0 or 2.  (These two fields
   // took the place of padding: the struct keeps its size, so no kernel parameter after it moves.)
   int32_t bank_row, n_bank_rows;
+  // per-env aircraft (only when fw_env_t.n_aircraft > 0): double rows air_row .. air_row + n_air_rows - 1, the requested
+  // value of each listed parameter (NaN = nominal).  16 bytes, so that every kernel parameter after it keeps its alignment.
+  int32_t air_row, n_air_rows;
+  int32_t _pad_air[2];
 };
 
 // metric accumulators, relative to FwLayout.m_drow (double) / m_irow (int32); k = target index
@@ -140,7 +144,7 @@ constexpr int fw_layout_build(const fw_env_t& E, int scale_actions, int64_t n, F
   }
   if (turb_mixed) { L.tl_row = L.i_rows; L.n_tl_rows = 2; L.i_rows += 2; }
   if (E.bank_enabled) { L.bank_row = L.i_rows; L.n_bank_rows = 2; L.i_rows += 2; }
-  if (E.n_rand < 0 || E.n_rand > FW_MAX_RAND || E.n_par_rows < 0 || E.n_par_rows > FW_N_PAR) return 6;
+  if (E.n_rand < 0 || E.n_rand > FW_MAX_RAND || E.n_par_rows < 0 || E.n_par_rows > FW_N_PAR + FW_N_INERTIA) return 6;
   L.par_row = row;
   L.n_par_rows = E.n_par_rows;
   row += E.n_par_rows;
@@ -148,6 +152,8 @@ constexpr int fw_layout_build(const fw_env_t& E, int scale_actions, int64_t n, F
   L.rs_row = row;
   L.n_rs_rows = E.n_scale_rows;
   row += E.n_scale_rows;
+  if (E.n_aircraft < 0 || E.n_aircraft > FW_MAX_AIRCRAFT) return 8;
+  if (E.n_aircraft) { L.air_row = row; L.n_air_rows = E.n_aircraft; row += E.n_aircraft; }
   L.d_rows = row;
   return 0;
 }
@@ -160,6 +166,7 @@ inline const char* fw_layout_error(int code) {
     case 5: return "integrator observation / int_error reward need integration_window > 0";
     case 6: return "bad simulator-parameter randomisation table";
     case 7: return "bad reward-scaling randomisation table";
+    case 8: return "bad number of aircraft parameters";
   }
   return "";
 }

@@ -104,7 +104,7 @@ def load_test_set(path):
 
 def evaluate_on_set(scenarios, config_path, controller="pid", config_kw=None, metrics=DEFAULT_METRICS,
                     turbulence_intensity="none", device="cuda:0", seed=0, max_steps=None, env_offset=0, num_envs=None,
-                    keep_rewards=True):
+                    keep_rewards=True, aircraft=None):
     """Run every scenario once (in parallel) under `controller`: "pid", a dict of saved MlpPolicy arrays
     (MlpController), or a callable(vec) -> actions tensor.
     Returns (res, vec_env): res[metric][state] lists in scenario order, res["rewards"], res["lengths"].
@@ -116,21 +116,34 @@ def evaluate_on_set(scenarios, config_path, controller="pid", config_kw=None, me
     of workers that take scenario after scenario, evaluate_controller.py:80-169): every env starts its next scenario
     when its episode ends, the controller is reset for it, and the results come back in scenario order in the same
     layout.  Envs are reused, so the reference's carry-overs across episodes apply (the goal-achieved latch of the
-    success reward).  `keep_rewards=False` drops the per-step reward traces (S x steps_max doubles on the device)."""
+    success reward).  `keep_rewards=False` drops the per-step reward traces (S x steps_max doubles on the device).
+    `aircraft`: a list of V variants, each a dict of model parameters (the names FixedWingVecEnv(aircraft_parameters=)
+    takes; parameters a variant leaves out keep their nominal values): the S scenarios x V variants fly as ONE batch (env
+    j * S + i is scenario i on variant j) and the first element of the return value is {j: res}.  Not together with a
+    list of turbulence levels."""
     levels = None if isinstance(turbulence_intensity, str) else list(turbulence_intensity)
+    variants = None if aircraft is None else [dict(v) for v in aircraft]
+    if variants is not None and levels is not None:
+        raise ValueError("evaluate_on_set flies either several turbulence levels or several aircraft, not both")
+    if variants is not None and not variants:
+        raise ValueError("aircraft: at least one variant")
     n_scen = len(scenarios)
-    n = n_scen if levels is None else n_scen * len(levels)
+    reps = len(levels) if levels is not None else (len(variants) if variants is not None else 1)
+    n = n_scen * reps
+    air_names, air = _aircraft_columns(variants, n_scen)
     if num_envs is not None and int(num_envs) < n:
         if max_steps is not None:
             raise ValueError("max_steps cuts episodes short; a banked evaluation flies every episode to its end")
         return _evaluate_banked(scenarios, config_path, controller, config_kw, metrics, levels, turbulence_intensity,
-                                device, seed, env_offset, int(num_envs), keep_rewards)
+                                device, seed, env_offset, int(num_envs), keep_rewards, air_names, air)
     kw, sim_kw = _eval_kw(config_kw, controller, levels, turbulence_intensity)
     vec = FixedWingVecEnv(config_path, n, device=device, config_kw=kw, sim_config_kw=sim_kw, seed=seed, metrics=True,
-                          auto_reset=True, env_offset=env_offset)
+                          auto_reset=True, env_offset=env_offset, aircraft_parameters=air_names)
     if levels is not None:
         vec.set_turbulence_intensity([lv for lv in levels for _ in range(n_scen)])
-    state, target = _scenario_columns(scenarios, 1 if levels is None else len(levels))
+    if air is not None:
+        vec.set_aircraft(air)
+    state, target = _scenario_columns(scenarios, reps)
     vec.enable_f64_outputs(True)
     vec.reset(state=state, target=target)
     pid = DevicePID(vec) if controller == "pid" else None
@@ -160,10 +173,29 @@ def evaluate_on_set(scenarios, config_path, controller="pid", config_kw=None, me
                 break
     lengths[alive] = min(t + 1, steps_cap)
     rows, tr, ln = ep_rows.cpu().numpy(), rew_trace.cpu().numpy(), lengths.cpu().numpy()
-    if levels is None:
-        return _results(vec, metrics, rows, tr, ln), vec
-    return {lv: _results(vec, metrics, rows[j * n_scen:(j + 1) * n_scen], tr[:, j * n_scen:(j + 1) * n_scen],
-                         ln[j * n_scen:(j + 1) * n_scen]) for j, lv in enumerate(levels)}, vec
+    return _split(vec, metrics, rows, tr, ln, n_scen, levels, variants), vec
+
+
+def _split(vec, metrics, rows, tr, ln, n_scen, levels, variants):
+    """res of one block of S envs, or {level: res} / {variant index: res} of consecutive blocks"""
+    keys = levels if levels is not None else (range(len(variants)) if variants is not None else None)
+    if keys is None:
+        return _results(vec, metrics, rows, tr, ln)
+    return {k: _results(vec, metrics, rows[j * n_scen:(j + 1) * n_scen],
+                        None if tr is None else tr[:, j * n_scen:(j + 1) * n_scen], ln[j * n_scen:(j + 1) * n_scen])
+            for j, k in enumerate(keys)}
+
+
+def _aircraft_columns(variants, n_scen):
+    """-> (aircraft_parameters, {name: value per env}) for V variants x S scenarios (env j * S + i flies variant j; a
+    parameter a variant leaves out is NaN = nominal), or ((), None) without variants."""
+    if variants is None:
+        return (), None
+    names = tuple(sorted({k for v in variants for k in v}))
+    if not names:
+        raise ValueError("aircraft: the variants set no parameter")
+    cols = {k: np.repeat(np.array([float(v.get(k, np.nan)) for v in variants]), n_scen) for k in names}
+    return names, cols
 
 
 def _eval_kw(config_kw, controller, levels, turbulence_intensity):
@@ -194,19 +226,20 @@ def _scenario_columns(scenarios, reps):
 
 
 def _evaluate_banked(scenarios, config_path, controller, config_kw, metrics, levels, turbulence_intensity, device, seed,
-                     env_offset, num_envs, keep_rewards):
-    """evaluate_on_set on `num_envs` envs: the S x L scenarios (scenario j * S + i = scenario i at level j) are a
-    scenario bank that the auto-resets consume."""
+                     env_offset, num_envs, keep_rewards, air_names=(), air=None):
+    """evaluate_on_set on `num_envs` envs: the S x L scenarios (scenario j * S + i = scenario i at level j, or on
+    aircraft variant j) are a scenario bank that the auto-resets consume."""
     n_scen = len(scenarios)
-    reps = 1 if levels is None else len(levels)
+    reps = len(levels) if levels is not None else (len(next(iter(air.values()))) // n_scen if air is not None else 1)
     total = n_scen * reps
     kw, sim_kw = _eval_kw(config_kw, controller, levels, turbulence_intensity)
     vec = FixedWingVecEnv(config_path, num_envs, device=device, config_kw=kw, sim_config_kw=sim_kw, seed=seed,
-                          metrics=True, auto_reset=True, env_offset=env_offset, scenario_bank=True)
+                          metrics=True, auto_reset=True, env_offset=env_offset, scenario_bank=True,
+                          aircraft_parameters=air_names)
     state, target = _scenario_columns(scenarios, reps)
     res = vec.set_scenario_bank(state=state, target=target,
                                 turbulence_intensity=None if levels is None else
-                                [lv for lv in levels for _ in range(n_scen)])
+                                [lv for lv in levels for _ in range(n_scen)], aircraft=air)
     vec.enable_f64_outputs(True)
     vec.reset()                                          # env e starts scenario e
     pid = DevicePID(vec) if controller == "pid" else None
@@ -238,11 +271,8 @@ def _evaluate_banked(scenarios, config_path, controller, config_kw, metrics, lev
         raise RuntimeError("banked evaluation did not finish every scenario")
     rows, ln = res["episode"].cpu().numpy(), res["length"].long().cpu().numpy()
     tr = None if rew_trace is None else rew_trace.cpu().numpy()
-    if levels is None:
-        return _results(vec, metrics, rows, tr, ln), vec
-    return {lv: _results(vec, metrics, rows[j * n_scen:(j + 1) * n_scen],
-                         None if tr is None else tr[:, j * n_scen:(j + 1) * n_scen], ln[j * n_scen:(j + 1) * n_scen])
-            for j, lv in enumerate(levels)}, vec
+    variants = None if air is None else [None] * reps
+    return _split(vec, metrics, rows, tr, ln, n_scen, levels, variants), vec
 
 
 def _results(vec, metrics, rows, tr, ln):

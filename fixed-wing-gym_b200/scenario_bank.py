@@ -1,7 +1,7 @@
 """Scenario banks (include/fwgym.h fw_bank_t): the host half - table building and validation, and a numpy mirror of
 the rule by which envs take scenarios.
 
-A bank is S scenarios of initial states and targets (NaN = sample it), optionally a Dryden level each.  Resets of a
+A bank is S scenarios of initial states and targets (NaN = sample it), optionally a Dryden level and an aircraft each.  Resets of a
 handle created with scenario_bank=True consume them in order on the device: env e flies first + e, then
 first + e + stride, first + e + 2 stride, ... (modulo S when cycling), and the env kernel writes each scenario's outcome
 into a row of its own.
@@ -48,11 +48,20 @@ def level_codes(levels):
 
 
 def build_tables(state=None, target=None, turbulence_intensity=None, target_names=(), mixed=False):
-    """-> (S, init_state [N_INIT_ROWS, S] or None, init_target [FW_MAX_TARGETS, S] or None, levels [S] int32 or None).
+    """-> (S, init_state [N_INIT_ROWS, S] or None, init_target [FW_MAX_TARGETS, S] or None, levels [S] int32 or None):
+    build_bank_tables without an aircraft column."""
+    return build_bank_tables(state, target, turbulence_intensity, target_names, mixed)[:4]
+
+
+def build_bank_tables(state=None, target=None, turbulence_intensity=None, target_names=(), mixed=False, aircraft=None,
+                      aircraft_parameters=()):
+    """-> (S, init_state [N_INIT_ROWS, S] or None, init_target [FW_MAX_TARGETS, S] or None, levels [S] int32 or None,
+    aircraft [len(aircraft_parameters), S] or None).
 
     `state` / `target`: dicts name -> one value per scenario (a scalar applies to every scenario), with the names
     reset(state=, target=) takes; "wind" is a [3, S] (or [3]) entry.  `turbulence_intensity`: one level per scenario
-    (mixed handles only).  S is the length of the per-scenario entries, which must all agree."""
+    (mixed handles only).  `aircraft`: dict name -> one value per scenario of the handle's `aircraft_parameters` (NaN =
+    the env's own request).  S is the length of the per-scenario entries, which must all agree."""
     cols = []          # (table, row, values)
     for name, val in dict(state or {}).items():
         if name == "wind":
@@ -68,6 +77,14 @@ def build_tables(state=None, target=None, turbulence_intensity=None, target_name
         if name not in target_names:
             raise ValueError("unknown target %r (targets of this configuration: %s)" % (name, ", ".join(target_names)))
         cols.append(("target", target_names.index(name), _column(val, name), name))
+    aircraft_parameters = tuple(aircraft_parameters)
+    if aircraft is not None and not aircraft_parameters:
+        raise ValueError("an aircraft column needs a handle with aircraft_parameters")
+    for name, val in dict(aircraft or {}).items():
+        if name not in aircraft_parameters:
+            raise ValueError("%r is not an aircraft parameter of this env (aircraft_parameters: %s)"
+                             % (name, ", ".join(aircraft_parameters)))
+        cols.append(("aircraft", aircraft_parameters.index(name), _column(val, name), name))
     levels = None
     if turbulence_intensity is not None:
         if not mixed:
@@ -84,19 +101,23 @@ def build_tables(state=None, target=None, turbulence_intensity=None, target_name
     S = lens.pop()
     if S < 1 or S > INT32_MAX:
         raise ValueError("a bank holds 1 .. 2^31 - 1 scenarios, not %d" % S)
-    init_state = init_target = None
+    init_state = init_target = air = None
     for table, row, v, _ in cols:
         if table == "state":
             if init_state is None:
                 init_state = np.full((N_INIT_ROWS, S), np.nan)
             init_state[row] = v
+        elif table == "aircraft":
+            if air is None:
+                air = np.full((len(aircraft_parameters), S), np.nan)
+            air[row] = v
         else:
             if init_target is None:
                 init_target = np.full((_capi.DEFINES["FW_MAX_TARGETS"], S), np.nan)
             init_target[row] = v
     if levels is not None and levels.shape[0] == 1:
         levels = np.full(S, levels[0], dtype=np.int32)
-    return S, init_state, init_target, levels
+    return S, init_state, init_target, levels, air
 
 
 def check_assignment(n_envs, n_scenarios, first, stride):

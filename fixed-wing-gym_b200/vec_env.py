@@ -87,7 +87,10 @@ class FixedWingVecEnv:
     def __init__(self, config_path=None, num_envs=1, device="cuda:0", sampler=None, sim_config_path=None,
                  sim_parameter_path=None, config_kw=None, sim_config_kw=None, seed=0, precision="fp64",
                  env_offset=0, auto_reset=True, keep_terminal_obs=False, metrics=False, info_keywords=(),
-                 scenario_bank=False):
+                 scenario_bank=False, aircraft_parameters=()):
+        """`aircraft_parameters`: names of model parameters that may differ per env (set_aircraft): the live model
+        parameters but ar, rho, g, Jx, Jy, Jz, Jxz (CompiledConfig.AIRCRAFT_PARAMS).  Not together with
+        simulator-parameter randomisation, and b only with turbulence off."""
         if sampler is not None:
             raise NotImplementedError("adaptive sampler hook is out of scope (SURVEY §2 #18)")
         self._lib = _capi.lib()   # raises if the CUDA extension is not built: no fallback
@@ -102,7 +105,8 @@ class FixedWingVecEnv:
         self.info_keywords = tuple(info_keywords)
         self.scenario_bank = bool(scenario_bank)   # keep the scenario-bank rows: set_scenario_bank
         self.cc = CompiledConfig(config_path, sim_config_path, sim_parameter_path, config_kw, sim_config_kw, precision,
-                                 metrics=self.metrics, scenario_bank=self.scenario_bank)
+                                 metrics=self.metrics, scenario_bank=self.scenario_bank,
+                                 aircraft_parameters=aircraft_parameters)
         self.cfg = self.cc.cfg
         self.target_names = list(self.cc._target_props_init["states"].keys())
         self.observation_space = Box(self.cc.observation_low, self.cc.observation_high)
@@ -443,29 +447,80 @@ class FixedWingVecEnv:
         lvl = TURB_LEVELS.index(sc.get("turbulence_intensity") or "light") if sc["turbulence"] else 0
         return torch.full((self.num_envs,), lvl, dtype=torch.int32, device=self.device)
 
+    # ------------------------------------------------------------------------------------------- per-env aircraft
+    def set_aircraft(self, values, indices=None):
+        """Request the aircraft of envs (all, or `indices`) from their next reset on (explicit or automatic; the running
+        episodes keep theirs).  `values`: dict name -> a scalar, an array / tensor with one value per selected env; the
+        names are among the handle's aircraft_parameters, and NaN goes back to the handle's nominal value.  An env flies
+        the aircraft a reference env built from a parameter file with these values would fly (include/fwgym.h
+        fw_set_aircraft).  Parameters not named keep their requests."""
+        names = self.cc.aircraft_parameters
+        if not names:
+            raise _capi.FwError("construct the env with aircraft_parameters=(...) to set aircraft per env")
+        idx = None if indices is None else torch.as_tensor(np.atleast_1d(indices), dtype=torch.long, device=self.device)
+        count = self.num_envs if idx is None else len(idx)
+        req = self.aircraft_requests().clone()
+        for name, val in dict(values).items():
+            if name not in names:
+                raise ValueError("%r is not an aircraft parameter of this env (aircraft_parameters: %s)"
+                                 % (name, ", ".join(names)))
+            v = torch.as_tensor(val.cpu() if torch.is_tensor(val) else np.asarray(val, dtype=np.float64),
+                                dtype=torch.float64).to(self.device).reshape(-1)
+            if v.numel() == 1 and count != 1:
+                v = v.expand(count)
+            if v.numel() != count:
+                raise ValueError("aircraft parameter %s: %d values for %d envs" % (name, v.numel(), count))
+            if idx is None:
+                req[names.index(name)] = v
+            else:
+                req[names.index(name), idx] = v
+        check_aircraft(self.cc, req)
+        req = req.contiguous()
+        _capi.check(self._lib.fw_set_aircraft(self._h, self._ptr(req), self._stream()))
+        self._aircraft_keepalive = req
+
+    def aircraft_requests(self):
+        """Device float64 [len(aircraft_parameters), N]: the requested value of every aircraft parameter per env (NaN =
+        nominal), rows in aircraft_parameters order."""
+        rows = self.state_rows()
+        if "aircraft_req" not in rows:
+            raise _capi.FwError("construct the env with aircraft_parameters=(...)")
+        return self.get_rows(rows.index("aircraft_req"), len(self.cc.aircraft_parameters))
+
+    def aircraft(self):
+        """name -> device float64 [N]: the requested aircraft of every env (NaN = nominal), as set_aircraft takes it."""
+        req = self.aircraft_requests()
+        return {n: req[j] for j, n in enumerate(self.cc.aircraft_parameters)}
+
     # ------------------------------------------------------------------------------------------ scenario banks
     def set_scenario_bank(self, state=None, target=None, turbulence_intensity=None, first=None, stride=None,
-                          cycle=False):
+                          cycle=False, aircraft=None):
         """Attach a bank of S scenarios that the resets of this env consume in order (include/fwgym.h fw_bank_t): every
         auto-reset, and reset() without state= / target=, starts the env's next scenario - env e flies first + e, then
         + stride per episode (modulo S with `cycle`) - until the env is past the bank, after which it samples as usual.
         `state` / `target`: the names reset(state=, target=) takes, one value per scenario (NaN = sample it; a scalar
-        applies to all); `turbulence_intensity`: one level per scenario (mixed handles; -1 = the env's own rule).
+        applies to all); `turbulence_intensity`: one level per scenario (mixed handles; -1 = the env's own rule);
+        `aircraft`: dict aircraft parameter -> one value per scenario (a finite value pins the scenario's aircraft like
+        set_aircraft, NaN = the env's own request).
         `first` / `stride` default to 0 / num_envs; sharded ranks pass first = env_offset and stride = the total env
         count.  Allocates the result rows scenario_results() returns (cycling banks: the counters only).  Takes effect
         at the envs' next reset.  Attaching clears every env's running scenario id: an episode that is running now (from
         an earlier bank) finishes, but reports no result anywhere."""
         if not self.scenario_bank:
             raise _capi.FwError("construct the env with scenario_bank=True")
-        S, st, tg, lv = scenario_bank.build_tables(state, target, turbulence_intensity, self.target_names,
-                                                   mixed=bool(self.cc.turbulence_mix))
+        S, st, tg, lv, air = scenario_bank.build_bank_tables(state, target, turbulence_intensity, self.target_names,
+                                                             mixed=bool(self.cc.turbulence_mix), aircraft=aircraft,
+                                                             aircraft_parameters=self.cc.aircraft_parameters)
+        if air is not None:
+            check_aircraft(self.cc, torch.as_tensor(air))
         first = 0 if first is None else int(first)
         stride = self.num_envs if stride is None else int(stride)
         scenario_bank.check_assignment(self.num_envs, S, first, stride)
         d = self.device
         keep = {"init_state": None if st is None else torch.as_tensor(st, device=d),
                 "init_target": None if tg is None else torch.as_tensor(tg, device=d),
-                "turb_level": None if lv is None else torch.as_tensor(lv, device=d)}
+                "turb_level": None if lv is None else torch.as_tensor(lv, device=d),
+                "aircraft": None if air is None else torch.as_tensor(air, device=d)}
         res = {"episodes": torch.zeros(S, dtype=torch.int32, device=d),
                "successes": torch.zeros(S, dtype=torch.int32, device=d)}
         if not cycle:
@@ -475,13 +530,16 @@ class FixedWingVecEnv:
             if self.metrics:
                 res["episode"] = torch.full((S, self.ep_dim), float("nan"), dtype=torch.float64, device=d)
         b = _capi.fw_bank_t()
-        b.init_state, b.init_target, b.turb_level = (t.data_ptr() if t is not None else None for t in keep.values())
+        b.init_state, b.init_target, b.turb_level = (keep[k].data_ptr() if keep[k] is not None else None
+                                                     for k in ("init_state", "init_target", "turb_level"))
         b.n_scenarios, b.first, b.stride, b.cycle = S, first, stride, 1 if cycle else 0
         for f, k in (("term", "term"), ("length", "length"), ("ret", "return"), ("episode", "episode"),
                      ("episodes", "episodes"), ("successes", "successes")):
             if k in res:
                 setattr(b, f, res[k].data_ptr())
         _capi.check(self._lib.fw_set_bank(self._h, ctypes.byref(b), self._stream()))
+        if keep["aircraft"] is not None:
+            _capi.check(self._lib.fw_set_bank_aircraft(self._h, self._ptr(keep["aircraft"])))
         self._bank = (keep, res)          # the device reads these while the bank is attached
         self.n_scenarios = S
         self.config_version += 1          # the bank is a kernel parameter: captured graphs hold the old one
@@ -574,6 +632,29 @@ class FixedWingVecEnv:
         pod = self.cc.pod()
         _capi.check(self._lib.fw_set_config(self._h, ctypes.byref(pod)))
         self.config_version += 1   # the configuration is a kernel parameter: captured graphs hold the old one
+
+
+def check_aircraft(cc, req):
+    """Refuse aircraft requests [len(cc.aircraft_parameters), M] (NaN = nominal) that no parameter file could hold: an
+    infinite value, mass, Jy, b or S_wing <= 0, or an inertia tensor with Jx Jz - Jxz^2 <= 0."""
+    names = cc.aircraft_parameters
+    req = req.to(torch.float64)
+    if bool(torch.isinf(req).any()):
+        raise ValueError("aircraft parameters must be finite (NaN = nominal)")
+    nominal = cc.aircraft_nominal()
+    par = dict(cc.params)
+
+    def value(name):
+        if name in names:
+            r = req[names.index(name)]
+            return torch.where(torch.isnan(r), torch.full_like(r, nominal[name]), r)
+        return torch.full(req.shape[1:], float(par[name]), dtype=torch.float64, device=req.device)
+    for name in ("mass", "Jy", "b", "S_wing"):
+        if name in names and not bool((value(name) > 0).all()):
+            raise ValueError("aircraft parameter %s must be > 0" % name)
+    if any(n in names for n in ("Jx", "Jz", "Jxz")):
+        if not bool((value("Jx") * value("Jz") - value("Jxz") ** 2 > 0).all()):
+            raise ValueError("aircraft inertia must have Jx * Jz - Jxz^2 > 0")
 
 
 class HostStepper:

@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define FW_ABI_VERSION 12
+#define FW_ABI_VERSION 13
 
 /* ---------------------------------------------------------------------------------------------- limits */
 #define FW_MAX_OBS_VARS 32
@@ -37,6 +37,8 @@ extern "C" {
 #define FW_N_PAR 53           /* == FW_PAR_N below (model parameters that can differ per env) */
 #define FW_MAX_RAND 64        /* entries of simulator-parameter randomisation per reset */
 #define FW_N_TURB_LEVELS 4    /* Dryden intensities of a mixed handle: 0 none, 1 light, 2 moderate, 3 severe */
+#define FW_N_INERTIA 9        /* inertia terms of the right-hand side: gammas[1..8], inv_Jy */
+#define FW_MAX_AIRCRAFT 53    /* per-env aircraft parameters: the live ones but ar, rho, g, Jx, Jy, Jz, Jxz */
 
 /* PyFly state-variable ids (order of oracle/pyfly_restated.py REQUIRED_VARIABLES + elevons) */
 enum fw_sv {
@@ -48,8 +50,10 @@ enum fw_sv {
 
 /* Model parameters the right-hand side reads LIVE at every evaluation (PyFly.params[...] / PyFly.rho / PyFly.g), i.e.
  * the ones whose per-episode randomisation (fixed_wing.py:523-570) changes the dynamics.  The inertia entries are not
- * here: PyFly folds them into gammas at construction, so randomising them consumes a draw and changes nothing.  The
- * last three are derived per env at reset (1/mass, 1/(pi e AR), exp(2 M a_0)). */
+ * here: PyFly folds them into gammas at construction, so randomising them consumes a draw and changes nothing (a
+ * per-env aircraft, fw_set_aircraft, does set them: see fw_air).  The last three are derived per env at reset (1/mass,
+ * 1/(pi e AR), exp(2 M a_0)).  FW_PAR_MASS .. FW_PAR_C_N_DELTA_R are in the order of the fw_sim_t fields mass ..
+ * C_n_delta_r. */
 enum fw_par {
   FW_PAR_MASS = 0, FW_PAR_S_WING, FW_PAR_B, FW_PAR_C, FW_PAR_S_PROP, FW_PAR_K_MOTOR, FW_PAR_K_T_P, FW_PAR_K_OMEGA,
   FW_PAR_C_PROP, FW_PAR_E, FW_PAR_M, FW_PAR_A_0, FW_PAR_AR,
@@ -65,6 +69,11 @@ enum fw_par {
   FW_PAR_INV_MASS, FW_PAR_INV_PI_E_AR, FW_PAR_EXP_2MA0,
   FW_PAR_N
 };
+
+/* Ids of the per-env aircraft parameters (fw_sim_t.air_id): a fw_par id for the live parameters but FW_PAR_AR (always
+ * b^2 / S_wing) and the derived ones, and these four for the inertia, which reaches the right-hand side only through
+ * gammas[1..8] and inv_Jy (FW_AIR_JX == FW_PAR_N). */
+enum fw_air { FW_AIR_JX = 53, FW_AIR_JY, FW_AIR_JZ, FW_AIR_JXZ };
 
 enum fw_status {
   FW_OK = 0, FW_ERR_ARG = -1, FW_ERR_CUDA = -2, FW_ERR_CONFIG = -3, FW_ERR_ALLOC = -4, FW_ERR_ABI = -5,
@@ -180,10 +189,18 @@ typedef struct {
   double turb_cdf[FW_N_TURB_LEVELS];
   double turb_C[FW_N_TURB_LEVELS][FW_N_FILT][FW_FILT_MAXN];
   double turb_D[FW_N_TURB_LEVELS][FW_N_FILT];
+  /* per-env aircraft (fw_env_t.n_aircraft > 0, fw_set_aircraft): aircraft request row j sets parameter air_id[j]
+   * (fw_air) at each reset; a NaN request flies the nominal value (the field above, or Jx / Jy / Jz / Jxz).  Listed
+   * parameters, ar (when b or S_wing is listed), the derived rows and the inertia terms live in per-env parameter rows:
+   * inertia_slot1[k] = 1 + row of gammas[1 + k] (k < 8) / inv_Jy (k = 8), 0 = the constant above.  All zero when no
+   * aircraft parameter is listed. */
+  double Jx, Jz, Jxz;
+  int32_t air_id[FW_MAX_AIRCRAFT];
+  int32_t inertia_slot1[FW_N_INERTIA];
   /* keeps sizeof(fw_sim_t) congruent to its earlier size (ABI 10) modulo 32, so every kernel parameter after it, also
    * behind the float image of the fp32 dynamics kernels (1.5x), keeps its 16-byte alignment and the compiler its
    * 128-bit constant loads: the kernels of existing configurations compile to the same instructions */
-  double _pad_turb[3];
+  int32_t _pad_air[2];
 } fw_sim_t;
 
 /* One draw of FixedWingAircraft.sample_simulator_parameters (fixed_wing.py:523-570), in the reference's order.
@@ -204,7 +221,8 @@ typedef struct {
   int32_t obs_len, obs_step, obs_nvar, obs_shape, obs_norm, obs_noise;
   double obs_noise_mean, obs_noise_std;
   fw_obs_var_t obs[FW_MAX_OBS_VARS];
-  int32_t has_bounds, _pad3;
+  int32_t has_bounds;
+  int32_t n_aircraft;             /* per-env aircraft parameters: double state rows "aircraft_req" (fw_set_aircraft) */
   double bounds_min[FW_N_ACT], bounds_max[FW_N_ACT];
   int32_t n_targets, resample_every, streak_req, on_success;   /* on_success: 0 none, 1 done, 2 new */
   double streak_fraction;
@@ -314,6 +332,16 @@ int fw_host_wait(fw_handle h, int slot, const float** obs, const float** rew, co
  * and active levels are the state rows "turb_level_req" / "turb_level" (fw_get_state / fw_set_state). */
 int fw_set_turbulence_levels(fw_handle h, const int32_t* levels, void* stream);
 
+/* Per-env aircraft (fw_env_t.n_aircraft > 0): values = device double [fw_aircraft_dim(h), N], row j = the requested value
+ * of parameter fw_sim_t.air_id[j] for every env, NaN = the handle's nominal value; NULL sets every request to NaN.
+ * Takes effect at each env's next reset (explicit or automatic): the reset writes the episode's parameters and
+ * recomputes what PyFly derives from them at construction (ar = b^2 / S_wing, 1/mass, 1/(pi e ar), exp(2 M a_0),
+ * gammas[1..8] and 1/Jy), so the running episode keeps its aircraft.  No random draw is added or moved.  FW_ERR_ARG on a
+ * handle without aircraft parameters.  The requests are the state rows "aircraft_req" (fw_get_state / fw_set_state). */
+int fw_set_aircraft(fw_handle h, const double* values, void* stream);
+/* Number of per-env aircraft parameters of the handle (rows of fw_set_aircraft), 0 when none. */
+int64_t fw_aircraft_dim(fw_handle h);
+
 /* Scenario bank (handles created with fw_env_t.bank_enabled): a device table of S initial states / targets that resets
  * consume in order, with one result row per scenario.  Every env keeps two int32 state rows: "bank_next" (scenario id of
  * its next banked episode) and "bank_scenario" (scenario id of the running episode, -1 when it is not from the bank).
@@ -345,8 +373,14 @@ typedef struct {
 } fw_bank_t;
 /* Attach (bank != NULL) or detach (NULL) a scenario bank.  FW_ERR_ARG: the handle was not created with bank_enabled,
  * S <= 0 or S > INT32_MAX, first < 0, stride < n_envs, an episode buffer without metrics, outcome rows (term / length /
- * ret / episode) together with cycle, or a level column on a handle that is not mixed. */
+ * ret / episode) together with cycle, or a level column on a handle that is not mixed.  Attaching or detaching also
+ * detaches the aircraft column (fw_set_bank_aircraft). */
 int fw_set_bank(fw_handle h, const fw_bank_t* bank, void* stream);
+/* Aircraft column of the attached bank (handles with aircraft parameters): aircraft = device double [fw_aircraft_dim(h),
+ * S], NULL = none.  A finite entry pins that parameter of the scenario's episodes like fw_set_aircraft; NaN keeps the
+ * env's request.  The column must stay valid while it is attached; the next fw_set_bank detaches it.  FW_ERR_ARG: the
+ * handle has no aircraft parameters, or no bank is attached. */
+int fw_set_bank_aircraft(fw_handle h, const double* aircraft);
 
 /* Rows [row0, row0 + nrows) of the state matrix below: device double [nrows, N] (e.g. the three target rows without
  * exporting the whole state). */
